@@ -283,9 +283,26 @@ def run_ours(args):
     if sampler:
         sampler.start()                                  # before any warm-up: starting it later stalls rank 0's launch thread
 
-    def measure(scaling, steps, with_kernels, with_e2e, in_dtype="f32"):
+    def step_outputs(loss, model, ts):
+        """What a caller of the timed step receives after it (host copies): the loss (with world > 1 the global mean, not
+        this rank's share), the parameters Adam updated (the dead encoder is never updated and is left out) and the
+        floating-point buffers the step updates (BatchNorm running statistics)."""
+        if world > 1:
+            loss = ts.global_loss()
+        out = {"loss": loss.detach().float().reshape(1).cpu().numpy()}
+        live = {id(p) for p in ts.opt.live}
+        for name, p in model.named_parameters():
+            if id(p) in live:
+                out["param." + name] = p.detach().float().cpu().numpy()
+        for name, b in model.named_buffers():
+            if b.is_floating_point():
+                out["buffer." + name] = b.detach().float().cpu().numpy()
+        return out
+
+    def measure(scaling, steps, with_kernels, with_e2e, in_dtype="f32", keep_outputs=False):
         """One workload (strong: args.total_utts in total; weak: per GPU) -> dict of measurements (same on every rank).
-        in_dtype "bf16": the bf16 input-feature mode (features stored in bf16, row pitch 1448 elements; everything else fp32)."""
+        in_dtype "bf16": the bf16 input-feature mode (features stored in bf16, row pitch 1448 elements; everything else fp32).
+        keep_outputs: out["outputs"] = step_outputs() of the last timed step of the headline loop."""
         weak = scaling == "weak"
         lengths_all = synth.config5_lengths(args.total_utts * (world if weak else 1), seed=0)
         total_utts = int(lengths_all.sum())
@@ -347,6 +364,8 @@ def run_ours(args):
                             "launches_per_step": (_lib.launch_count() - launches0) / steps}
             out["ksum"] = timer.summary()
             out["step_kernel_ms"] = sum(t for _, t in out["ksum"].values()) / steps
+            if keep_outputs:
+                out["outputs"] = step_outputs(last, model, ts)
             return last
 
         if with_kernels or args.mode == "eager":
@@ -384,6 +403,8 @@ def run_ours(args):
                                 "step_ms": [round(a.elapsed_time(b), 3) for a, b in zip([e0] + marks[:-1], marks)],
                                 "host_launches_in_timed_region": _lib.launch_count() - lc0,
                                 "cuda_mallocs_in_timed_region": int(mem_after.get("num_device_alloc", 0) - mem_before.get("num_device_alloc", 0))}
+                if keep_outputs:
+                    out["outputs"] = step_outputs(loss, model, ts)
             except Exception as e:                             # report, and fall back to the eager numbers
                 graph_err = "%s: %s" % (type(e).__name__, str(e)[:300])
                 out["graph_error"] = graph_err
@@ -482,11 +503,14 @@ def run_ours(args):
         torch.cuda.empty_cache()
         return out
 
-    head = measure(args.scaling, args.steps, with_kernels=True, with_e2e=True)
+    head = measure(args.scaling, args.steps, with_kernels=True, with_e2e=True, keep_outputs=bool(args.dump_outputs))
     if args.profile_step:
         if rank == 0:
             emit(head)
         return
+    outputs = head.pop("outputs", None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
     clocks = sampler.finish() if sampler else None
     other = None
     if world > 1 and not args.no_second_scaling:
@@ -623,6 +647,22 @@ def run_ours(args):
         os._exit(0)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """Writes each array as <directory>/<name>.npy, so that two builds run with the same arguments (hence the same inputs)
+    can be compared output by output."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes of outputs exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_library_yardstick(args):
     """NOT the product path: times what a library gives for the two projection GEMMs of the workload on this box --
     cuBLAS through torch.matmul in exact fp32 (allow_tf32 off), in TF32 (10-bit mantissa: 1e-3 accuracy, outside the 1e-5 bar)
@@ -737,7 +777,13 @@ def main():
                     help="time cuBLAS (fp32 / TF32 / bf16) on the projection GEMM shapes next to libercgraph's kernels and exit")
     ap.add_argument("--no-bf16-mode", action="store_true", help="N = 1: skip the extra bf16 input-feature-mode measurement")
     ap.add_argument("--no-second-scaling", action="store_true", help="N > 1: skip the extra weak- (or strong-) scaling measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (loss.npy; param.<name>.npy: the parameters "
+                         "Adam updated; buffer.<name>.npy: BatchNorm running statistics; float32) to DIR")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.library_yardstick or args.profile_step):
+        ap.error("--dump-outputs needs the timed train step of our arm (not --impl reference, --library-yardstick "
+                 "or --profile-step)")
     _quiet_stdout()
     if args.library_yardstick:
         run_library_yardstick(args)

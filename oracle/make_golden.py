@@ -111,7 +111,7 @@ def cogmen_fixture(ref):
         out["param/" + k] = v
     for k, v in grads.items():
         out["grad/" + k] = v
-    np.savez_compressed(os.path.join(OUT, "cogmen_small.npz"), **out)
+    _save_split("cogmen_small", out)
     print("cogmen_small.npz loss", float(loss), "live grads", len(grads))
 
 
@@ -151,8 +151,14 @@ def dgcn_fixture(ref):
         out["param/" + k] = v
     for k, v in grads.items():
         out["grad/" + k] = v
-    np.savez_compressed(os.path.join(OUT, "dgcn_small.npz"), **out)
+    _save_split("dgcn_small", out)
     print("dgcn_small.npz loss", float(loss), "live grads", len(grads))
+
+
+def _save_split(name, out):
+    """name.npz without the gradients, name_grads.npz with them: each file stays under 1 MB."""
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **{k: v for k, v in out.items() if not k.startswith("grad/")})
+    np.savez_compressed(os.path.join(OUT, name + "_grads.npz"), **{k: v for k, v in out.items() if k.startswith("grad/")})
 
 
 def _store_grads(out, grads, big=4096):

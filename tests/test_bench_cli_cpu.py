@@ -19,7 +19,8 @@ def _bench():
 def test_help_prints_every_option():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stderr[-1000:]
-    for opt in ("--gpus", "--steps", "--warmup", "--impl", "--scaling", "--transport", "--bn-sync", "--library-yardstick"):
+    for opt in ("--gpus", "--steps", "--warmup", "--impl", "--scaling", "--transport", "--bn-sync", "--library-yardstick",
+                "--dump-outputs"):
         assert opt in r.stdout, opt
 
 
@@ -35,3 +36,26 @@ def test_kernel_labels_match_the_traffic_table():
     traffic = json.load(open(os.path.join(ROOT, "profiles", "traffic.json")))
     for key in ("gemm_nn_tc[K=1443,N=100]", "gemm_tn_tc[K1=1443,N1=100]"):
         assert key in traffic, key
+
+
+def test_dump_outputs_writes_one_npy_per_array_and_refuses_more_than_64_mb(tmp_path):
+    import numpy as np
+    import pytest
+    b = _bench()
+    arrays = {"loss": np.array([1.5], dtype=np.float32), "param.cls.0.weight": np.arange(6, dtype=np.float32).reshape(2, 3)}
+    b.dump_outputs(str(tmp_path / "out"), arrays)
+    assert sorted(os.listdir(tmp_path / "out")) == ["loss.npy", "param.cls.0.weight.npy"]
+    for k, v in arrays.items():
+        got = np.load(tmp_path / "out" / (k + ".npy"))
+        assert got.dtype == v.dtype and np.array_equal(got, v)
+    with pytest.raises(SystemExit):
+        b.dump_outputs(str(tmp_path / "big"), {"x": np.zeros(b.DUMP_LIMIT_BYTES // 4 + 1, dtype=np.float32)})
+    assert not (tmp_path / "big").exists()
+
+
+def test_dump_outputs_is_refused_where_no_train_step_is_timed(tmp_path):
+    for extra in (["--impl", "reference"], ["--library-yardstick"], ["--profile-step"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", str(tmp_path / "d")] + extra,
+                           capture_output=True, text=True, timeout=300)
+        assert r.returncode == 2 and "--dump-outputs" in r.stderr, (extra, r.stderr[-500:])
+        assert not (tmp_path / "d").exists()
