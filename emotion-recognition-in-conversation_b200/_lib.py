@@ -85,6 +85,8 @@ SIGNATURES = {
     "ercg_lstm_fwd": (I, [P, L, P, P, I, I, P, L, P, P, P, P]),
     "ercg_lstm_bwd": (I, [P, L, P, P, P, P, I, I, P, L, P]),
     "ercg_dropout": (I, [P, P, L, F, U64, P]),
+    "ercg_gru_fwd": (I, [P, L, P, P, P, I, I, P, L, P, P, P]),
+    "ercg_gru_bwd": (I, [P, L, P, P, P, P, I, I, P, L, P, L, P]),
     "ercg_bn_workspace_bytes": (SZ, [L, I]),
     "ercg_bn_stats": (I, [P, L, L, I, P, P, P, SZ, P]),
     "ercg_bn_running_update": (I, [P, P, P, P, P, F, F, I, P]),

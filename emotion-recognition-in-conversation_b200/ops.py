@@ -747,6 +747,49 @@ def lstm_layer(gx, whh, graph):
     return _LstmLayer.apply(gx, whh, graph)
 
 
+# ------------------------------------------------------------------------------------------- K6b GRU
+class _GruLayer(torch.autograd.Function):
+    """One bidirectional nn.GRU layer on packed rows: gx [N, 6*Hd] (= x W_ih^T + b_ih, both directions), whh [2, 3*Hd, Hd],
+    bhh [2, 3*Hd] -> out [N, 2*Hd].  b_hh is applied inside the recurrence (b_hn is scaled by the reset gate)."""
+
+    @staticmethod
+    def forward(ctx, gx, whh, bhh, graph):
+        gx, ldgx = _rows(gx)
+        whh, bhh = whh.contiguous(), bhh.contiguous()
+        N, Hd = gx.size(0), whh.size(2)
+        assert gx.size(1) == 6 * Hd and whh.shape == (2, 3 * Hd, Hd) and bhh.shape == (2, 3 * Hd), (gx.shape, whh.shape, bhh.shape)
+        dev = gx.device
+        out = torch.empty((N, 2 * Hd), dtype=torch.float32, device=dev)
+        gates = torch.empty((N, 8 * Hd), dtype=torch.float32, device=dev)
+        hprev = torch.empty((N, 2 * Hd), dtype=torch.float32, device=dev)
+        check(lib().ercg_gru_fwd(_p(gx), ldgx, _p(whh), _p(bhh), _p(graph.node_off), graph.B, Hd, _p(out), 2 * Hd, _p(gates),
+                                 _p(hprev), _stream()), "ercg_gru_fwd")
+        ctx.graph, ctx.Hd = graph, Hd
+        ctx.save_for_backward(whh, gates, hprev)
+        return out
+
+    @staticmethod
+    def backward(ctx, dout):
+        whh, gates, hprev = ctx.saved_tensors
+        g, Hd = ctx.graph, ctx.Hd
+        dout, ldo = _rows(dout)
+        N = dout.size(0)
+        dgx = torch.empty((N, 6 * Hd), dtype=torch.float32, device=dout.device)
+        dgh = torch.empty((N, 6 * Hd), dtype=torch.float32, device=dout.device)
+        check(lib().ercg_gru_bwd(_p(dout), ldo, _p(gates), _p(hprev), _p(whh), _p(g.node_off), g.B, Hd, _p(dgx), 6 * Hd,
+                                 _p(dgh), 6 * Hd, _stream()), "ercg_gru_bwd")
+        dwhh = dbhh = None
+        if ctx.needs_input_grad[1]:
+            dwhh = torch.stack([gemm_tn(dgh[:, d * 3 * Hd:(d + 1) * 3 * Hd], hprev[:, d * Hd:(d + 1) * Hd]) for d in range(2)])
+        if ctx.needs_input_grad[2]:
+            dbhh = colsum(dgh).view(2, 3 * Hd)
+        return dgx, dwhh, dbhh, None
+
+
+def gru_layer(gx, whh, bhh, graph):
+    return _GruLayer.apply(gx, whh, bhh, graph)
+
+
 class _Dropout(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, p, seed):

@@ -2,7 +2,7 @@
 EdgeAtt, Classifier with the reference's constructor arguments, forward signatures and state_dict keys.
 
 Kernel mapping:
-  SeqContext   packed 2-layer BiLSTM = hoisted input GEMM (K2) + register-resident recurrence (K6)   :10-33
+  SeqContext   packed 2-layer BiLSTM / BiGRU = hoisted input GEMM (K2) + register-resident recurrence (K6 / K6b) :10-33
   EdgeAtt      u = x W^T (K2) + per-source window softmax (K5); no B*L python loop                  :121-152
   batch_graphify  K1 packed CSR + EdgeAtt weights as edge_norm (canonical edge order)                :51-92
   GCN          vendored RGCNConv(edge_norm) = basis GEMM + relation GEMM + gather (K2,K3); GraphConv :36-48
@@ -22,18 +22,25 @@ def _fresh_seed():
     return int(torch.empty((), dtype=torch.int64).random_().item())
 
 
-def bilstm_forward(rnn, x2d, graph, a_rows, training):
-    """Multi-layer bidirectional nn.LSTM over the dialogues of ``graph`` (packed-sequence semantics): per layer one
-    hoisted input GEMM for all utterances and both directions (K2) + the recurrence kernel (K6)."""
+def birnn_forward(rnn, x2d, graph, a_rows, training):
+    """Multi-layer bidirectional nn.LSTM or nn.GRU over the dialogues of ``graph`` (packed-sequence semantics): per layer one
+    hoisted input GEMM for all utterances and both directions (K2) + the recurrence kernel (K6 LSTM, K6b GRU)."""
+    gru = isinstance(rnn, nn.GRU)
+    assert gru or isinstance(rnn, nn.LSTM), type(rnn)
     h = x2d
     for layer in range(rnn.num_layers):
         sfx = "_l%d" % layer
         w_ih = torch.cat([getattr(rnn, "weight_ih" + sfx), getattr(rnn, "weight_ih" + sfx + "_reverse")], 0)
-        b = torch.cat([getattr(rnn, "bias_ih" + sfx) + getattr(rnn, "bias_hh" + sfx),
-                       getattr(rnn, "bias_ih" + sfx + "_reverse") + getattr(rnn, "bias_hh" + sfx + "_reverse")], 0)
         w_hh = torch.stack([getattr(rnn, "weight_hh" + sfx), getattr(rnn, "weight_hh" + sfx + "_reverse")], 0)
-        gx = ops.linear(h, w_ih, b, a_rows=a_rows if layer == 0 else None)
-        h = ops.lstm_layer(gx, w_hh, graph)
+        b_ih = (getattr(rnn, "bias_ih" + sfx), getattr(rnn, "bias_ih" + sfx + "_reverse"))
+        b_hh = (getattr(rnn, "bias_hh" + sfx), getattr(rnn, "bias_hh" + sfx + "_reverse"))
+        rows = a_rows if layer == 0 else None
+        if gru:           # b_hn is scaled by the reset gate, so b_hh stays out of the hoisted GEMM
+            gx = ops.linear(h, w_ih, torch.cat(b_ih, 0), a_rows=rows)
+            h = ops.gru_layer(gx, w_hh, torch.stack(b_hh, 0), graph)
+        else:
+            gx = ops.linear(h, w_ih, torch.cat([b_ih[0] + b_hh[0], b_ih[1] + b_hh[1]], 0), a_rows=rows)
+            h = ops.lstm_layer(gx, w_hh, graph)
         if training and rnn.dropout > 0 and layer + 1 < rnn.num_layers:
             h = ops.dropout(h, rnn.dropout, _fresh_seed())
     return h
@@ -43,13 +50,16 @@ class SeqContext(nn.Module):
     def __init__(self, u_dim, g_dim, dropout=0.4, rnn_type="lstm"):
         super().__init__()
         self.input_size, self.hidden_dim = u_dim, g_dim
-        if rnn_type != "lstm":
-            raise NotImplementedError("DGCNModule always builds the LSTM variant (track_mm/dgcn.py:65)")
-        self.rnn = nn.LSTM(u_dim, g_dim // 2, dropout=dropout, bidirectional=True, num_layers=2, batch_first=True)
+        if rnn_type == "lstm":
+            self.rnn = nn.LSTM(u_dim, g_dim // 2, dropout=dropout, bidirectional=True, num_layers=2, batch_first=True)
+        elif rnn_type == "gru":
+            self.rnn = nn.GRU(u_dim, g_dim // 2, dropout=dropout, bidirectional=True, num_layers=2, batch_first=True)
+        else:
+            raise ValueError("rnn_type must be 'lstm' or 'gru', got %r" % (rnn_type,))
 
     def packed_forward(self, x2d, graph, a_rows=None):
         """x2d: [rows, u_dim]; a_rows maps packed node -> row of x2d (None = already packed). -> [N, g_dim]"""
-        return bilstm_forward(self.rnn, x2d, graph, a_rows, self.training)
+        return birnn_forward(self.rnn, x2d, graph, a_rows, self.training)
 
     def forward(self, text_len_tensor, text_tensor):
         """Reference signature: -> zero-padded [B, max(L), g_dim] like pad_packed_sequence."""

@@ -1,13 +1,14 @@
 """Drop-in for ``DGCNModule`` of track_mm/dgcnv2.py (reference :54-181; declare-lab DialogueGCN): same constructor, forward
 signature ``(input_tensor [L,B,D], speaker_tensor one-hot [L,B,n], attention_mask [B,L], text_length)`` (seq-first, one-hot
 speakers: dgcnv2.py:44-45), return values (logits [N,C] of the real utterances, features [N,2*hidden]) and state_dict keys.
-Base models: 'LSTM' (the default, dgcnv2.py:31: unpacked 2-layer BiLSTM over the padded batch) and 'None' (a Linear)."""
+Base models: 'LSTM' (the default, dgcnv2.py:31: unpacked 2-layer BiLSTM over the padded batch), 'GRU' (the same with a 2-layer
+BiGRU, K6b) and 'None' (a Linear).  'DialogRNN' is not rebuilt: no reference output pins the DialogueRNN classes."""
 import torch
 from torch import nn
 
 from .. import ops, ops_mmgcn
 from ..graph import build_graph, standard_edge_dict
-from .dgcn_models import bilstm_forward
+from .dgcn_models import birnn_forward
 from .dgcnv2_models import MaskedEdgeAttention, GraphNetwork
 from .mmgcn_utils import lengths_graph
 
@@ -20,10 +21,13 @@ class DGCNModule(nn.Module):
         graph_hidden_size, max_seq_len = 100, 110
         if base_model == "LSTM":
             self.lstm = nn.LSTM(input_size=input_size, hidden_size=hidden_size, num_layers=2, bidirectional=True, dropout=dropout)
+        elif base_model == "GRU":
+            self.gru = nn.GRU(input_size=input_size, hidden_size=hidden_size, num_layers=2, bidirectional=True, dropout=dropout)
         elif base_model == "None":
             self.base_linear = nn.Linear(input_size, 2 * hidden_size)
-        elif base_model in ("DialogRNN", "GRU"):
-            raise NotImplementedError("base_model=%r: only the default 'LSTM' (dgcnv2.py:31) and 'None' run on libercgraph" % base_model)
+        elif base_model == "DialogRNN":
+            raise NotImplementedError("base_model='DialogRNN' is not implemented: the DialogueRNN classes of dgcnv2_models.py are "
+                                      "not rebuilt, as no reference output pins them; use 'LSTM', 'GRU' or 'None'")
         else:
             raise NotImplementedError("Base model must be one of DialogRNN/LSTM/GRU")
         if avec:
@@ -44,8 +48,9 @@ class DGCNModule(nn.Module):
         gf = lengths_graph(torch.full((B,), Lmax, dtype=torch.int64), dev)     # every dialogue as a full-length sequence
         rows_full = ops_mmgcn.node_rows(gf, Lmax, seq_first=True)
         x2d = input_tensor.reshape(Lmax * B, D)
-        if self.base_model == "LSTM":                                          # unpacked: runs over the padding, dgcnv2.py:151
-            emo = bilstm_forward(self.lstm, x2d, gf, rows_full, self.training)
+        if self.base_model in ("LSTM", "GRU"):                                 # unpacked: runs over the padding, dgcnv2.py:151
+            rnn = self.lstm if self.base_model == "LSTM" else self.gru
+            emo = birnn_forward(rnn, x2d, gf, rows_full, self.training)
         else:
             emo = ops.linear(x2d, self.base_linear.weight, self.base_linear.bias, a_rows=rows_full)
         edge_norm = self.att_model.edge_weights(emo, g, Lmax)                  # [E], canonical by-destination order

@@ -11,8 +11,8 @@ Kernel mapping
                                                   fully connected per-dialogue graph (K1 with window -1 / -1)
   linear -> ReLU -> dropout -> smax_fc            ops.mlp_head
 The unused attention variants of the file (SimpleAttention, Attention 'mlp', MatchingAttention 'dot' / 'general' / 'concat')
-and the DialogueRNN / GRU base models are parameter holders or NotImplementedError: DGCNModule's default path (LSTM base,
-'attn1', nodal 'general2') never executes them.
+and the DialogueRNN base model are parameter holders or NotImplementedError: DGCNModule with 'attn1' and nodal 'general2'
+never executes them, whichever of its recurrent or linear bases it runs.
 """
 import torch
 from torch import nn

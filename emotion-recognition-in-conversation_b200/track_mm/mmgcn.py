@@ -13,7 +13,7 @@ from torch import nn
 
 from .. import ops, ops_mmgcn
 from ..graph import build_graph, standard_edge_dict
-from .dgcn_models import bilstm_forward
+from .dgcn_models import birnn_forward
 from .mmgcn_models import MMGCN, _fresh_seed
 from .mmgcn_utils import simple_batch_graphify, lengths_graph  # noqa: F401
 
@@ -87,7 +87,7 @@ class MMGCNModule(nn.Module):
             gf = lengths_graph(full_len, dev)
             rows_full = ops_mmgcn.node_rows(gf, Lmax, seq_first=True)
             t200 = ops.linear(text_feature.reshape(Lmax * B, -1), self.linear_l.weight, self.linear_l.bias, a_rows=rows_full)
-            emo = bilstm_forward(self.lstm_l, t200, gf, None, self.training)  # [B*Lmax, 200]
+            emo = birnn_forward(self.lstm_l, t200, gf, None, self.training)  # [B*Lmax, 200]
             fl = ops.pack_rows(emo.view(B, Lmax, -1), g, seq_first=False)
         feat = self.graph_model(fa, fv, fl, text_length, speaker_tensor, graph=g)
         p = self.dropout_.p if self.training else 0.0

@@ -329,6 +329,26 @@ int ercg_lstm_bwd(const float* dout, int64_t ldo, const float* gates, const floa
 int ercg_dropout(const float* x, float* out, int64_t n, float p, uint64_t seed, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * K6b packed bidirectional GRU recurrence, one layer: the nn.GRU context encoders of DGCNModule("GRU")
+ * (track_mm/dgcnv2.py, 2 layers run unpacked over the padded batch) and SeqContext(rnn_type="gru")
+ * (track_mm/dgcn_models.py:46-47, 2 layers over the packed sequence).  torch.nn.GRU semantics, gate order r,z,n:
+ *   r = sigmoid(gx_r + W_hr h + b_hr), z = sigmoid(gx_z + W_hz h + b_hz), n = tanh(gx_n + r (W_hn h + b_hn)),
+ *   h' = (1 - z) n + z h.
+ * gx[N, 6*Hd] = x @ [W_ih; W_ih_reverse]^T + b_ih (b_ih ONLY) is produced by ercg_gemm_nn; b_hh cannot be folded into it
+ * (b_hn is multiplied by r) and is added inside the recurrence.  whh = [2][3*Hd][Hd], bhh = [2][3*Hd] (forward, reverse).
+ * Dialogue d owns rows node_off[d]..node_off[d+1] (packed-sequence semantics, zero initial state).
+ * fwd writes out[N,2*Hd] and saves gates[N,8*Hd] (per direction r, z, n, hn = W_hn h + b_hn) and hprev[N,2*Hd] (= h_{t-1}).
+ * bwd writes dgx[N,6*Hd] = (da_r, da_z, da_n), the gradient w.r.t. gx, and dgh[N,6*Hd] = (da_r, da_z, r da_n), the
+ * gradient w.r.t. W_hh h + b_hh; the caller forms dW_hh = dgh^T @ hprev, db_hh = colsum(dgh), dW_ih = dgx^T @ x,
+ * db_ih = colsum(dgx), dx = dgx @ [W_ih; W_ih_reverse] with K2.
+ * Hd in {100 (the size the reference instantiates), 64, 48, 32, 24, 16, 8}; other values return ERCG_EINVAL.
+ * ------------------------------------------------------------------------------------------- */
+int ercg_gru_fwd(const float* gx, int64_t ldgx, const float* whh, const float* bhh, const int32_t* node_off, int B, int Hd,
+                 float* out, int64_t ldo, float* gates, float* hprev, void* stream);
+int ercg_gru_bwd(const float* dout, int64_t ldo, const float* gates, const float* hprev, const float* whh,
+                 const int32_t* node_off, int B, int Hd, float* dgx, int64_t lddgx, float* dgh, int64_t lddgh, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * BatchNorm1d (training statistics) + LeakyReLU of GNN.forward (cogmen.py:67-68,72).
  * stats: mean[H], var[H] (biased) over the N rows, fixed-order reduction.
  * ------------------------------------------------------------------------------------------- */
