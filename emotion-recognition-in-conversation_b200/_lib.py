@@ -67,9 +67,6 @@ SIGNATURES = {
     "ercg_colsum": (I, [P, L, L, I, P, P, SZ, P]),
     "ercg_gather_fwd": (I, [P, L, P, P, P, P, P, I, P, P, L, L, I, P]),
     "ercg_gather_bwd": (I, [P, L, P, L, P, P, P, P, P, P, I, I, P, L, P, L, I, P]),
-    "ercg_rgcn_window_workspace_bytes": (SZ, [L, I, I, I]),
-    "ercg_rgcn_window_supported": (I, [P, L, P, L, L, I, I, I, I, I]),
-    "ercg_rgcn_window": (I, [P, L, P, P, P, P, P, P, I, P, L, P, P, L, P, L, P, L, I, I, I, I, P, SZ, P]),
     "ercg_gather_window_bwd": (I, [P, L, P, P, P, P, P, P, I, I, P, L, L, I, I, I, P]),
     "ercg_attn_fwd": (I, [P, P, P, P, L, P, P, F, P, L, P, P, L, I, P]),
     "ercg_attn_bwd_dst": (I, [P, L, P, P, L, P, P, P, F, P, P, L, P, P, L, I, P]),

@@ -44,11 +44,6 @@ struct TcEpilogue {
   int dbg;   // ERCG_TC_DBG: performance experiments only (1 no MMA, 8 no B loads)
   long long* trace;   // ERCG_TC_TRACE: CTA 0 records clock64() per role and k-chunk (pipeline timeline, diagnostics only)
   const unsigned long long* seed_dev = nullptr;   // optional device word added to `seed` (fresh dropout mask per graph replay)
-  // AGG kernels only (aggregate-first relational convolution, see gemm_tc_nn_kernel<..., AGG>): CSR by row of a window graph
-  const int* g_rowptr = nullptr; const int* g_col = nullptr; const unsigned char* g_etype = nullptr; const int* g_eid = nullptr;
-  const int* g_rel_slot = nullptr; const float* g_w = nullptr; float* g_zside = nullptr; long long g_ldz = 0;
-  int g_S = 0, g_wlo = 0, g_box_rows = 0, g_H = 0;
-  const float* g_meta = nullptr;      // [tiles][AGG_META_WORDS][128] row metadata (rgcn_rowmeta_kernel)
 };
 constexpr int TR_N = 160;          // traced chunks
 constexpr int TR_ROLES = 5;        // 0 A producer, 1 splitter, 2 MMA, 3 epilogue (per group), 4 B producer
@@ -214,24 +209,18 @@ constexpr int TC_THREADS = 352;   // 4 splitter + 4 epilogue warps, A producer, 
 #ifndef TC_R2S_
 #define TC_R2S_ 4
 #endif
-constexpr int AGG_DMAX = 11;                 // maximum row degree of the aggregate-first kernels (window wlo + whi + 1)
-constexpr uint32_t AGG_STAGE_BYTES = 18432;   // one 32-column box of the tile rows + halo: up to 144 rows x 128 B
-constexpr int AGG_META_WORDS = 16;            // per row: deg | d0, slots lo, slots hi, 11 weights (word-major inside a tile)
-constexpr uint32_t AGG_META_TILE_BYTES = AGG_META_WORDS * TC_BM * 4;     // 8 KB per 128-row tile
-template <bool TWO, bool WIDE = false, bool AGG = false>
+template <bool TWO, bool WIDE = false>
 struct NnCfg {
   // pair + short tiles (WIDE: K <= 512, i.e. the K = 100 transforms with A resident across N tiles and the K = 300 / 400 input
   // gradients) keep the 4-slab staging -- with 4-16 chunks per tile the epilogue is a large share of a tile and staging slab
   // by slab, with its column sums in between, measured slower in the step -- and spend the freed B bytes on ring depth only;
   // pair + long K (K = 1443: 46 chunks per tile) stages one slab at a time and takes two more A stages
-  static constexpr int R = AGG ? 4 : (TWO ? (WIDE ? TC_R2S_ : TC_R2_) : TC_R_);
-  static constexpr uint32_t A_STAGE = AGG ? AGG_STAGE_BYTES : TC_A_BYTES;
+  static constexpr int R = TWO ? (WIDE ? TC_R2S_ : TC_R2_) : TC_R_;
   static constexpr int Q = TWO ? TC_Q2_ : TC_Q_;
   static constexpr uint32_t BT_BYTES = TWO ? TC_B_BYTES / 2 : TC_B_BYTES;       // one B tile (fp32 hi, or bf16 pairs) of this CTA
   static constexpr int SLABS = (TWO && !WIDE) ? 1 : 4;                          // staging slabs per epilogue warp
   static constexpr uint32_t STAGE_BYTES = 4 * SLABS * TC_SLAB_BYTES;
-  static constexpr uint32_t META_BYTES = AGG ? 2 * AGG_META_TILE_BYTES : 0;      // two tiles of row metadata (AGG kernels)
-  static constexpr uint32_t SMEM_BYTES = R * A_STAGE + Q * 2 * BT_BYTES + STAGE_BYTES + META_BYTES + 1024 /*align*/ + 512 /*barriers*/;
+  static constexpr uint32_t SMEM_BYTES = R * TC_A_BYTES + Q * 2 * BT_BYTES + STAGE_BYTES + 1024 /*align*/ + 512 /*barriers*/;
   static constexpr int A_FULL = 0;                   // [R]  TMA bytes of the raw A tile landed
   static constexpr int R_FREE = A_FULL + R;          // [R]  splitter has read the raw tile (128 arrivals)
   static constexpr int TA_FULL = R_FREE + R;         // [TC_TA] A_hi / A_lo written to TMEM
@@ -347,10 +336,6 @@ __device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap
       "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
       ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(cluster_bar) : "memory");
 }
-__device__ __forceinline__ void bulk_load_1d(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
 __device__ __forceinline__ void cluster_sync_all() {
   asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
   asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
@@ -427,38 +412,23 @@ __device__ __forceinline__ float4 tc_finish4(float4 x, const TcEpilogue& ep, lon
 // leader's MMA warp issues M = 256 instructions for both.  The peer's TMA completes its bytes on the LEADER's B_FULL
 // barrier; splitter and epilogue warps of both CTAs arrive (one lane per warp) on the leader's TA_FULL / ACC_EMPTY; what
 // the MMAs release is a multicast commit to both CTAs.
-// AGG: aggregate-first relational convolution (PyG RGCNConv on K1's window graphs, and its input gradient) in ONE kernel:
-//     out[k] = sum_s ( sum_{e in row k, slot(e) = s} w_e x[col_e] ) W_s  +  x[k] W_root  (+ bias)
-// The transform-first formulation writes Y = x [W_0 | ... | W_root] ([N, (S+1) H]) with one GEMM and reads it back with a
-// gather (3.4 GB of HBM traffic per 2^20 nodes at S = 2, H = 100); here the A operand of the GEMM is PRODUCED by the
-// splitter warps from the x rows of the tile + halo (neighbours of a row are the contiguous window [k - wlo, k + whi]):
-//   * the A producer loads, per 32-column slice c of x, ONE box of 128 + wlo + whi rows (TMA, 128-byte swizzle; rows
-//     before the first / past the last node are zero-filled);
-//   * splitter thread = tile row k keeps its edge list in registers (weights, 4-bit relation slots, first neighbour) and,
-//     per slice and slot, sums the neighbour rows of that slot from the box (conflict-free: consecutive rows sit in
-//     different swizzle positions), splits the sum hi / lo and writes it to tensor memory as K-chunk (c, s);
-//   * K = Kc x (S + 1) x 32 with the weight rows permuted to match (host side); MMA, B ring, epilogue are the pair kernel's.
-// Optional side output zside[N, (S+1) H] = the aggregated rows themselves (for the input-gradient pass these are the dY of
-// the transform-first formulation, which the weight-gradient GEMM consumes).  HBM traffic: x in, out (and zside) out.
-template <int ACT, bool SMALLK, bool ABF16, bool TWO = false, bool ONESLAB = false, bool AGG = false>
+template <int ACT, bool SMALLK, bool ABF16, bool TWO = false, bool ONESLAB = false>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 gemm_tc_nn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmBh,
                   const __grid_constant__ CUtensorMap tmBl, const __grid_constant__ CUtensorMap tmC,
                   float* __restrict__ C, long long ldc, long long M, int N,
                   int K, int bn /* UMMA N for this launch: multiple of 16, <= 128 */, const TcEpilogue ep_in,
                   float* __restrict__ colsum_partial /* [gridDim.x][4][128] column sums of C (N <= 128 only), or NULL */) {
-  using Cfg = NnCfg<TWO, !ONESLAB, AGG>;
-  static_assert(!AGG || (TWO && !SMALLK && ONESLAB && !ABF16), "aggregate-first: pair kernel, one-slab staging");
+  using Cfg = NnCfg<TWO, !ONESLAB>;
   TcEpilogue ep = ep_in;                                   // the device seed word is read ONCE, not per float4 of the epilogue
   if (ACT == ERCG_ACT_RELU_DROPOUT && ep.seed_dev) { ep.seed += *ep.seed_dev; ep.seed_dev = nullptr; }
   static_assert(!TWO || !ABF16, "pair mode: fp32 features");
   static_assert(!ONESLAB || (TWO && !SMALLK), "one-slab staging: pair mode, long K");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* bring = smem + Cfg::R * Cfg::A_STAGE;
+  uint8_t* bring = smem + Cfg::R * TC_A_BYTES;
   uint8_t* stage_all = bring + Cfg::Q * 2 * Cfg::BT_BYTES;          // 1024-byte aligned (every ring is a multiple of 1 KB)
-  uint8_t* meta_all = stage_all + Cfg::STAGE_BYTES;                  // AGG: [2][AGG_META_WORDS][128] words
-  uint64_t* bars = reinterpret_cast<uint64_t*>(meta_all + Cfg::META_BYTES);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(stage_all + Cfg::STAGE_BYTES);
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + Cfg::COUNT);
   const uint32_t bar0 = smem_u32(bars);
   auto BAR = [&](int i) { return bar0 + 8u * i; };
@@ -503,7 +473,7 @@ gemm_tc_nn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   const long long t_first = TWO ? blockIdx.x / 2 : blockIdx.x, t_step = TWO ? gridDim.x / 2 : gridDim.x;
   auto TILE = [&](long long t) { return TWO ? 2 * t + (long long)rank : t; };
   const int n_tiles = (N + bn - 1) / bn;
-  const int k_chunks = (K + TC_BK - 1) / TC_BK;               // AGG: K = Kc * (S + 1) * 32 (host), chunk = (slice c, slot s)
+  const int k_chunks = (K + TC_BK - 1) / TC_BK;
   const bool resident = n_tiles > 1 && k_chunks <= TC_TA;     // A stays in TMEM across the N tiles of an M tile
   const int a_reps = resident ? 1 : n_tiles;                  // A chunk loads per M tile = a_reps * k_chunks
   const uint32_t raw_base = smem_u32(smem), b_base = smem_u32(bring);
@@ -513,30 +483,6 @@ gemm_tc_nn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 
   if (warp == 8) {
     // ------------------------------------------------------------------ A producer (HBM stream)
-    if (AGG) {
-      if (lane == 0) {   // one box of (tile + halo) rows per 32-column slice of x; rows outside [0, M) arrive as zeros
-        uint32_t n = 0;
-        const int slices = k_chunks / (ep.g_S + 1);
-        const uint32_t box_bytes = (uint32_t)ep.g_box_rows * 128u;
-        uint32_t tn = 0;                                            // tiles done by this CTA (metadata buffer parity)
-        for (long long t = t_first; t < m_tiles; t += t_step, ++tn) {
-          const int m0 = (int)TILE(t) * TC_BM;
-          for (int c = 0; c < slices; ++c, ++n) {
-            const int r = n % Cfg::R;
-            TC_TRACE(0, n, 0);
-            mbar_wait_relaxed(BAR(Cfg::R_FREE + r), ((n / Cfg::R) & 1) ^ 1);
-            TC_TRACE(0, n, 1);
-            // slice 0 also brings the tile's row metadata (8 KB, written by rgcn_rowmeta_kernel) into buffer (tile & 1):
-            // the buffer of two tiles ago is free because this stage was last used by the previous tile's slice 0
-            mbar_expect_tx(BAR(Cfg::A_FULL + r), box_bytes + (c == 0 ? AGG_META_TILE_BYTES : 0u));
-            tma_load_2d(raw_base + r * Cfg::A_STAGE, &tmA, c * TC_BK, m0 - ep.g_wlo, BAR(Cfg::A_FULL + r));
-            if (c == 0)
-              bulk_load_1d(smem_u32(meta_all) + (uint32_t)(tn & 1) * AGG_META_TILE_BYTES,
-                           ep.g_meta + (size_t)TILE(t) * (AGG_META_TILE_BYTES / 4), AGG_META_TILE_BYTES, BAR(Cfg::A_FULL + r));
-          }
-        }
-      }
-    } else
     if (lane == 0) {
       uint32_t n = 0;
       for (long long t = t_first; t < m_tiles; t += t_step) {
@@ -548,7 +494,7 @@ gemm_tc_nn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             mbar_wait_relaxed(BAR(Cfg::R_FREE + r), ((n / Cfg::R) & 1) ^ 1);
             TC_TRACE(0, n, 1);
             mbar_expect_tx(BAR(Cfg::A_FULL + r), ABF16 ? TC_A_BYTES / 2 : TC_A_BYTES);
-            tma_load_2d(raw_base + r * Cfg::A_STAGE, &tmA, kc * TC_BK, m0, BAR(Cfg::A_FULL + r));
+            tma_load_2d(raw_base + r * TC_A_BYTES, &tmA, kc * TC_BK, m0, BAR(Cfg::A_FULL + r));
           }
       }
     }
@@ -613,10 +559,8 @@ gemm_tc_nn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           // k-steps that still hold real columns (TMA zero-fills the K tail: K = 100 needs 13 tf32 steps of 8, not 16)
           const uint32_t n_mma = (uint32_t)((nt == n_tiles - 1 ? n_tail : bn) >> 3) << 17;   // pairs: half of it per CTA
           const uint32_t idesc = idesc_base | n_mma, idesc16 = idesc16_base | n_mma;
-          // (AGG: chunk kc is slice kc / (S + 1) of the H input columns -- the last slice of H = 100 holds 4 real columns)
-          const int krem = AGG ? ep.g_H - (kc / (ep.g_S + 1)) * TC_BK : K - kc * TC_BK;
-          const int ks_n = (ep.dbg & 1) ? 0 : min(TC_BK / 8, (krem + 7) >> 3);
-          const int k16_n = (ep.dbg & 1) ? 0 : min(TC_BK / 16, (krem + 15) >> 4);
+          const int ks_n = (ep.dbg & 1) ? 0 : min(TC_BK / 8, (K - kc * TC_BK + 7) >> 3);
+          const int k16_n = (ep.dbg & 1) ? 0 : min(TC_BK / 16, (K - kc * TC_BK + 15) >> 4);
           const uint32_t ah0 = TA_HI(s);
           const uint64_t bh0 = desc_hi | (uint64_t)((B_HI(q) >> 4) & 0x3FFF), b16 = desc_hi | (uint64_t)((B_LO(q) >> 4) & 0x3FFF);
           if (elect_one()) {
@@ -674,131 +618,6 @@ gemm_tc_nn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
     const int row = threadIdx.x;
     const uint32_t lane_addr = (uint32_t)(warp * 32) << 16;
     uint32_t n = 0;
-    if (AGG) {
-      const int S = ep.g_S, slices = k_chunks / (S + 1), wlo = ep.g_wlo, H = ep.g_H;
-      uint32_t an = 0;                                             // K-chunk counter (TMEM A stages)
-      // This row's edge list (degree, offset of the first neighbour, 4-bit relation slots -- 0xF: no message --, weights) comes
-      // from shared memory: rgcn_rowmeta_kernel wrote it once per graph, word-major inside a tile, and the A producer brings
-      // the tile's 8 KB along with slice 0.  (Loading it from the CSR here, edge by edge at the top of every tile, cost a
-      // ~9 600 clk bubble per tile; keeping it, and the next tile's, in registers spilled the accumulators:
-      // profiles/r02w_agg_trace_v1.txt, _v2.txt.)
-      uint32_t tn = 0;
-      // emit one K chunk: (optional) side output of the aggregated 32 columns, hi / lo split, tensor-memory store, arrive
-      auto emit = [&](float (&acc)[32], int sl, int c, int r, long long node, bool last_of_box) {
-        if (ep.g_zside && node < M) {
-          float* z = ep.g_zside + node * ep.g_ldz + (long long)sl * H + c * TC_BK;
-#pragma unroll
-          for (int q = 0; q < 8; ++q)
-            if (c * TC_BK + 4 * q < H)
-              *reinterpret_cast<float4*>(z + 4 * q) = make_float4(acc[4 * q], acc[4 * q + 1], acc[4 * q + 2], acc[4 * q + 3]);
-        }
-        uint32_t hi[32], p16[32];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) {
-          uint32_t l0, l1, l2, l3;
-          split_tf32(acc[4 * q + 0], hi[4 * q + 0], l0);
-          split_tf32(acc[4 * q + 1], hi[4 * q + 1], l1);
-          split_tf32(acc[4 * q + 2], hi[4 * q + 2], l2);
-          split_tf32(acc[4 * q + 3], hi[4 * q + 3], l3);
-          p16[2 * q + 0] = pack_bf16x2(__uint_as_float(hi[4 * q + 0]), __uint_as_float(hi[4 * q + 1]));
-          p16[2 * q + 1] = pack_bf16x2(__uint_as_float(hi[4 * q + 2]), __uint_as_float(hi[4 * q + 3]));
-          p16[16 + 2 * q + 0] = pack_bf16x2(__uint_as_float(l0), __uint_as_float(l1));
-          p16[16 + 2 * q + 1] = pack_bf16x2(__uint_as_float(l2), __uint_as_float(l3));
-        }
-        const int s = an % TC_TA;
-        if (threadIdx.x == 0) TC_TRACE(1, an, 1);
-        mbar_wait(BAR(Cfg::TA_FREE + s), ((an / TC_TA) & 1) ^ 1);
-        if (threadIdx.x == 0) TC_TRACE(1, an, 2);
-        tc_fence_after();
-        tc_st32(TA_HI(s) + lane_addr, hi);
-        tc_st32(TA_HI(s) + 32 + lane_addr, p16);
-        tc_wait_st();
-        if (last_of_box) mbar_arrive(BAR(Cfg::R_FREE + r));         // every load of this box has been consumed
-        tc_fence_before();
-        arrive_leader(LBAR(Cfg::TA_FULL + s));
-        if (threadIdx.x == 0) TC_TRACE(1, an, 3);
-        ++an;
-      };
-      for (long long t = t_first; t < m_tiles; t += t_step, ++tn) {
-        const long long node = TILE(t) * TC_BM + row;
-        const uint32_t mbase = smem_u32(meta_all) + (uint32_t)(tn & 1) * AGG_META_TILE_BYTES + (uint32_t)row * 4u;
-        auto MW = [&](int j) { return __float_as_uint(lds1(mbase + (uint32_t)j * (TC_BM * 4u))); };
-        int deg = 0, d0 = 0;
-        unsigned long long slots = ~0ull;
-        const int lr = row + wlo;                                   // this row inside the box (the box starts wlo rows earlier)
-        for (int c = 0; c < slices; ++c, ++n) {
-          const int r = n % Cfg::R;
-          mbar_wait(BAR(Cfg::A_FULL + r), (n / Cfg::R) & 1);
-          if (c == 0) {                                             // the metadata landed with this box
-            const uint32_t w0 = MW(0);
-            deg = (int)(w0 & 0xFFu);
-            d0 = (int)((w0 >> 8) & 0xFFu) - 64;
-            slots = (unsigned long long)MW(1) | ((unsigned long long)MW(2) << 32);
-          }
-          const uint32_t base = raw_base + r * Cfg::A_STAGE;
-          // relation slots two at a time: ONE pass over the row's edges feeds both accumulators, so for S <= 2 (one-speaker
-          // data) every neighbour row chunk is read from shared memory once per slice -- the floor of this formulation
-          for (int s0 = 0; s0 < S; s0 += 2) {
-            if (threadIdx.x == 0) TC_TRACE(1, an, 0);
-            float a0[32], a1[32];
-#pragma unroll
-            for (int i = 0; i < 32; ++i) a0[i] = a1[i] = 0.f;
-            if (S <= 2) {
-              // one or two relation slots (one-speaker data): every edge feeds this pass -- straight-line code, no votes, so
-              // the loads of the next edge overlap the multiply-adds of this one
-#pragma unroll
-              for (int e = 0; e < AGG_DMAX; ++e) {
-                const int nib = (int)((slots >> (4 * e)) & 0xFull);
-                const float we = __uint_as_float(MW(3 + e));                // 0 past the degree / without a slot
-                const float w0 = nib == 0 ? we : 0.f, w1 = nib == 1 ? we : 0.f;
-                const int rr = (e < deg) ? lr + d0 + e : lr;               // (keep the load inside the box)
-                const uint32_t src = base + (uint32_t)rr * 128u;
-#pragma unroll
-                for (int q = 0; q < 8; ++q) {
-                  const float4 x = lds4(src + ((q ^ (rr & 7)) << 4));
-                  a0[4 * q] = fmaf(w0, x.x, a0[4 * q]); a0[4 * q + 1] = fmaf(w0, x.y, a0[4 * q + 1]);
-                  a0[4 * q + 2] = fmaf(w0, x.z, a0[4 * q + 2]); a0[4 * q + 3] = fmaf(w0, x.w, a0[4 * q + 3]);
-                  a1[4 * q] = fmaf(w1, x.x, a1[4 * q]); a1[4 * q + 1] = fmaf(w1, x.y, a1[4 * q + 1]);
-                  a1[4 * q + 2] = fmaf(w1, x.z, a1[4 * q + 2]); a1[4 * q + 3] = fmaf(w1, x.w, a1[4 * q + 3]);
-                }
-              }
-            } else {
-#pragma unroll
-            for (int e = 0; e < AGG_DMAX; ++e) {
-              const int nib = (int)((slots >> (4 * e)) & 0xFull);
-              const float we = __uint_as_float(MW(3 + e));                  // 0 past the degree / without a slot
-              const float w0 = nib == s0 ? we : 0.f, w1 = nib == s0 + 1 ? we : 0.f;
-              if (__any_sync(0xffffffffu, w0 != 0.f || w1 != 0.f)) {        // warp-uniform: nobody needs this edge in this pass
-                const int rr = (e < deg) ? lr + d0 + e : lr;               // (keep the load inside the box)
-                const uint32_t src = base + (uint32_t)rr * 128u;
-#pragma unroll
-                for (int q = 0; q < 8; ++q) {
-                  const float4 x = lds4(src + ((q ^ (rr & 7)) << 4));
-                  a0[4 * q] = fmaf(w0, x.x, a0[4 * q]); a0[4 * q + 1] = fmaf(w0, x.y, a0[4 * q + 1]);
-                  a0[4 * q + 2] = fmaf(w0, x.z, a0[4 * q + 2]); a0[4 * q + 3] = fmaf(w0, x.w, a0[4 * q + 3]);
-                  a1[4 * q] = fmaf(w1, x.x, a1[4 * q]); a1[4 * q + 1] = fmaf(w1, x.y, a1[4 * q + 1]);
-                  a1[4 * q + 2] = fmaf(w1, x.z, a1[4 * q + 2]); a1[4 * q + 3] = fmaf(w1, x.w, a1[4 * q + 3]);
-                }
-              }
-            }
-            }
-            emit(a0, s0, c, r, node, false);
-            if (s0 + 1 < S) emit(a1, s0 + 1, c, r, node, false);
-          }
-          {                                                         // root slot: the row itself
-            if (threadIdx.x == 0) TC_TRACE(1, an, 0);
-            float a0[32];
-            const uint32_t src = base + (uint32_t)lr * 128u;
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-              const float4 x = lds4(src + ((q ^ (lr & 7)) << 4));
-              a0[4 * q] = x.x; a0[4 * q + 1] = x.y; a0[4 * q + 2] = x.z; a0[4 * q + 3] = x.w;
-            }
-            emit(a0, S, c, r, node, true);
-          }
-        }
-      }
-    } else
     for (long long t = t_first; t < m_tiles; t += t_step) {
       for (int rep = 0; rep < a_reps; ++rep)
         for (int kc = 0; kc < k_chunks; ++kc, ++n) {
@@ -806,7 +625,7 @@ gemm_tc_nn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
           if (threadIdx.x == 0) TC_TRACE(1, n, 0);
           mbar_wait(BAR(Cfg::A_FULL + r), (n / Cfg::R) & 1);          // raw tile landed
           if (threadIdx.x == 0) TC_TRACE(1, n, 1);
-          const uint32_t src = raw_base + r * Cfg::A_STAGE + (ABF16 ? row * 64 : row * 128);
+          const uint32_t src = raw_base + r * TC_A_BYTES + (ABF16 ? row * 64 : row * 128);
           uint32_t hi[32], p16[32];                                // tf32 A_hi | bf16 pairs: [0,16) A_hi, [16,32) A_lo
           if (ABF16) {
             // 64-byte rows, TMA 64-byte swizzle: logical 16-byte chunk c sits at position c ^ ((row >> 1) & 3)
@@ -1804,144 +1623,6 @@ extern "C" int ercg_gemm_nn_tc(const float* A, int64_t lda, const float* B, int6
     rc = finish_launch();
     if (rc) return rc;
     tc_colsum_final_kernel<<<fin_blocks(N), 256, 0, st>>>(partial, grid * 4, 128, N, colsum_out);
-  }
-  return finish_launch();
-}
-
-// ---------------------------------------------------------------------------------------------- aggregate-first RGCN
-
-// Row metadata of the aggregate-first kernels, once per graph and direction: per 128-row tile [AGG_META_WORDS][128] words
-// (word-major, so the splitter threads of the main kernel read it from shared memory without bank conflicts):
-//   word 0: degree | (first neighbour - row + 64) << 8;  words 1-2: 4-bit relation slot of edge e (0xF: no message);
-//   words 3..13: weight of edge e (0 past the degree or without a slot).
-namespace ercg {
-__global__ void __launch_bounds__(128)
-rgcn_rowmeta_kernel(const int* __restrict__ rowptr, const int* __restrict__ col, const unsigned char* __restrict__ etype,
-                    const int* __restrict__ eid, const int* __restrict__ rel_slot, const float* __restrict__ w, int S,
-                    long long N, float* __restrict__ meta) {
-  const long long tile = blockIdx.x, node = tile * TC_BM + threadIdx.x;
-  uint32_t* out = reinterpret_cast<uint32_t*>(meta) + tile * (AGG_META_WORDS * TC_BM) + threadIdx.x;
-  int deg = 0, d0 = 0;
-  unsigned long long slots = ~0ull;
-  float wg[AGG_DMAX];
-#pragma unroll
-  for (int e = 0; e < AGG_DMAX; ++e) wg[e] = 0.f;
-  if (node < N) {
-    const int beg = rowptr[node];
-    deg = rowptr[node + 1] - beg;
-    if (deg > AGG_DMAX) deg = AGG_DMAX;
-    if (deg > 0) d0 = col[beg] - (int)node;
-#pragma unroll
-    for (int e = 0; e < AGG_DMAX; ++e) {
-      const int ee = beg + (e < deg ? e : 0);                     // clamped: branch-free, all loads in flight together
-      int tt = (etype && deg > 0) ? (int)etype[ee] : 0;
-      if (rel_slot) tt = __ldg(rel_slot + tt);
-      const float wv = (w && deg > 0) ? w[eid ? eid[ee] : ee] : 1.f;
-      const bool on = e < deg && tt >= 0 && tt < S;
-      wg[e] = on ? wv : 0.f;
-      slots = (slots & ~(0xFull << (4 * e))) | ((on ? (unsigned long long)tt : 0xFull) << (4 * e));
-    }
-  }
-  out[0] = (uint32_t)deg | ((uint32_t)(d0 + 64) << 8);
-  out[TC_BM] = (uint32_t)slots;
-  out[2 * TC_BM] = (uint32_t)(slots >> 32);
-#pragma unroll
-  for (int e = 0; e < AGG_DMAX; ++e) out[(3 + e) * TC_BM] = __float_as_uint(wg[e]);
-  out[14 * TC_BM] = 0u;
-  out[15 * TC_BM] = 0u;
-}
-}  // namespace ercg
-
-static size_t rgcn_window_gemm_ws(int Nout, int K, int S) {
-  return (ercg_gemm_nn_tc_workspace_bytes(Nout, (K + TC_BK - 1) / TC_BK * TC_BK * (S + 1)) + 255) & ~(size_t)255;
-}
-extern "C" size_t ercg_rgcn_window_workspace_bytes(int64_t N, int Nout, int K, int S) {
-  if (N <= 0 || Nout <= 0 || K <= 0 || S < 0) return 0;
-  return rgcn_window_gemm_ws(Nout, K, S) + (size_t)(((N + TC_BM - 1) / TC_BM + 1) & ~1LL) * AGG_META_TILE_BYTES + 256;   // whole tile PAIRS
-}
-
-extern "C" int ercg_rgcn_window_supported(const float* x, int64_t ldx, const float* out, int64_t ldo, int64_t N, int K,
-                                          int Nout, int S, int wlo, int whi) {
-  if (N < 1 || K < 1 || Nout < 1 || Nout > TC_BN || S < 0 || S > 14 || wlo < 0 || whi < 0) return 0;
-  if (wlo + whi + 1 > AGG_DMAX || (TC_BM + wlo + whi) * 128 > (int)AGG_STAGE_BYTES) return 0;
-  if (K <= 3 * TC_BK) return 0;          // >= 4 column slices per tile: the two metadata buffers rely on it (see the A producer)
-  if ((ldx & 3) || (ldo & 3) || !aligned16(x) || !aligned16(out) || N >= 2147483647LL) return 0;
-  if ((N + TC_BM - 1) / TC_BM < 2 * (kNumSMs / 2) || !nn_pairs_enabled()) return 0;    // pairs only, machine-filling sizes
-  return nn_pair_capacity() >= kNumSMs / 2 - 8 ? 1 : 0;
-}
-
-extern "C" int ercg_rgcn_window(const float* x, int64_t ldx, const int32_t* rowptr, const int32_t* col, const uint8_t* etype,
-                                const int32_t* eid, const int32_t* rel_slot, const float* w, int S, const float* Wp,
-                                int64_t ldw, const float* bias, float* out, int64_t ldo, float* zside, int64_t ldz,
-                                float* colsum_out, int64_t N, int K, int Nout, int wlo, int whi, void* workspace,
-                                size_t workspace_bytes, void* stream) {
-  if (!x || !rowptr || !col || !Wp || !out || ldx < K || ldw < Nout || ldo < Nout) return ERCG_EINVAL;
-  if (!ercg_rgcn_window_supported(x, ldx, out, ldo, N, K, Nout, S, wlo, whi)) return ERCG_EINVAL;
-  if ((bias && !aligned16(bias)) || (zside && ((ldz & 3) || !aligned16(zside) || ldz < (int64_t)(S + 1) * K)) || (K & 3))
-    return ERCG_EALIGN;
-  if (colsum_out && bias) return ERCG_EINVAL;
-  if (workspace_bytes < ercg_rgcn_window_workspace_bytes(N, Nout, K, S) || !workspace) return ERCG_EWORKSPACE;
-  cudaStream_t st = (cudaStream_t)stream;
-  const int slices = (K + TC_BK - 1) / TC_BK;
-  const long long row_tiles = ((N + TC_BM - 1) / TC_BM + 1) & ~1LL;      // whole tile pairs: the idle half of the last pair reads degree 0
-  float* meta = reinterpret_cast<float*>(((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255)) + rgcn_window_gemm_ws(Nout, K, S));
-  rgcn_rowmeta_kernel<<<(unsigned)row_tiles, 128, 0, st>>>(rowptr, col, etype, eid, etype ? rel_slot : nullptr, w, S, N, meta);
-  if (int rc0 = finish_launch()) return rc0;
-  const int Keff = slices * (S + 1) * TC_BK, Kc = Keff / TC_BK;
-  float* bhi = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-  __nv_bfloat16* b16 = reinterpret_cast<__nv_bfloat16*>(
-      (reinterpret_cast<uintptr_t>(bhi + (size_t)Nout * Keff) + 255) & ~uintptr_t(255));
-  split_bt_kernel<<<dim3(Kc, (Nout + 31) / 32), dim3(32, 8), 0, st>>>(Wp, ldw, Keff, Nout, Keff, Kc, bhi, b16);
-  int rc = finish_launch();
-  if (rc) return rc;
-  const int bn = (Nout + PAIR_N_GRAN - 1) / PAIR_N_GRAN * PAIR_N_GRAN;
-  const int box_rows = TC_BM + wlo + whi;
-  CUtensorMap tmA, tmBh, tmBl, tmC;
-  if (!make_map(&tmA, x, N, K, ldx, box_rows) || !make_map(&tmBh, bhi, Nout, Keff, Keff, bn / 2) ||
-      !make_map_b16(&tmBl, b16, Nout, Kc, bn / 2) || !make_map(&tmC, out, N, Nout, ldo, 32))
-    return ERCG_ECUDA;
-  auto kern = gemm_tc_nn_kernel<0, false, false, true, true, true>;
-  constexpr uint32_t smem = NnCfg<true, false, true>::SMEM_BYTES;
-  static DeviceOnce attr_set;
-  if (attr_set.need()) {
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return ERCG_ECUDA;
-    attr_set.mark();
-  }
-  const int pair_cap = nn_pair_capacity();
-  const int grid = 2 * pair_cap;
-  TcEpilogue ep{bias, ERCG_ACT_NONE, nullptr, 0, 1.f, 0.f, 0ull, 0, nullptr};
-#ifdef ERCG_TRACE
-  if (getenv("ERCG_TC_TRACE") && atoi(getenv("ERCG_TC_TRACE")) == 4) {          // trace the aggregate-first kernel (diagnostics build)
-    if (!trace_buf && cudaMalloc(&trace_buf, sizeof(long long) * TR_ROLES * TR_N * 4) != cudaSuccess) trace_buf = nullptr;
-    if (trace_buf) cudaMemsetAsync(trace_buf, 0, sizeof(long long) * TR_ROLES * TR_N * 4, st);
-    ep.trace = trace_buf;
-  }
-#endif
-  ep.g_rowptr = rowptr; ep.g_col = col; ep.g_etype = etype; ep.g_eid = eid; ep.g_rel_slot = etype ? rel_slot : nullptr;
-  ep.g_w = w; ep.g_zside = zside; ep.g_ldz = ldz; ep.g_S = S; ep.g_wlo = wlo; ep.g_box_rows = box_rows; ep.g_H = K;
-  ep.g_meta = meta;
-  float* partial = colsum_out ? reinterpret_cast<float*>(b16 + (size_t)Nout * Kc * 64) : nullptr;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid, 1, 1);
-  cfg.blockDim = dim3(TC_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  const long long ldc_ll = ldo, M_ll = N;
-  if (cudaLaunchKernelEx(&cfg, kern, tmA, tmBh, tmBl, tmC, out, ldc_ll, M_ll, Nout, Keff, bn, ep, partial) != cudaSuccess) {
-    cudaGetLastError();
-    return ERCG_ECUDA;
-  }
-  if (colsum_out) {
-    rc = finish_launch();
-    if (rc) return rc;
-    tc_colsum_final_kernel<<<fin_blocks(Nout), 256, 0, st>>>(partial, grid * 4, 128, Nout, colsum_out);
   }
   return finish_launch();
 }

@@ -323,89 +323,6 @@ def gather(Y, graph, H, R, w=None, bias=None, root_off=-1, use_types=True, rel_s
     return _Gather.apply(Y, w, bias, graph, H, R, root_off, use_types, rel_slot)
 
 
-# ------------------------------------------------------------------------------------------- aggregate-first RGCN
-# Aggregate-first RGCNConv in ONE tensor-core kernel per direction (ercg_rgcn_window).  Parity-green (tests/test_gpu_ops.py)
-# and 4x fewer HBM bytes than transform-first, but MEASURED SLOWER on B200 (1.17 vs 0.92 ms per direction at 2^20 nodes,
-# step 11.54 vs 11.32 ms: the four splitter warps that form the aggregated A operand are the bottleneck -- DESIGN.md 5), so
-# it is off by default; set True to use it.
-RGCN_FUSED = False
-
-
-def _rgcn_permuted_weights(blocks, K):
-    """[S+1] matrices [K, Nout] -> Wp [(S+1) * Kc * 32, Nout]: row ((c * (S+1) + s) * 32 + kk) = W_s[32 c + kk] (zero past K)."""
-    S1, Nout = len(blocks), blocks[0].size(1)
-    Kc = (K + 31) // 32
-    Wall = torch.zeros((S1, Kc * 32, Nout), dtype=torch.float32, device=blocks[0].device)
-    for i, b in enumerate(blocks):
-        Wall[i, :K] = b
-    return Wall.view(S1, Kc, 32, Nout).permute(1, 0, 2, 3).reshape(Kc * S1 * 32, Nout).contiguous()
-
-
-def rgcn_window_supported(x, graph, K, H, S):
-    """True when RGCNConv on this K1 window graph can run as ONE aggregate-first tensor-core kernel (ercg_rgcn_window)."""
-    if not RGCN_FUSED or GEMM_ENGINE != "tc" or x.dim() != 2 or getattr(graph, "inv_cnt", None) is None:
-        return False
-    win = _window(graph, H)
-    if win is None or (K & 3) or (H & 3):
-        return False
-    xx, ldx = _rows(x)
-    return bool(lib().ercg_rgcn_window_supported(_p(xx), ldx, _p(xx), H, xx.size(0), K, H, S, win[0], win[1]) and
-                lib().ercg_rgcn_window_supported(_p(xx), H, _p(xx), ldx, xx.size(0), H, K, S, win[1], win[0]))
-
-
-class _RgcnWindow(torch.autograd.Function):
-    """out = sum_s mean_{N_s}(x) W_s + x W_root + b as one kernel per direction (include/ercgraph.h: ercg_rgcn_window).
-
-    forward : by-destination CSR, weights inv_cnt                                   -> out
-    backward: by-source CSR (t_*), the same weights through t_eid                    -> dx, and as a side output the
-              aggregated dout rows dY [N, (S+1) H] = what ercg_gather_bwd produces;   dWcat = x^T dY (ercg_gemm_tn_tc)"""
-
-    @staticmethod
-    def forward(ctx, x, wrel, root, bias, graph, rel_slot):
-        x, ldx = _rows(x)
-        N, K = x.shape
-        S, H = wrel.size(0), wrel.size(2)
-        wf, wp = _window(graph, H)
-        Wp = _rgcn_permuted_weights([wrel[i] for i in range(S)] + [root], K)
-        out = torch.empty((N, H), dtype=torch.float32, device=x.device)
-        ws = _ws(lib().ercg_rgcn_window_workspace_bytes(N, H, K, S), x.device)
-        check(lib().ercg_rgcn_window(_p(x), ldx, _p(graph.rowptr), _p(graph.col), _p(graph.etype), None, _p(rel_slot),
-                                     _p(graph.inv_cnt), S, _p(Wp), H, _p(bias), _p(out), H, None, 0, None, N, K, H, wf, wp,
-                                     _p(ws), ws.numel(), _stream()), "ercg_rgcn_window")
-        ctx.graph, ctx.rel_slot, ctx.has_bias = graph, rel_slot, bias is not None
-        ctx.save_for_backward(x, wrel, root)
-        return out
-
-    @staticmethod
-    def backward(ctx, dout):
-        x, wrel, root = ctx.saved_tensors
-        g = ctx.graph
-        dout, ldo = _rows(dout.contiguous())
-        N, K = x.shape
-        S, H = wrel.size(0), wrel.size(2)
-        wf, wp = _window(g, H)
-        WpT = _rgcn_permuted_weights([wrel[i].t() for i in range(S)] + [root.t()], H)          # [.., K]
-        dx = torch.empty((N, K), dtype=torch.float32, device=x.device)
-        dY = torch.empty((N, (S + 1) * H), dtype=torch.float32, device=x.device)
-        cs = torch.empty(K, dtype=torch.float32, device=x.device)
-        ws = _ws(lib().ercg_rgcn_window_workspace_bytes(N, K, H, S), x.device)
-        check(lib().ercg_rgcn_window(_p(dout), ldo, _p(g.t_rowptr), _p(g.t_col), _p(g.t_etype), _p(g.t_eid), _p(ctx.rel_slot),
-                                     _p(g.inv_cnt), S, _p(WpT), K, None, _p(dx), K, _p(dY), dY.stride(0), _p(cs), N, H, K,
-                                     wp, wf, _p(ws), ws.numel(), _stream()), "ercg_rgcn_window (input gradient)")
-        _tag_set(dx, "_ercg_colsum", cs)                  # bias gradient of the producing Linear, as gemm_nn(want_colsum)
-        dWcat = gemm_tn(x, dY)                            # [K, (S+1) H]
-        dwrel = dWcat[:, :S * H].reshape(K, S, H).permute(1, 0, 2)
-        droot = dWcat[:, S * H:]
-        dbias = colsum(dout) if ctx.has_bias else None
-        return dx, dwrel, droot, dbias, None, None
-
-
-def rgcn_window(x, wrel, root, bias, graph, rel_slot=None):
-    """RGCNConv (mean aggregation, root weight, bias) on a K1 window graph: wrel [S, K, H] are the relation weights of the
-    slots the layer uses (rel_slot maps relation ids to them, None = identity), root [K, H]."""
-    return _RgcnWindow.apply(x, wrel, root, bias, graph, rel_slot)
-
-
 # ------------------------------------------------------------------------------------------- K4 attention
 def _window(graph, H):
     """(wf, wp) when ``graph`` is a K1 window graph the tiled attention kernels support, else None."""

@@ -69,14 +69,9 @@ class RGCNConv(nn.Module):
             P = len(ids)
             sel = g.relation_sel()
             wrel = self.weight.index_select(0, sel)
-            if ops.rgcn_window_supported(x, g, self.in_channels, H, P):
-                # aggregate-first in ONE kernel per direction: Y = x [W_0 | ... | W_root] is never written
-                return ops.rgcn_window(x, wrel, self.root, self.bias, g, rel_slot)
             wcat = torch.cat([wrel.permute(1, 0, 2).reshape(self.in_channels, P * H), self.root], dim=1)
             y = ops.matmul_kn(x, wcat)
             return ops.gather(y, g, H, R, w=g.mean_weight(), bias=self.bias, root_off=P * H, rel_slot=rel_slot, n_slots=P)
-        if g.num_relations == R and ops.rgcn_window_supported(x, g, self.in_channels, H, R):
-            return ops.rgcn_window(x, self.weight, self.root, self.bias, g, None)
         wcat = torch.cat([self.weight.permute(1, 0, 2).reshape(self.in_channels, R * H), self.root], dim=1)
         y = ops.matmul_kn(x, wcat)
         return ops.gather(y, g, H, R, w=g.mean_weight(), bias=self.bias, root_off=R * H)

@@ -222,26 +222,6 @@ int ercg_gather_bwd(const float* dout, int64_t ldo, const float* Y, int64_t ldy,
                     const int32_t* t_rowptr, const int32_t* t_col, const uint8_t* t_etype,
                     const int32_t* t_eid, const int32_t* rel_slot, const float* w, int R, int root_off,
                     float* dY, int64_t lddy, float* dw, int64_t N, int H, void* stream);
-/* Aggregate-first relational convolution on window graphs in ONE tensor-core kernel (PyG RGCNConv, aggr = 'mean',
- * cogmen.py:65,71 -- and, with the by-source arrays, its input gradient):
- *     out[k, :] = sum_s ( sum_{e in row k, slot(e) = s} w[wid(e)] x[col[e], :] ) @ W_s  +  x[k, :] @ W_root  (+ bias)
- * The transform-first formulation (ercg_gemm_nn_tc + ercg_gather_fwd) writes Y = x [W_0 | ... | W_root] and reads it back;
- * here the aggregated rows are produced inside the GEMM from the x rows of the tile + halo and never touch HBM.
- * rowptr / col / etype: CSR by row of a graph whose row k has the contiguous ascending neighbours [k - wlo, k + whi] clipped to
- * its dialogue (by destination: wlo = wf, whi = wp of batch_graphify; by source: wlo = wp, whi = wf); rel_slot: relation id ->
- * slot in [0, S) or -1 (no message), NULL = identity; w: edge weights (NULL = 1) indexed by eid[e] when eid is given (the
- * by-source traversal passes t_eid) else by e.  Wp [(S + 1) * Kc * 32, Nout], Kc = ceil(K / 32): row ((c * (S + 1) + s) * 32 + kk)
- * = W_s[32 c + kk, :] (s = S: W_root; rows with 32 c + kk >= K are zero).  zside (optional) [N, (S + 1) * K]: the aggregated rows
- * themselves, root slot = x (the dY of the transform-first backward: ercg_gather_bwd's output).  colsum_out (optional, no bias):
- * column sums of out.  Needs CTA pairs, >= 148 row tiles, 96 < K, Nout <= 128, wlo + whi <= 10: ercg_rgcn_window_supported says
- * whether this launch can run (callers fall back to ercg_gemm_nn_tc + ercg_gather_fwd / _bwd). */
-size_t ercg_rgcn_window_workspace_bytes(int64_t N, int Nout, int K, int S);
-int ercg_rgcn_window_supported(const float* x, int64_t ldx, const float* out, int64_t ldo, int64_t N, int K, int Nout, int S,
-                               int wlo, int whi);
-int ercg_rgcn_window(const float* x, int64_t ldx, const int32_t* rowptr, const int32_t* col, const uint8_t* etype,
-                     const int32_t* eid, const int32_t* rel_slot, const float* w, int S, const float* Wp, int64_t ldw,
-                     const float* bias, float* out, int64_t ldo, float* zside, int64_t ldz, float* colsum_out, int64_t N, int K,
-                     int Nout, int wlo, int whi, void* workspace, size_t workspace_bytes, void* stream);
 /* Backward on window graphs (every graph ercg_graphify_csr builds: the destinations of source j lie in [j - wlo, j + whi],
  * wlo = wp, whi = wf of batch_graphify; same limits as ercg_attn_window_supported): a CTA stages the dout rows around its 32
  * sources in shared memory.  n_slots = relation slots of dY (P with rel_slot, R without).  No dw (use ercg_gather_bwd when
