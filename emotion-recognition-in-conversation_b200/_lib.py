@@ -98,6 +98,7 @@ SIGNATURES = {
     "ercg_sumsq_workspace_bytes": (SZ, [L]),
     "ercg_sumsq": (I, [P, L, P, P, SZ, P]),
     "ercg_adam_step": (I, [P, P, P, P, L, F, F, F, F, F, I, F, P, F, P, P]),
+    "ercg_adam_step_guarded": (I, [P, P, P, P, L, F, F, F, F, F, I, F, P, F, P, P, P]),
     # peer-memory all-reduce (csrc/p2p.cu)
     "ercg_p2p_region_bytes": (SZ, [SZ]),
     "ercg_p2p_alloc": (I, [SZ, P, P]),
@@ -105,6 +106,7 @@ SIGNATURES = {
     "ercg_p2p_close": (I, [P]),
     "ercg_p2p_free": (I, [P]),
     "ercg_p2p_status": (I, [P, P]),
+    "ercg_p2p_status_word": (I, [P, P]),
     "ercg_p2p_allreduce": (I, [P, I, I, P, P, L, I, SZ, P]),
     "ercg_p2p_bn_stats": (I, [P, I, I, P, L, L, I, D, P, P, P, P, P, F, P, SZ, SZ, P]),
     "ercg_p2p_bn_act_bwd_reduce": (I, [P, I, I, P, L, P, L, P, P, F, P, P, F, P, P, L, I, P, SZ, SZ, P]),
@@ -174,7 +176,7 @@ class _Timed:
         fn = getattr(self._h, name)
         if name.endswith("_bytes") or name.endswith("_supported") or name.endswith("_tiles") or name in ("ercg_strerror", "ercg_version", "ercg_launch_count",
                                                "ercg_graphify_sizes_host", "ercg_p2p_alloc", "ercg_p2p_open", "ercg_p2p_close",
-                                               "ercg_p2p_free", "ercg_p2p_status"):
+                                               "ercg_p2p_free", "ercg_p2p_status", "ercg_p2p_status_word"):
             setattr(self, name, fn)
             return fn
 

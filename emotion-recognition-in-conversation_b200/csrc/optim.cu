@@ -55,7 +55,11 @@ __device__ __forceinline__ float adam_one(float p, float g, float& m, float& v, 
   return p - (a.lr / c1) * (m / denom);                        // param.addcdiv_(exp_avg, denom, value=-lr / bias_correction1)
 }
 
-__global__ void __launch_bounds__(256) adam_kernel(AdamArgs a) {
+// GUARDED (ercg_adam_step_guarded): every thread returns before touching p, m, v when *skip != 0 -- the status word of a
+// peer-memory exchange that timed out, so a garbage-summed gradient is never applied.  The arithmetic is the same either way.
+template <bool GUARDED>
+__global__ void __launch_bounds__(256) adam_kernel(AdamArgs a, const int* __restrict__ skip) {
+  if (GUARDED && *skip != 0) return;
   const long long t = a.step[0] + 1;                           // the counter is bumped by a SEPARATE launch after this one
   const float c1 = (float)(1.0 - pow((double)a.beta1, (double)t));          // bias corrections in double, like torch.optim
   const float c2s = (float)sqrt(1.0 - pow((double)a.beta2, (double)t));
@@ -84,7 +88,36 @@ __global__ void __launch_bounds__(256) adam_kernel(AdamArgs a) {
   }
 }
 // separate single-thread launch: bumping the counter inside adam_kernel would race with blocks that have not read it yet
-__global__ void step_bump_kernel(long long* step) { step[0] += 1; }
+template <bool GUARDED>
+__global__ void step_bump_kernel(long long* step, const int* __restrict__ skip) {
+  if (GUARDED && *skip != 0) return;
+  step[0] += 1;
+}
+
+template <bool GUARDED>
+int adam_launch(const AdamArgs& a, const int* skip, cudaStream_t stream) {
+  if (a.n > 0) {
+    long long want = (a.n / 4 + 255) / 256;
+    const long long cap = 8LL * device_sm_count();
+    const int nb = (int)(want < 1 ? 1 : (want > cap ? cap : want));
+    adam_kernel<GUARDED><<<nb, 256, 0, stream>>>(a, skip);
+    int rc = finish_launch();
+    if (rc) return rc;
+  }
+  step_bump_kernel<GUARDED><<<1, 1, 0, stream>>>(a.step, skip);
+  return finish_launch();
+}
+
+int adam_args(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2, float eps,
+              float weight_decay, int decoupled, float grad_scale, const float* sumsq, float max_norm, int64_t* step_dev,
+              AdamArgs* a) {
+  if (n < 0 || !step_dev) return ERCG_EINVAL;
+  if (n > 0 && (!p || !g || !m || !v)) return ERCG_EINVAL;
+  if (!(beta1 >= 0.f && beta1 < 1.f) || !(beta2 >= 0.f && beta2 < 1.f) || !(eps >= 0.f)) return ERCG_EINVAL;
+  *a = AdamArgs{p, g, m, v, (long long)n, lr, beta1, beta2, eps, weight_decay, decoupled, grad_scale, sumsq, max_norm,
+                reinterpret_cast<long long*>(step_dev)};
+  return ERCG_OK;
+}
 
 }  // namespace ercg
 
@@ -111,19 +144,19 @@ extern "C" int ercg_sumsq(const float* x, int64_t n, float* out, void* workspace
 extern "C" int ercg_adam_step(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
                               float eps, float weight_decay, int decoupled, float grad_scale, const float* sumsq,
                               float max_norm, int64_t* step_dev, void* stream) {
-  if (n < 0 || !step_dev) return ERCG_EINVAL;
-  if (n > 0 && (!p || !g || !m || !v)) return ERCG_EINVAL;
-  if (!(beta1 >= 0.f && beta1 < 1.f) || !(beta2 >= 0.f && beta2 < 1.f) || !(eps >= 0.f)) return ERCG_EINVAL;
-  AdamArgs a{p, g, m, v, (long long)n, lr, beta1, beta2, eps, weight_decay, decoupled, grad_scale, sumsq, max_norm,
-             reinterpret_cast<long long*>(step_dev)};
-  if (n > 0) {
-    long long want = (n / 4 + 255) / 256;
-    const long long cap = 8LL * device_sm_count();
-    const int nb = (int)(want < 1 ? 1 : (want > cap ? cap : want));
-    adam_kernel<<<nb, 256, 0, (cudaStream_t)stream>>>(a);
-    int rc = finish_launch();
-    if (rc) return rc;
-  }
-  step_bump_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(reinterpret_cast<long long*>(step_dev));
-  return finish_launch();
+  AdamArgs a;
+  const int rc = adam_args(p, g, m, v, n, lr, beta1, beta2, eps, weight_decay, decoupled, grad_scale, sumsq, max_norm, step_dev, &a);
+  return rc ? rc : adam_launch<false>(a, nullptr, (cudaStream_t)stream);
+}
+
+// The data-parallel trainer's step after a peer-memory gradient all-reduce (train_mm.py under torchrun): skip_if_nonzero is
+// that communicator's sticky status word (ercg_p2p_status_word), so once an exchange has timed out no update is applied.
+extern "C" int ercg_adam_step_guarded(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1,
+                                      float beta2, float eps, float weight_decay, int decoupled, float grad_scale,
+                                      const float* sumsq, float max_norm, int64_t* step_dev, void* stream,
+                                      const int* skip_if_nonzero) {
+  if (!skip_if_nonzero) return ERCG_EINVAL;
+  AdamArgs a;
+  const int rc = adam_args(p, g, m, v, n, lr, beta1, beta2, eps, weight_decay, decoupled, grad_scale, sumsq, max_norm, step_dev, &a);
+  return rc ? rc : adam_launch<true>(a, skip_if_nonzero, (cudaStream_t)stream);
 }

@@ -161,6 +161,14 @@ extern "C" int ercg_p2p_status(const void* region, int* status_host) {
   return cudaMemcpy(status_host, &h->status, sizeof(int), cudaMemcpyDeviceToHost) == cudaSuccess ? ERCG_OK : ERCG_ECUDA;
 }
 
+// The device address of the same word, for kernels that must not consume the result of a failed exchange
+// (ercg_adam_step_guarded).  No synchronisation: the word lives in this rank's own region.
+extern "C" int ercg_p2p_status_word(void* region, int** status_dev) {
+  if (!region || !status_dev) return ERCG_EINVAL;
+  *status_dev = &reinterpret_cast<P2pHeader*>(region)->status;
+  return ERCG_OK;
+}
+
 extern "C" int ercg_p2p_allreduce(void* const* regions_dev, int rank, int world, const void* in, void* out, int64_t n,
                                   int dtype, size_t max_bytes, void* stream) {
   if (!regions_dev || world < 1 || world > P2P_MAX_WORLD || rank < 0 || rank >= world || n < 0 || (dtype != 0 && dtype != 1))

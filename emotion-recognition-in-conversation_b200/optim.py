@@ -30,6 +30,9 @@ class FlatAdam:
         self.live = None
         self.flat_p = self.flat_g = self.m = self.v = self.step_dev = None
         self.grad_scale = 1.0
+        # device address of an int (a PeerComm's status word): when set, update() runs ercg_adam_step_guarded, which leaves
+        # p, m, v and the step counter untouched while that int is non-zero
+        self.skip_if_nonzero = None
 
     # ---- one-time layout, decided after the first backward (only then is it known which parameters are live)
     def attach(self, order=None):
@@ -92,10 +95,13 @@ class FlatAdam:
             check(lib().ercg_sumsq(_p(self.flat_g), self.n, _p(self._sumsq), _p(self._sumsq_ws), self._sumsq_ws.numel(), _stream()),
                   "ercg_sumsq")
             sumsq = self._sumsq
-        check(lib().ercg_adam_step(_p(self.flat_p), _p(self.flat_g), _p(self.m), _p(self.v), self.n, self.lr, self.betas[0],
-                                   self.betas[1], self.eps, self.weight_decay, 1 if self.decoupled else 0, float(self.grad_scale),
-                                   _p(sumsq), float(self.max_norm if self.max_norm is not None else 0.0), _p(self.step_dev),
-                                   _stream()), "ercg_adam_step")
+        args = (_p(self.flat_p), _p(self.flat_g), _p(self.m), _p(self.v), self.n, self.lr, self.betas[0], self.betas[1], self.eps,
+                self.weight_decay, 1 if self.decoupled else 0, float(self.grad_scale), _p(sumsq),
+                float(self.max_norm if self.max_norm is not None else 0.0), _p(self.step_dev), _stream())
+        if self.skip_if_nonzero is None:
+            check(lib().ercg_adam_step(*args), "ercg_adam_step")
+        else:
+            check(lib().ercg_adam_step_guarded(*args, self.skip_if_nonzero), "ercg_adam_step_guarded")
 
     def step(self, allreduce=None):
         """gather -> [allreduce(flat gradient buffer)] -> update.  ``allreduce``: callable taking the flat tensor."""

@@ -111,6 +111,12 @@ class PeerComm:
         check(lib().ercg_p2p_status(self._own, ctypes.byref(st)), "ercg_p2p_status")
         return st.value
 
+    def status_word(self):
+        """Device address of this rank's sticky status word (for FlatAdam.skip_if_nonzero / ercg_adam_step_guarded)."""
+        ptr = ctypes.c_void_p()
+        check(lib().ercg_p2p_status_word(self._own, ctypes.byref(ptr)), "ercg_p2p_status_word")
+        return ptr.value
+
     def check(self):
         st = self.status()
         if st != 0:

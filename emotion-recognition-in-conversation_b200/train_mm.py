@@ -17,6 +17,17 @@ What is different
   * ``mmdatasets`` (the reference's feature pickles) is not part of this repo: ``--data=<file>`` loads a pickle
     ``{"train": [sample, ...], "test": [...]}`` of samples in the reference's format (mmbase.py:374-384); without it a seeded
     synthetic data set of the data set's SHAPE is generated (``--train_dialogues``, ``--test_dialogues``).
+
+Several GPUs (the reference's ``accelerate launch --num_processes N``, lumo/trainer/trainer.py:62-64,315-327)::
+
+    python -m torch.distributed.run --standalone --nproc_per_node N train_mm.py --module=dgcn ...
+
+One process per GPU (WORLD_SIZE / RANK / LOCAL_RANK; rank r runs on cuda:LOCAL_RANK, ``--device`` is ignored), with DDP's
+semantics: ``--train.batch_size`` is the per-GPU batch, optimizer step s trains rank r on batch s*N + r of the epoch's list
+(``deal_batches``), every rank takes the mean loss of its own batch and the update uses the average of the N gradients
+(one all-reduce of the flat gradient buffer: libercgraph's peer-memory kernel, else NCCL), BatchNorm running statistics are
+rank 0's.  The test pass is split over the ranks batch by batch and gathered back into the one-GPU order; only rank 0 logs
+and writes checkpoints.  Without WORLD_SIZE (or with 1) nothing of this runs.
 """
 import json
 import math
@@ -153,6 +164,43 @@ def load_data(p):
             "synthetic (%s shape: t=%d a=%d v=%d)" % (p["dataset"], p["hidden_text"], p["hidden_audio"], p["hidden_visual"]))
 
 
+# ------------------------------------------------------------------------------------------------ data parallelism
+def init_distributed(p, log=print):
+    """The torchrun environment (as bench.py reads it): WORLD_SIZE, RANK, LOCAL_RANK.  Returns (rank, world).  With
+    WORLD_SIZE unset or 1 nothing is touched; otherwise p["device"] becomes LOCAL_RANK and the NCCL process group is
+    initialised on that device (the caller destroys it)."""
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if world <= 1:
+        return 0, 1
+    import torch.distributed as dist
+    rank, local = int(os.environ["RANK"]), int(os.environ.get("LOCAL_RANK", "0"))
+    if rank == 0:
+        log("train_mm: %d processes; each runs on cuda:LOCAL_RANK, --device=%s is ignored" % (world, p["device"]))
+    p["device"] = local
+    dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    return rank, world
+
+
+def deal_batches(n_batches, world):
+    """Per optimizer step, the index of the batch each rank trains on: step s takes batches s*W .. s*W+W-1 of the epoch's
+    list and rank r the (s*W + r)-th (accelerate's BatchSamplerShard with split_batches=False).  A last round the list does
+    not fill is completed with batches from its start (even_batches=True).  world = 1: [[0], [1], ...]."""
+    steps = (n_batches + world - 1) // world
+    return [[(s * world + r) % n_batches for r in range(world)] for s in range(steps)]
+
+
+def shard_test_batches(n_batches, rank, world):
+    """The test batches ``rank`` evaluates: r, r+W, r+2W, ... of the one-GPU batch list (each keeps its one-GPU composition
+    and padding, which the unpacked reverse LSTMs of dgcnv2 / MMGCN run over)."""
+    return list(range(rank, n_batches, world))
+
+
+def restore_order(per_rank):
+    """per_rank[r] = the results of rank r's batches (shard_test_batches) -> the results in the one-GPU batch order."""
+    world = len(per_rank)
+    return [per_rank[i % world][i // world] for i in range(sum(len(x) for x in per_rank))]
+
+
 # ------------------------------------------------------------------------------------------------ trainer
 DGCN_LOSS_WEIGHTS = [1 / 0.086747, 1 / 0.144406, 1 / 0.227883, 1 / 0.160585, 1 / 0.127711, 1 / 0.252668]      # dgcn.py:109-110
 
@@ -180,10 +228,12 @@ def build_model(p, dev):
 
 
 class Trainer:
-    def __init__(self, p):
+    def __init__(self, p, rank=0, world=1, log=print):
+        """rank / world from init_distributed; world > 1 needs the process group initialised."""
         from .collate import DeviceCollate
         from .optim import FlatAdam
         self.p = p
+        self.rank, self.world, self.log = rank, world, log
         self.dev = torch.device("cuda", int(p["device"])) if p["device"] != "cpu" else None
         if self.dev is None or not torch.cuda.is_available():
             raise SystemExit("train_mm: the libercgraph modules need a CUDA device (there is no CPU path)")
@@ -192,7 +242,14 @@ class Trainer:
         self.model = build_model(p, self.dev)
         self.collate = DeviceCollate(p["modality"], p["batch_first"], p["speaker_onehot"], p["n_speakers"], device=self.dev)
         self.optim = FlatAdam(self.model.parameters(), lr=p["lr"], weight_decay=p["weight_decay"], decoupled=p["optim"] == "AdamW",
-                              max_norm=5.0 if p["module"] == "dagerc" else None)                    # dagerc.py:229-231
+                              max_norm=5.0 if p["module"] == "dagerc" else None,                    # dagerc.py:229-231
+                              extra_slots=2 if world > 1 else 0)           # this rank's loss and accuracy ride with the gradient
+        self.comm = self.reduce = None
+        if world > 1:
+            import torch.distributed as dist
+            for t in list(self.model.parameters()) + list(self.model.buffers()):
+                dist.broadcast(t.data, 0)                  # rank 0's state everywhere, as DDP does when it wraps the model
+            self.optim.grad_scale = 1.0 / world            # the Adam kernel averages the summed gradients (and the clip norm)
         self.class_weight = None
         if p["module"] in ("dgcn", "dgcnv2") and p.get("loss_weights") and p["n_classes"] == 6:
             self.class_weight = torch.tensor(DGCN_LOSS_WEIGHTS, device=self.dev)
@@ -221,28 +278,93 @@ class Trainer:
         loss = ops.cross_entropy(logits, batch["label"], self.class_weight)
         self.optim.zero_grad()
         loss.backward()
+        if self.world > 1:
+            return self._step_data_parallel(loss.detach(), logits, batch["label"])
         self.optim.step()
         with torch.no_grad():
             acc = (logits.argmax(-1) == batch["label"]).float().mean()
         return loss.detach(), acc
+
+    def _step_data_parallel(self, loss, logits, labels):
+        """gather -> all-reduce(sum) of the flat gradient buffer -> Adam with grad_scale = 1/W (DDP's averaged gradient;
+        DAG-ERC's clip then acts on the norm of the average).  Returns the mean over the ranks of loss and accuracy, which
+        ride in the buffer's two extra slots."""
+        opt = self.optim
+        if opt.live is None:
+            self._attach_data_parallel()
+        opt.gather()
+        with torch.no_grad():
+            acc = (logits.argmax(-1) == labels).float().mean()
+            opt.extra.copy_(torch.stack([loss.float().reshape(()), acc]))
+        self.reduce(opt.flat_g)
+        opt.update()
+        mean = opt.extra / self.world
+        return mean[0], mean[1]
+
+    def _attach_data_parallel(self):
+        """After the first backward: the flat layout (must be the same on every rank, or the sum would mix parameters), then
+        the communicator, collectively -- peer memory when every rank can open its peers, else NCCL."""
+        import torch.distributed as dist
+        from .p2p import PeerComm, Reducer
+        opt = self.optim.attach()
+        names = {id(t): k for k, t in self.model.named_parameters()}
+        layout = [(names[id(t)], t.numel(), off) for t, off in zip(opt.live, opt.offsets)]
+        layouts = [None] * self.world
+        dist.all_gather_object(layouts, layout)
+        bad = [r for r, lay in enumerate(layouts) if lay != layouts[0]]
+        if bad:
+            raise RuntimeError("train_mm: the parameters that received a gradient differ between rank 0 and rank(s) %s; "
+                               "their flat gradient buffers cannot be summed" % bad)
+        nbytes = opt.flat_g.numel() * opt.flat_g.element_size()
+        comms = PeerComm.create(dist.group.WORLD, self.dev, max_bytes=nbytes)
+        self.comm = comms[0] if comms else None
+        self.reduce = Reducer(None, self.comm)
+        if self.comm is not None:
+            opt.skip_if_nonzero = self.comm.status_word()  # a timed-out exchange is never applied (ercg_adam_step_guarded)
+        self.log("train_mm: gradient all-reduce of %d floats over %d GPUs through %s" % (opt.flat_g.numel(), self.world,
+                                                                                          self.reduce.transport))
+
+    def _check_exchange(self):
+        """Raise on every rank if a peer-memory all-reduce timed out on any rank (no update was applied after it)."""
+        import torch.distributed as dist
+        from ._lib import ErcgError, lib
+        status = [None] * self.world
+        dist.all_gather_object(status, self.comm.status())
+        bad = [(r, s) for r, s in enumerate(status) if s != 0]
+        if bad:
+            raise ErcgError("train_mm: peer-memory gradient all-reduce failed: %s" % ", ".join(
+                "rank %d: %s (%d)" % (r, lib().ercg_strerror(s).decode(), s) for r, s in bad))
 
     @torch.no_grad()
     def test(self, data):
         """mmbase.py:180-201 + on_test_end :262-283."""
         from sklearn import metrics
         from . import ops
+        if self.world > 1:
+            import torch.distributed as dist
+            for b in self.model.buffers():
+                dist.broadcast(b, 0)                      # rank 0's BatchNorm running statistics (DDP broadcast_buffers)
         self.model.eval()
-        true, pred, lsum, n = [], [], 0.0, 0
         bs = self.p["batch_size"]
-        for i in range(0, len(data), bs):
-            batch = self.collate(data[i:i + bs])
+        starts = list(range(0, len(data), bs))
+        mine = []
+        for i in shard_test_batches(len(starts), self.rank, self.world):
+            batch = self.collate(data[starts[i]:starts[i] + bs])
             logits = self._logits(batch)
             ys = batch["label"]
-            lsum += float(ops.cross_entropy(logits, ys)) * ys.numel()
-            n += ys.numel()
-            true.extend(ys.cpu().tolist())
-            pred.extend(logits.argmax(-1).cpu().tolist())
+            mine.append((float(ops.cross_entropy(logits, ys)), ys.cpu().tolist(), logits.argmax(-1).cpu().tolist()))
         self.model.train()
+        results = mine
+        if self.world > 1:
+            per_rank = [None] * self.world
+            dist.all_gather_object(per_rank, mine)
+            results = restore_order(per_rank)
+        true, pred, lsum, n = [], [], 0.0, 0
+        for ce, ys, ps in results:
+            lsum += ce * len(ys)
+            n += len(ys)
+            true.extend(ys)
+            pred.extend(ps)
         return {"Lall": lsum / max(n, 1), "acc": metrics.accuracy_score(true, pred),
                 "wa": metrics.balanced_accuracy_score(true, pred),
                 "f1": metrics.f1_score(true, pred, average="weighted"), "mif1": metrics.f1_score(true, pred, average="micro"),
@@ -251,7 +373,7 @@ class Trainer:
 
     def save(self, name):
         d = self.p.get("save_dir")
-        if not d:
+        if not d or self.rank != 0:
             return None
         os.makedirs(d, exist_ok=True)
         path = os.path.join(d, name)
@@ -267,15 +389,18 @@ class Trainer:
             order = rng.permutation(len(train))
             t0 = time.perf_counter()
             lsum, asum, nb, utts = 0.0, 0.0, 0, 0
-            for i in range(0, len(order), p["batch_size"]):
-                samples = [train[j] for j in order[i:i + p["batch_size"]]]
+            batches = [order[i:i + p["batch_size"]] for i in range(0, len(order), p["batch_size"])]
+            for dealt in deal_batches(len(batches), self.world):
+                samples = [train[j] for j in batches[dealt[self.rank]]]
                 loss, acc = self.train_step(samples)
                 lsum += float(loss)
                 asum += float(acc)
                 nb += 1
-                utts += sum(len(s[0]["text"]) for s in samples)
+                utts += sum(len(train[j][0]["text"]) for b in dealt for j in batches[b])     # the utterances of every rank
             torch.cuda.synchronize()
             dt = time.perf_counter() - t0
+            if self.comm is not None:
+                self._check_exchange()
             te = self.test(test)                                                                      # test_per_epoch = 1, mmbase.py:136
             rec = {"epoch": epoch, "train_Lall": lsum / nb, "train_Acc": asum / nb, "utt_per_s": utts / dt,
                    **{"test_" + k: v for k, v in te.items() if k != "cm"}}
@@ -292,15 +417,27 @@ class Trainer:
 def main(argv=None, log=print):
     args = parse_args(list(sys.argv[1:] if argv is None else argv))
     p = resolve_params(args)
-    train, test, what = load_data(p)
-    log("train_mm: module=%s dataset=%s modality=%s hidden_all=%d n_classes=%d n_speakers=%d | %s: %d / %d dialogues" % (
-        p["module"], p["dataset"], p["modality"], p["hidden_all"], p["n_classes"], p["n_speakers"], what, len(train), len(test)))
-    tr = Trainer(p)
-    if p.get("eval_first"):
-        log("eval_first:", {k: v for k, v in tr.test(test).items() if k != "cm"})
-    hist = tr.train(train, test, log=log)
-    log("Best Results", json.dumps({k: v for k, v in tr.best.items() if k != "cm"}))
-    return {"params": p, "history": hist, "best": tr.best, "trainer": tr}
+    rank, world = init_distributed(p, log)
+    if rank != 0:
+        log = lambda *a: None                                                                   # only rank 0 logs
+    try:
+        train, test, what = load_data(p)
+        log("train_mm: module=%s dataset=%s modality=%s hidden_all=%d n_classes=%d n_speakers=%d | %s: %d / %d dialogues" % (
+            p["module"], p["dataset"], p["modality"], p["hidden_all"], p["n_classes"], p["n_speakers"], what, len(train), len(test)))
+        tr = Trainer(p, rank, world, log=log)
+        if p.get("eval_first"):
+            log("eval_first:", {k: v for k, v in tr.test(test).items() if k != "cm"})
+        hist = tr.train(train, test, log=log)
+        log("Best Results", json.dumps({k: v for k, v in tr.best.items() if k != "cm"}))
+        if tr.comm is not None:
+            import torch.distributed as dist
+            dist.barrier()                                 # no peer still reads this rank's region
+            tr.comm.close()
+        return {"params": p, "history": hist, "best": tr.best, "trainer": tr}
+    finally:
+        if world > 1:
+            import torch.distributed as dist
+            dist.destroy_process_group()
 
 
 if __name__ == "__main__":

@@ -461,6 +461,15 @@ int ercg_sumsq(const float* x, int64_t n, float* out, void* workspace, size_t wo
 int ercg_adam_step(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
                    float eps, float weight_decay, int decoupled, float grad_scale, const float* sumsq,
                    float max_norm, int64_t* step_dev, void* stream);
+/* ercg_adam_step_guarded: ercg_adam_step (same arguments, same arithmetic bit for bit) that first reads the DEVICE int
+ * *skip_if_nonzero: when it is not 0, both launches return before touching p, m, v or *step_dev.  The data-parallel trainer
+ * passes the sticky status word of its peer-memory communicator (ercg_p2p_status_word), so the gradient of a timed-out
+ * exchange is never applied -- DDP's all-reduce under accelerate (lumo/trainer/trainer.py:315-327) followed by
+ * optimizer.step() (track_mm/cogmen.py:187-189, dgcn.py:127-129, mmgcn.py:141-157, dagerc.py:229-231) raises instead of
+ * stepping on a failed collective.  skip_if_nonzero = NULL: ERCG_EINVAL. */
+int ercg_adam_step_guarded(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
+                           float eps, float weight_decay, int decoupled, float grad_scale, const float* sumsq,
+                           float max_norm, int64_t* step_dev, void* stream, const int* skip_if_nonzero);
 
 /* ---------------------------------------------------------------------------------------------
  * Peer-memory all-reduce over NVLink / NVSwitch for the exchanges of the dialogue-sharded train step: BatchNorm statistics,
@@ -494,6 +503,9 @@ int ercg_p2p_open(const unsigned char* ipc_handle, void** region);
 int ercg_p2p_close(void* peer_region);
 int ercg_p2p_free(void* region);
 int ercg_p2p_status(const void* region, int* status_host);
+/* ercg_p2p_status_word: *status_dev = DEVICE address of the region's sticky status word (the value ercg_p2p_status copies),
+ * for ercg_adam_step_guarded.  Host only, no synchronisation. */
+int ercg_p2p_status_word(void* region, int** status_dev);
 int ercg_p2p_allreduce(void* const* regions_dev, int rank, int world, const void* in, void* out, int64_t n, int dtype,
                        size_t max_bytes, void* stream);
 /* ercg_p2p_bn_act_bwd_reduce: ercg_bn_act_bwd_reduce fused with the exchange of its result: sums[2H] = this rank's
