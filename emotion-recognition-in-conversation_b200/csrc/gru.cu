@@ -15,6 +15,7 @@
 // dgh = [da_r, da_z, r * da_n] next to dgx = [da_r, da_z, da_n], and the caller forms dW_hh = dgh^T @ h_prev and
 // db_hh = colsum(dgh) with the fixed-order reductions of K2.
 #include "common.cuh"
+#include "rnn_cluster.cuh"
 #include <math.h>
 
 namespace ercg {
@@ -136,6 +137,8 @@ extern "C" int ercg_gru_fwd(const float* gx, int64_t ldgx, const float* whh, con
   if (B < 0) return ERCG_EINVAL;
   if (B == 0) return ERCG_OK;
   if (!gx || !whh || !bhh || !node_off || !out || !gates || !hprev) return ERCG_EINVAL;
+  if (Hd >= RNN_CLUSTER_MIN_HD && Hd <= RNN_CLUSTER_MAX_HD)     // K6c (rnn_cluster.cu)
+    return gru_cluster_fwd(gx, ldgx, whh, bhh, node_off, B, Hd, out, ldo, gates, hprev, (cudaStream_t)stream);
   long long want = 2LL * B;
   int grid = (int)(want < 2 * kNumSMs ? want : 2 * kNumSMs);
 #define ERCG_GRU_F(HD_)                                                                                                \
@@ -157,6 +160,8 @@ extern "C" int ercg_gru_bwd(const float* dout, int64_t ldo, const float* gates, 
   if (B < 0) return ERCG_EINVAL;
   if (B == 0) return ERCG_OK;
   if (!dout || !gates || !hprev || !whh || !node_off || !dgx || !dgh) return ERCG_EINVAL;
+  if (Hd >= RNN_CLUSTER_MIN_HD && Hd <= RNN_CLUSTER_MAX_HD)
+    return gru_cluster_bwd(dout, ldo, gates, hprev, whh, node_off, B, Hd, dgx, lddgx, dgh, lddgh, (cudaStream_t)stream);
   long long want = 2LL * B;
   int grid = (int)(want < 2 * kNumSMs ? want : 2 * kNumSMs);
 #define ERCG_GRU_B(HD_)                                                                                                 \

@@ -14,6 +14,7 @@
 // The weight gradients are NOT accumulated here: the kernel stores dpre[N, 8*Hd] and h_{t-1}[N, 2*Hd] and the
 // caller forms dW_hh = dpre^T @ h_prev, dW_ih = dpre^T @ x, db = colsum(dpre) with the split-K GEMM (K2).
 #include "common.cuh"
+#include "rnn_cluster.cuh"
 #include <math.h>
 
 namespace ercg {
@@ -137,6 +138,8 @@ extern "C" int ercg_lstm_fwd(const float* gx, int64_t ldgx, const float* whh, co
   if (B < 0) return ERCG_EINVAL;
   if (B == 0) return ERCG_OK;
   if (!gx || !whh || !node_off || !out || !gates || !cells || !hprev) return ERCG_EINVAL;
+  if (Hd >= RNN_CLUSTER_MIN_HD && Hd <= RNN_CLUSTER_MAX_HD)     // K6c (rnn_cluster.cu)
+    return lstm_cluster_fwd(gx, ldgx, whh, node_off, B, Hd, out, ldo, gates, cells, hprev, (cudaStream_t)stream);
   long long want = 2LL * B;
   int grid = (int)(want < 2 * kNumSMs ? want : 2 * kNumSMs);
 #define ERCG_LSTM_F(HD_)                                                                                         \
@@ -157,6 +160,8 @@ extern "C" int ercg_lstm_bwd(const float* dout, int64_t ldo, const float* gates,
   if (B < 0) return ERCG_EINVAL;
   if (B == 0) return ERCG_OK;
   if (!dout || !gates || !cells || !whh || !node_off || !dgx) return ERCG_EINVAL;
+  if (Hd >= RNN_CLUSTER_MIN_HD && Hd <= RNN_CLUSTER_MAX_HD)
+    return lstm_cluster_bwd(dout, ldo, gates, cells, whh, node_off, B, Hd, dgx, lddgx, (cudaStream_t)stream);
   long long want = 2LL * B;
   int grid = (int)(want < 2 * kNumSMs ? want : 2 * kNumSMs);
 #define ERCG_LSTM_B(HD_)                                                                                              \

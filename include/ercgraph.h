@@ -298,7 +298,10 @@ int ercg_edgeatt_bwd_dst(const float* dsig, const float* x, int64_t ldx,
  * fwd writes out[N,2*Hd] and saves gates[N,8*Hd] (post-activation), cells[N,2*Hd], hprev[N,2*Hd] (= h_{t-1}).
  * bwd writes dgx[N,8*Hd] (gradient w.r.t. the pre-activations); the caller forms
  *   dW_hh = dgx^T @ hprev, dW_ih = dgx^T @ x, db = colsum(dgx), dx = dgx @ [W_ih; W_ih_reverse] with K2.
- * Hd in {100 (the size the reference instantiates), 64, 48, 32, 24, 16, 8}; Hd % 4 == 0.
+ * Hd in {100 (the size the reference instantiates), 64, 48, 32, 24, 16, 8} runs K6 (lstm.cu: one CTA per direction and
+ * dialogue slice, W_hh rows in registers); any Hd in 101..384 runs K6c (rnn_cluster.cu: W_hh spread over the shared memory
+ * of a thread-block cluster of 8 CTAs, or a non-portable 16 when a slice does not fit at 8, with DSMEM exchange of h and of
+ * the W_hh^T da partials).  Other sizes return ERCG_EINVAL; ERCG_ECUDA if the device cannot schedule the cluster shape.
  * ------------------------------------------------------------------------------------------- */
 int ercg_lstm_fwd(const float* gx, int64_t ldgx, const float* whh, const int32_t* node_off, int B, int Hd,
                   float* out, int64_t ldo, float* gates, float* cells, float* hprev, void* stream);
@@ -321,7 +324,9 @@ int ercg_dropout(const float* x, float* out, int64_t n, float p, uint64_t seed, 
  * bwd writes dgx[N,6*Hd] = (da_r, da_z, da_n), the gradient w.r.t. gx, and dgh[N,6*Hd] = (da_r, da_z, r da_n), the
  * gradient w.r.t. W_hh h + b_hh; the caller forms dW_hh = dgh^T @ hprev, db_hh = colsum(dgh), dW_ih = dgx^T @ x,
  * db_ih = colsum(dgx), dx = dgx @ [W_ih; W_ih_reverse] with K2.
- * Hd in {100 (the size the reference instantiates), 64, 48, 32, 24, 16, 8}; other values return ERCG_EINVAL.
+ * Hd in {100 (the size the reference instantiates), 64, 48, 32, 24, 16, 8} runs K6b (gru.cu); any Hd in 101..384 runs K6c
+ * (rnn_cluster.cu, thread-block clusters of 8 or 16 CTAs, as for the LSTM).  Other values return ERCG_EINVAL; ERCG_ECUDA if
+ * the device cannot schedule the cluster shape.
  * ------------------------------------------------------------------------------------------- */
 int ercg_gru_fwd(const float* gx, int64_t ldgx, const float* whh, const float* bhh, const int32_t* node_off, int B, int Hd,
                  float* out, int64_t ldo, float* gates, float* hprev, void* stream);
