@@ -11,6 +11,8 @@
 // to an online (running max / rescale) chunked loop.  Score, softmax and aggregation are one kernel:
 // k_j and v_j rows are read once per edge from L1/L2, q_i/s_i/out_i once per node from HBM.
 // Algorithmic HBM bytes per node (SURVEY.md 8d): 5*4H (q,k,v,s,out) + 4 (rowptr) + 8*deg (col, alpha).
+// The float4 kernels here take H <= 384, H % 4 == 0 and 16-byte aligned rows; attn_wide.cuh runs the same algorithm for
+// every other even H <= 1024 and for 8-byte aligned rows (float4 or float2 chunks, chosen from H and the operands).
 #include "common.cuh"
 #include "attn_blk.cuh"
 #include <math.h>
@@ -735,10 +737,23 @@ edgeatt_bwd_dst_kernel(const float* __restrict__ dsig, const float* __restrict__
   }
 }
 
+#include "attn_wide.cuh"
+
+// window (tile) kernels and the NC = 1..3 kernels above: 16-byte aligned rows, H % 4 == 0, H <= 384
 static int chk(const void* p, long long ld, int H) {
   if ((H & 3) || H <= 0 || H > 384) return ERCG_EINVAL;
   if (!p) return ERCG_EINVAL;
   if ((ld & 3) || !aligned16(p)) return ERCG_EALIGN;
+  return ERCG_OK;
+}
+
+// warp-per-node kernels: any even H <= 1024, 8-byte aligned rows; *v4 stays true while every row so far also allows
+// float4 chunks (16-byte aligned, ld % 4 == 0)
+static int chk_row(const void* p, long long ld, int H, bool* v4) {
+  if ((H & 1) || H <= 0 || H > 1024) return ERCG_EINVAL;
+  if (!p) return ERCG_EINVAL;
+  if ((ld & 1) || (reinterpret_cast<uintptr_t>(p) & 7u)) return ERCG_EALIGN;
+  *v4 = *v4 && (ld & 3) == 0 && aligned16(p);
   return ERCG_OK;
 }
 
@@ -747,13 +762,24 @@ static int chk(const void* p, long long ld, int H) {
 using namespace ercg;
 
 #define ERCG_CHK(p, ld) do { int rc_ = chk(p, ld, H); if (rc_) return rc_; } while (0)
-#define ERCG_LAUNCH_NC(kernel, ...)                                                            \
-  do {                                                                                         \
-    const unsigned blocks_ = (unsigned)((N + AW - 1) / AW);                                    \
-    if (H <= 128) kernel<1><<<blocks_, AW * 32, 0, (cudaStream_t)stream>>>(__VA_ARGS__);       \
-    else if (H <= 256) kernel<2><<<blocks_, AW * 32, 0, (cudaStream_t)stream>>>(__VA_ARGS__);  \
-    else kernel<3><<<blocks_, AW * 32, 0, (cudaStream_t)stream>>>(__VA_ARGS__);                \
-    return finish_launch();                                                                    \
+#define ERCG_CHK_ROW(p, ld) do { int rc_ = chk_row(p, ld, H, &v4_); if (rc_) return rc_; } while (0)
+// float4 chunks NC = 1..3 where every row allows them and H <= 384 (the original kernels); float4 NC = 4..8 for wider
+// rows; float2 chunks when H % 4 == 2 or a row is only 8-byte aligned.  The choice depends on H and the operands only.
+#define ERCG_LAUNCH_NC(kernel, wide, ...)                                                               \
+  do {                                                                                                  \
+    const unsigned blocks_ = (unsigned)((N + AW - 1) / AW);                                             \
+    cudaStream_t st_ = (cudaStream_t)stream;                                                            \
+    if (v4_ && H <= 128) kernel<1><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                          \
+    else if (v4_ && H <= 256) kernel<2><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                     \
+    else if (v4_ && H <= 384) kernel<3><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                     \
+    else if (v4_ && H <= 512) wide<float4, 4><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);               \
+    else if (v4_ && H <= 768) wide<float4, 6><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);               \
+    else if (v4_) wide<float4, 8><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                           \
+    else if (H <= 256) wide<float2, 4><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                      \
+    else if (H <= 512) wide<float2, 8><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                      \
+    else if (H <= 768) wide<float2, 12><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                     \
+    else wide<float2, 16><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                                   \
+    return finish_launch();                                                                             \
   } while (0)
 
 extern "C" int ercg_attn_fwd(const float* q, const float* k, const float* v, const float* s, int64_t ld,
@@ -762,9 +788,10 @@ extern "C" int ercg_attn_fwd(const float* q, const float* k, const float* v, con
   if (N < 0) return ERCG_EINVAL;
   if (N == 0) return ERCG_OK;
   if (!rowptr || !col) return ERCG_EINVAL;
-  ERCG_CHK(q, ld); ERCG_CHK(k, ld); ERCG_CHK(v, ld); ERCG_CHK(out, ldo);
-  if (s) ERCG_CHK(s, ld);
-  ERCG_LAUNCH_NC(attn_fwd_kernel, q, k, v, s, ld, rowptr, col, scale, out, ldo, alpha, dact, N, H);
+  bool v4_ = (H & 3) == 0;
+  ERCG_CHK_ROW(q, ld); ERCG_CHK_ROW(k, ld); ERCG_CHK_ROW(v, ld); ERCG_CHK_ROW(out, ldo);
+  if (s) ERCG_CHK_ROW(s, ld);
+  ERCG_LAUNCH_NC(attn_fwd_kernel, attn_fwd_wide_kernel, q, k, v, s, ld, rowptr, col, scale, out, ldo, alpha, dact, N, H);
 }
 
 extern "C" int ercg_attn_bwd_dst(const float* dout, int64_t ldo, const float* k, const float* v, int64_t ld,
@@ -774,9 +801,10 @@ extern "C" int ercg_attn_bwd_dst(const float* dout, int64_t ldo, const float* k,
   if (N < 0) return ERCG_EINVAL;
   if (N == 0) return ERCG_OK;
   if (!rowptr || !col || !alpha || !dsig) return ERCG_EINVAL;
-  ERCG_CHK(dout, ldo); ERCG_CHK(k, ld); ERCG_CHK(v, ld); ERCG_CHK(dq, ldd);
-  if (ds) ERCG_CHK(ds, ldd);
-  ERCG_LAUNCH_NC(attn_bwd_dst_kernel, dout, ldo, k, v, ld, rowptr, col, alpha, scale, dq, ds, ldd, dsig, dact, N, H);
+  bool v4_ = (H & 3) == 0;
+  ERCG_CHK_ROW(dout, ldo); ERCG_CHK_ROW(k, ld); ERCG_CHK_ROW(v, ld); ERCG_CHK_ROW(dq, ldd);
+  if (ds) ERCG_CHK_ROW(ds, ldd);
+  ERCG_LAUNCH_NC(attn_bwd_dst_kernel, attn_bwd_dst_wide_kernel, dout, ldo, k, v, ld, rowptr, col, alpha, scale, dq, ds, ldd, dsig, dact, N, H);
 }
 
 extern "C" int ercg_attn_bwd_src(const float* dout, int64_t ldo, const float* q, int64_t ld,
@@ -786,8 +814,9 @@ extern "C" int ercg_attn_bwd_src(const float* dout, int64_t ldo, const float* q,
   if (N < 0) return ERCG_EINVAL;
   if (N == 0) return ERCG_OK;
   if (!t_rowptr || !t_col || !t_eid || !alpha || !dsig) return ERCG_EINVAL;
-  ERCG_CHK(dout, ldo); ERCG_CHK(q, ld); ERCG_CHK(dk, ldd); ERCG_CHK(dv, ldd);
-  ERCG_LAUNCH_NC(attn_bwd_src_kernel, dout, ldo, q, ld, t_rowptr, t_col, t_eid, alpha, dsig, scale, dk, dv, ldd, N, H);
+  bool v4_ = (H & 3) == 0;
+  ERCG_CHK_ROW(dout, ldo); ERCG_CHK_ROW(q, ld); ERCG_CHK_ROW(dk, ldd); ERCG_CHK_ROW(dv, ldd);
+  ERCG_LAUNCH_NC(attn_bwd_src_kernel, attn_bwd_src_wide_kernel, dout, ldo, q, ld, t_rowptr, t_col, t_eid, alpha, dsig, scale, dk, dv, ldd, N, H);
 }
 
 // ---- window-graph variants (contract: the in-neighbours of node i lie in [i - wlo, i + whi]; violated -> trap)
@@ -904,8 +933,9 @@ extern "C" int ercg_edgeatt_fwd(const float* x, int64_t ldx, const float* u, int
   if (N < 0) return ERCG_EINVAL;
   if (N == 0) return ERCG_OK;
   if (!t_rowptr || !t_col || !t_eid || !nu) return ERCG_EINVAL;
-  ERCG_CHK(x, ldx); ERCG_CHK(u, ldu);
-  ERCG_LAUNCH_NC(edgeatt_fwd_kernel, x, ldx, u, ldu, t_rowptr, t_col, t_eid, nu, N, H);
+  bool v4_ = (H & 3) == 0;
+  ERCG_CHK_ROW(x, ldx); ERCG_CHK_ROW(u, ldu);
+  ERCG_LAUNCH_NC(edgeatt_fwd_kernel, edgeatt_fwd_wide_kernel, x, ldx, u, ldu, t_rowptr, t_col, t_eid, nu, N, H);
 }
 
 extern "C" int ercg_edgeatt_bwd_src(const float* dnu, const float* nu, const float* u, int64_t ldu,
@@ -914,8 +944,9 @@ extern "C" int ercg_edgeatt_bwd_src(const float* dnu, const float* nu, const flo
   if (N < 0) return ERCG_EINVAL;
   if (N == 0) return ERCG_OK;
   if (!dnu || !nu || !t_rowptr || !t_col || !t_eid || !dsig) return ERCG_EINVAL;
-  ERCG_CHK(u, ldu); ERCG_CHK(dx, lddx);
-  ERCG_LAUNCH_NC(edgeatt_bwd_src_kernel, dnu, nu, u, ldu, t_rowptr, t_col, t_eid, dsig, dx, lddx, N, H);
+  bool v4_ = (H & 3) == 0;
+  ERCG_CHK_ROW(u, ldu); ERCG_CHK_ROW(dx, lddx);
+  ERCG_LAUNCH_NC(edgeatt_bwd_src_kernel, edgeatt_bwd_src_wide_kernel, dnu, nu, u, ldu, t_rowptr, t_col, t_eid, dsig, dx, lddx, N, H);
 }
 
 extern "C" int ercg_edgeatt_bwd_dst(const float* dsig, const float* x, int64_t ldx,
@@ -924,6 +955,7 @@ extern "C" int ercg_edgeatt_bwd_dst(const float* dsig, const float* x, int64_t l
   if (N < 0) return ERCG_EINVAL;
   if (N == 0) return ERCG_OK;
   if (!dsig || !rowptr || !col) return ERCG_EINVAL;
-  ERCG_CHK(x, ldx); ERCG_CHK(du, lddu);
-  ERCG_LAUNCH_NC(edgeatt_bwd_dst_kernel, dsig, x, ldx, rowptr, col, du, lddu, N, H);
+  bool v4_ = (H & 3) == 0;
+  ERCG_CHK_ROW(x, ldx); ERCG_CHK_ROW(du, lddu);
+  ERCG_LAUNCH_NC(edgeatt_bwd_dst_kernel, edgeatt_bwd_dst_wide_kernel, dsig, x, ldx, rowptr, col, du, lddu, N, H);
 }

@@ -295,6 +295,12 @@ class _Gather(torch.autograd.Function):
         Y, w = ctx.saved_tensors
         g, H, R = ctx.graph, ctx.H, ctx.R
         dout, ldo = _rows(dout)
+        if (ldo & 3) or (dout.data_ptr() & 15):
+            # the gradient of a column slice of a wider concatenation -- DialogueGCN's [features | graph out] at g = 2 (mod 4),
+            # dgcnv2's [features | graph out] at odd hidden sizes -- has rows only 8-byte aligned; the gather kernels read
+            # 16-byte chunks, so such a gradient is repacked once ([N, H], H = the graph width of 100)
+            dout = dout.clone(memory_format=torch.contiguous_format)
+            ldo = dout.stride(0)
         N = dout.size(0)
         dY = torch.empty((N, ctx.ycols), dtype=torch.float32, device=dout.device)
         dw = torch.empty(g.E, dtype=torch.float32, device=dout.device) if ctx.w_grad else None

@@ -236,13 +236,17 @@ int ercg_gather_window_bwd(const float* dout, int64_t ldo, const int32_t* t_rowp
  * softmax over the in-edges of each destination (max-subtracted, denominator + 1e-16), weighted
  * aggregate of v, plus the skip row:  out[i] = sum_j alpha[j->i] v[j] + s[i].
  * alpha[E] (by-destination order) is saved for the backward.  q,k,v,s share one leading dimension.
+ * H: any even value in [2, 1024] (odd, <= 0 or > 1024 -> ERCG_EINVAL).  Rows need 8-byte alignment: every pointer
+ * 8-byte aligned and every leading dimension even (else ERCG_EALIGN).  16-byte aligned rows with H % 4 == 0 load
+ * float4 chunks, others float2 chunks; both are bit-reproducible.  N == 0: no-op; N < 0: ERCG_EINVAL.
  * ------------------------------------------------------------------------------------------- */
 int ercg_attn_fwd(const float* q, const float* k, const float* v, const float* s, int64_t ld,
                   const int32_t* rowptr, const int32_t* col, float scale,
                   float* out, int64_t ldo, float* alpha, float* dact, int64_t N, int H, void* stream);
 /* dact (optional, [E]): the softmax runs over tanh(score) instead of the score -- nodal MatchingAttention 'general2' of the
  * declare-lab DialogueGCN (track_mm/dgcnv2_models.py:119-146, used over fully connected per-dialogue graphs, s = NULL,
- * scale = 1) -- and dact[e] = 1 - tanh^2 is saved for ercg_attn_bwd_dst, which folds it into dsig.  H <= 384. */
+ * scale = 1) -- and dact[e] = 1 - tanh^2 is saved for ercg_attn_bwd_dst, which folds it into dsig.  Same H range and
+ * alignment as above, so the key half of dgcnv2's [xt | e] may start 8 bytes past a 16-byte boundary. */
 /* by-destination half: dq[i], ds[i] = dout[i], dsig[e] = alpha_e (dalpha_e - sum alpha dalpha) [* dact_e] */
 int ercg_attn_bwd_dst(const float* dout, int64_t ldo, const float* k, const float* v, int64_t ld,
                       const int32_t* rowptr, const int32_t* col, const float* alpha, float scale,
@@ -279,6 +283,8 @@ int ercg_attn_window_bwd_src(const float* dout, int64_t ldo, const float* q, int
  *   nu[j->k] = softmax_{k in out(j)} <x_j, u_k>,  u = x @ W^T  (u computed by ercg_gemm_nn)
  * written in by-destination edge order (nu[t_eid]).  Backward: dsig per edge, dx_j += sum dsig u_k
  * (by source), du_k = sum_j dsig x_j (by destination).
+ * H = g_dim: any even value in [2, 1024]; rows 8-byte aligned with even leading dimensions (same checks and return codes
+ * as K4's ercg_attn_fwd).
  * ------------------------------------------------------------------------------------------- */
 int ercg_edgeatt_fwd(const float* x, int64_t ldx, const float* u, int64_t ldu,
                      const int32_t* t_rowptr, const int32_t* t_col, const int32_t* t_eid,
