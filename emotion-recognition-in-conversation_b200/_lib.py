@@ -32,6 +32,17 @@ class DagLayer(Structure):
                                          "dH1", "dpre", "dGseq", "dM", "dS", "dHdir", "ga")])
 
 
+class DialogueRnnArgs(Structure):
+    """ercg_dialogue_rnn (include/ercgraph.h)."""
+    _fields_ = ([(n, c_int) for n in ("L", "B", "Dg", "Dp", "De", "P")] + [("drop_p", c_float), ("reserved", c_int)] +
+                [(n, c_uint64) for n in ("seed_g", "seed_q", "seed_e")] +
+                [("qmask", c_void_p), ("pre", c_void_p), ("ldpre", c_int64), ("xq", c_void_p), ("ldxq", c_int64)] +
+                [(n, c_void_p) for n in ("Wgq", "Whh_g", "bhh_g", "Wpc", "Whh_p", "bhh_p", "Wih_e", "Whh_e", "bih_e", "bhh_e",
+                                         "e", "g", "c", "qprev", "qcur", "gates_g", "gates_p", "gates_e", "alpha", "qstate",
+                                         "de", "dpre")] + [("lddpre", c_int64), ("dxq", c_void_p), ("lddxq", c_int64)] +
+                [(n, c_void_p) for n in ("dgh", "dph", "dei", "deh", "dG", "dQ", "dEh", "dc")])
+
+
 P, I, L, F, D, U64, SZ = c_void_p, c_int, c_int64, c_float, c_double, c_uint64, c_size_t
 
 # name -> (restype, argtypes); mirrors include/ercgraph.h one to one
@@ -131,6 +142,9 @@ SIGNATURES = {
     "ercg_dag_layer_bwd": (I, [POINTER(DagLayer), P]),
     "ercg_dag_gat_fwd": (I, [P, L, P, L, L, P, L, L, P, P, L, P, P, P, P, I, I, I, P]),
     "ercg_dag_gat_bwd": (I, [P, L, L, P, L, P, P, P, P, P, P, P, P, I, I, I, P]),
+    # K12 (DialogueRNN)
+    "ercg_dialogue_rnn_fwd": (I, [POINTER(DialogueRnnArgs), P]),
+    "ercg_dialogue_rnn_bwd": (I, [POINTER(DialogueRnnArgs), P]),
 }
 
 _lib = None

@@ -1,6 +1,7 @@
-"""Drop-in for the DialogueGCN part of track_mm/dgcnv2_models.py (reference :517-773; SURVEY.md 8f-2): ``MatchingAttention``
-('general2'), ``MaskedEdgeAttention`` ('attn1'), ``edge_perms``, ``batch_graphify`` and ``GraphNetwork`` with the reference's
-constructor arguments, signatures and state_dict keys.
+"""Drop-in for track_mm/dgcnv2_models.py (SURVEY.md 8f-2): the DialogueGCN part (reference :517-773) -- ``MatchingAttention``
+('general2'), ``MaskedEdgeAttention`` ('attn1'), ``edge_perms``, ``batch_graphify`` and ``GraphNetwork`` -- and the DialogueRNN
+recurrence (:235-348) -- ``SimpleAttention``, ``DialogueRNNCell``, ``DialogueRNN`` -- with the reference's constructor
+arguments, signatures and state_dict keys.
 
 Kernel mapping
   MaskedEdgeAttention.scalar (Linear 2D -> 110)   K2 over the dialogue-major full-length rows
@@ -10,9 +11,13 @@ Kernel mapping
   nodal MatchingAttention over each dialogue      transform = K2, then the generic K4 kernels with the tanh option on the
                                                   fully connected per-dialogue graph (K1 with window -1 / -1)
   linear -> ReLU -> dropout -> smax_fc            ops.mlp_head
-The unused attention variants of the file (SimpleAttention, Attention 'mlp', MatchingAttention 'dot' / 'general' / 'concat')
-and the DialogueRNN base model are parameter holders or NotImplementedError: DGCNModule with 'attn1' and nodal 'general2'
-never executes them, whichever of its recurrent or linear bases it runs.
+  DialogueRNN (all L steps, all dialogues)        the U columns of g_cell / p_cell and the 'general' transform: one K2 GEMM
+                                                  over all L*B rows; the three GRUCells, the attention over the global-state
+                                                  history and the party-state update: K12 (csrc/dialogue_rnn.cu), one
+                                                  persistent kernel forward and one backward
+The unused attention variants of the file (Attention 'mlp', MatchingAttention 'dot' / 'concat') are parameter holders or
+NotImplementedError: DGCNModule with 'attn1' and nodal 'general2' never executes them.  DialogueRNN runs stand-alone;
+DGCNModule("DialogRNN") still raises NotImplementedError.
 """
 import torch
 from torch import nn
@@ -28,10 +33,11 @@ from .dgcn_models import _fresh_seed
 class MatchingAttention(nn.Module):
     def __init__(self, mem_dim, cand_dim, alpha_dim=None, att_type="general"):
         super().__init__()
-        if att_type != "general2":
-            raise NotImplementedError("only att_type='general2' is instantiated by the DialogueGCN path (dgcnv2_models.py:531,761)")
+        if att_type not in ("general", "general2"):
+            raise NotImplementedError("att_type %r: only 'general' (DialogueRNN's context attention) and 'general2' (the "
+                                      "DialogueGCN path, dgcnv2_models.py:531,761) are instantiated" % (att_type,))
         self.mem_dim, self.cand_dim, self.att_type = mem_dim, cand_dim, att_type
-        self.transform = nn.Linear(cand_dim, mem_dim, bias=True)
+        self.transform = nn.Linear(cand_dim, mem_dim, bias=att_type == "general2")
 
     def pooled(self, emotions, graph_full):
         """All nodes at once: out_t = sum_j softmax_j(tanh(<transform(e_t), e_j>)) e_j over node t's own dialogue."""
@@ -44,6 +50,74 @@ class MatchingAttention(nn.Module):
         path evaluates all positions of all dialogues at once (``pooled``)."""
         raise NotImplementedError("MatchingAttention.forward(M, x, mask): use pooled(emotions, graph_full) -- every node of "
                                   "every dialogue in one launch (same arithmetic as the reference's loop over positions)")
+
+
+class SimpleAttention(nn.Module):
+    """Parameter holder of the 'simple' context attention: alpha = softmax over the history of
+    scalar(M); DialogueRNN runs it inside K12."""
+
+    def __init__(self, input_dim):
+        super().__init__()
+        self.input_dim = input_dim
+        self.scalar = nn.Linear(input_dim, 1, bias=False)
+
+    def forward(self, M, x=None):
+        raise NotImplementedError("SimpleAttention.forward: DialogueRNN evaluates the attention of every step inside K12")
+
+
+class DialogueRNNCell(nn.Module):
+    """One step of DialogueRNN (dgcnv2_models.py:235-313).  Holds the reference's parameters; the recurrence over all steps
+    runs in DialogueRNN.forward (K12)."""
+
+    def __init__(self, D_m, D_g, D_p, D_e, listener_state=False, context_attention="simple", D_a=100, dropout=0.5):
+        super().__init__()
+        if listener_state:
+            raise NotImplementedError("DialogueRNNCell(listener_state=True) is not implemented")
+        if context_attention not in ("simple", "general"):
+            raise NotImplementedError("context_attention %r: only 'simple' and 'general' are implemented" % (context_attention,))
+        self.D_m, self.D_g, self.D_p, self.D_e = D_m, D_g, D_p, D_e
+        self.listener_state, self.context_attention = listener_state, context_attention
+        self.g_cell = nn.GRUCell(D_m + D_p, D_g)
+        self.p_cell = nn.GRUCell(D_m + D_g, D_p)
+        self.e_cell = nn.GRUCell(D_p, D_e)
+        self.dropout = nn.Dropout(dropout)
+        if context_attention == "simple":
+            self.attention = SimpleAttention(D_g)
+        else:
+            self.attention = MatchingAttention(D_g, D_m, D_a, context_attention)
+
+    def forward(self, U, qmask, g_hist, q0, e0):
+        raise NotImplementedError("DialogueRNNCell.forward (one step): use DialogueRNN.forward(U, qmask) -- all steps of all "
+                                  "dialogues in one K12 launch per direction")
+
+
+class DialogueRNN(nn.Module):
+    """dgcnv2_models.py:316-348.  forward(U [L,B,D_m], qmask [L,B,P]) -> (e [L,B,D_e], alpha: L-1 tensors [B, t]).
+    Every dialogue runs all L steps (no lengths, as in the reference).  The party cell is evaluated for the speaker
+    (first argmax of the qmask row) only, which equals the reference's blend over all parties when each qmask row has at
+    most one non-zero entry (one-hot or all-zero rows)."""
+
+    def __init__(self, D_m, D_g, D_p, D_e, listener_state=False, context_attention="simple", D_a=100, dropout=0.5):
+        super().__init__()
+        self.D_m, self.D_g, self.D_p, self.D_e = D_m, D_g, D_p, D_e
+        self.dropout = nn.Dropout(dropout)          # owned but never applied by the reference's forward
+        self.dialogue_cell = DialogueRNNCell(D_m, D_g, D_p, D_e, listener_state, context_attention, D_a, dropout)
+
+    def forward(self, U, qmask):
+        cell = self.dialogue_cell
+        if U.dim() != 3 or qmask.dim() != 3:
+            raise ValueError("U [L, B, D_m] and qmask [L, B, P] must be 3-D, got %s and %s" % (tuple(U.shape), tuple(qmask.shape)))
+        if U.size(2) != self.D_m or qmask.shape[:2] != U.shape[:2]:
+            raise ValueError("shape mismatch: U %s (D_m = %d), qmask %s" % (tuple(U.shape), self.D_m, tuple(qmask.shape)))
+        dev = cell.g_cell.weight_hh.device
+        if U.device != dev or qmask.device != dev or dev.type != "cuda":
+            raise ValueError("U (%s), qmask (%s) and the parameters (%s) must be on the same CUDA device" % (U.device, qmask.device, dev))
+        if U.dtype != torch.float32:
+            raise ValueError("U must be float32, got %s" % U.dtype)
+        p = cell.dropout.p if self.training else 0.0
+        seeds = (_fresh_seed(), _fresh_seed(), _fresh_seed()) if p > 0 else (0, 0, 0)
+        att = cell.attention.scalar.weight if cell.context_attention == "simple" else cell.attention.transform.weight
+        return ops_dgcnv2.dialogue_rnn(U, qmask, cell.g_cell, cell.p_cell, cell.e_cell, att, cell.context_attention, p, seeds)
 
 
 class MaskedEdgeAttention(nn.Module):

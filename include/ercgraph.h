@@ -611,6 +611,54 @@ int ercg_dag_gat_bwd(const float* V, int64_t ldv_b, int64_t ldv_n, const float* 
                      const float* w_linear, const float* alpha, const float* dalpha, const float* dS01, float* de,
                      float* dQ, float* dK, float* dV, int B, int N, int D, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * K12  DialogueRNN recurrence (DialogueRNN / DialogueRNNCell of the declare-lab DialogueRNN, track_mm/dgcnv2_models.py:235-348,
+ * listener_state=False, context_attention 'simple' or 'general') over B dialogues of L steps each (seq-first rows r = t*B + b;
+ * every dialogue runs all L steps).  Per step, with s = argmax_p qmask[r] (first on ties) and m = qmask[r, s]:
+ *   g_t = drop_g(GRUCell_g([U_t ; q_{t-1}[s]], g_{t-1}))
+ *   c_t = sum_{j<t} alpha_j g_j, alpha = softmax_j(xq_r . g_j)  (c_0 = 0; xq_r = W_a U_t for 'general', the weight w of
+ *         'simple' for every row)
+ *   q_t[s] = q_{t-1}[s] (1 - m) + m drop_q(GRUCell_p([U_t ; c_t], q_{t-1}[s])),  q_t[p] = q_{t-1}[p] for p != s
+ *   e_t = drop_e(GRUCell_e(q_t[s], e_{t-1}))
+ * nn.GRUCell semantics (gate order r, z, n), zero initial states.  The reference runs the party cell for every party and
+ * blends with qmask; running it for the speaker only is exact when each qmask row has at most one non-zero entry.
+ * The U-dependent input-gate terms are hoisted: pre[L*B, >= 3Dg+3Dp] = U @ [W_ih^g[:, :Dm] ; W_ih^p[:, :Dm]]^T + [b_ih^g ;
+ * b_ih^p] (ercg_gemm_nn), columns [0, 3Dg) for the g cell and [3Dg, 3Dg+3Dp) for the party cell.  Dropout (drop_p in
+ * [0, 1)): element (r, u) of cell x in {g, q, e} is kept iff hash_uniform(seed_x, r*D_x + u) >= drop_p and then scaled by
+ * 1 / (1 - drop_p) -- ercg_dropout's mask on a contiguous [L*B, D_x] tensor.
+ * Dg, Dp, De in 1..256, P in 1..16; negative sizes, other widths or P, or drop_p outside [0, 1): ERCG_EINVAL before any
+ * launch.  B == 0 or L == 0: no-op.  One persistent cooperative kernel per direction (weights sliced by hidden unit over
+ * the CTAs' shared memory, all dialogues in lockstep, grid.sync between phases); ERCG_ECUDA if the device cannot
+ * co-schedule the grid.  Fixed-order fp32 arithmetic, no atomics: results are bit-reproducible.
+ * fwd writes e[L*B,De] and saves g[L*B,Dg] (after dropout), c[L*B,Dg], qprev / qcur[L*B,Dp] (q_{t-1}[s], q_t[s]),
+ * gates_{g,p,e}[L*B, 4D] (r, z, n, W_hn h + b_hn) and alpha (step t >= 1 is the [B, t] block at offset B*t*(t-1)/2);
+ * qstate[B*P*Dp] is workspace.
+ * bwd reads de[L*B,De] and writes dpre (gradient w.r.t. the pre columns, row stride lddpre), dxq[L*B,Dg] (w.r.t. xq_r, row
+ * stride lddxq;
+ * 'simple': dw = column sums), dgh[L*B,3Dg], dph[L*B,3Dp], deh[L*B,3De] (w.r.t. W_hh h + b_hh of each cell: dW_hh = dgh^T @
+ * h_{t-1}, db_hh = colsum) and dei[L*B,3De] (w.r.t. W_ih^e q_t[s] + b_ih^e).  dG[L*B,Dg], dQ[B*P*Dp], dEh[B*De] and
+ * dc[B*Dg] are workspace.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct ercg_dialogue_rnn {
+  int32_t L, B, Dg, Dp, De, P;
+  float drop_p;
+  int32_t reserved;
+  uint64_t seed_g, seed_q, seed_e;
+  const float* qmask;                         /* [L*B, P] */
+  const float* pre; int64_t ldpre;
+  const float* xq; int64_t ldxq;              /* [L*B, Dg] rows, or one row with ldxq = 0 */
+  const float *Wgq, *Whh_g, *bhh_g;           /* g_cell.weight_ih[:, Dm:] [3Dg,Dp], weight_hh [3Dg,Dg], bias_hh [3Dg] */
+  const float *Wpc, *Whh_p, *bhh_p;           /* p_cell.weight_ih[:, Dm:] [3Dp,Dg], weight_hh [3Dp,Dp], bias_hh [3Dp] */
+  const float *Wih_e, *Whh_e, *bih_e, *bhh_e; /* e_cell [3De,Dp], [3De,De], [3De], [3De] */
+  float *e, *g, *c, *qprev, *qcur, *gates_g, *gates_p, *gates_e, *alpha, *qstate;
+  const float* de;                            /* backward only from here on */
+  float* dpre; int64_t lddpre;
+  float* dxq; int64_t lddxq;
+  float *dgh, *dph, *dei, *deh, *dG, *dQ, *dEh, *dc;
+} ercg_dialogue_rnn;
+int ercg_dialogue_rnn_fwd(const ercg_dialogue_rnn* args, void* stream);
+int ercg_dialogue_rnn_bwd(const ercg_dialogue_rnn* args, void* stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
