@@ -832,14 +832,7 @@ static bool attn_use_blk(int H, int wlo, int whi) {
   const char* e = getenv("ERCG_ATTN_BLK");
   return (!e || atoi(e) != 0) && attn_blk_ok(H, wlo, whi);
 }
-template <typename K>
-static bool blk_attr(K kernel, DeviceOnce& once) {
-  if (once.need()) {
-    if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024) != cudaSuccess) return false;
-    once.mark();
-  }
-  return true;
-}
+constexpr int ATTN_SMEM_LIMIT = 100 * 1024;   // dynamic shared memory limit of the window-attention kernels
 
 extern "C" int ercg_attn_window_supported(int H, int wlo, int whi) { return attn_tile_ok(H, wlo, whi) ? 1 : 0; }
 extern "C" int64_t ercg_attn_window_tiles(int64_t N) { return N <= 0 ? 0 : (N + WT - 1) / WT; }
@@ -856,17 +849,12 @@ extern "C" int ercg_attn_window_fwd(const float* q, const float* k, const float*
   const unsigned blocks = (unsigned)((N + WT - 1) / WT);
   cudaStream_t st = (cudaStream_t)stream;
   if (attn_use_blk(H, wlo, whi)) {
-    static DeviceOnce once;
-    if (!blk_attr(attn_fwd_blk_kernel<BTH_FWD>, once)) return ERCG_ECUDA;
+    if (!smem_limit<attn_fwd_blk_kernel<BTH_FWD>>(ATTN_SMEM_LIMIT)) return ERCG_ECUDA;
     attn_fwd_blk_kernel<BTH_FWD><<<blocks, BTH_FWD, attn_blk_smem(H, wlo, whi, 0), st>>>(q, k, v, s, ld, rowptr, col, scale, out, ldo, alpha, N, H, wlo, whi);
     return finish_launch();
   }
-  static DeviceOnce attr;
-  if (attr.need()) {
-    cudaFuncSetAttribute(attn_fwd_tile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-    cudaFuncSetAttribute(attn_fwd_tile_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-    attr.mark();
-  }
+  if (!smem_limit<attn_fwd_tile_kernel<true>>(ATTN_SMEM_LIMIT) || !smem_limit<attn_fwd_tile_kernel<false>>(ATTN_SMEM_LIMIT))
+    return ERCG_ECUDA;
   if (wlo + whi + 1 <= 16) attn_fwd_tile_kernel<true><<<blocks, 256, sm, st>>>(q, k, v, s, ld, rowptr, col, scale, out, ldo, alpha, N, H, wlo, whi);
   else attn_fwd_tile_kernel<false><<<blocks, 256, sm, st>>>(q, k, v, s, ld, rowptr, col, scale, out, ldo, alpha, N, H, wlo, whi);
   return finish_launch();
@@ -885,17 +873,12 @@ extern "C" int ercg_attn_window_bwd_dst(const float* dout, int64_t ldo, const fl
   const unsigned blocks = (unsigned)((N + WT - 1) / WT);
   cudaStream_t st = (cudaStream_t)stream;
   if (attn_use_blk(H, wlo, whi)) {
-    static DeviceOnce once;
-    if (!blk_attr(attn_bwd_dst_blk_kernel<BTH_DST>, once)) return ERCG_ECUDA;
+    if (!smem_limit<attn_bwd_dst_blk_kernel<BTH_DST>>(ATTN_SMEM_LIMIT)) return ERCG_ECUDA;
     attn_bwd_dst_blk_kernel<BTH_DST><<<blocks, BTH_DST, attn_blk_smem(H, wlo, whi, 1), st>>>(dout, ldo, k, v, ld, rowptr, col, alpha, scale, dq, ds, ldd, dsig, colsum_partial, N, H, wlo, whi);
     return finish_launch();
   }
-  static DeviceOnce attr;
-  if (attr.need()) {
-    cudaFuncSetAttribute(attn_bwd_dst_tile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-    cudaFuncSetAttribute(attn_bwd_dst_tile_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-    attr.mark();
-  }
+  if (!smem_limit<attn_bwd_dst_tile_kernel<true>>(ATTN_SMEM_LIMIT) || !smem_limit<attn_bwd_dst_tile_kernel<false>>(ATTN_SMEM_LIMIT))
+    return ERCG_ECUDA;
   if (wlo + whi + 1 <= 16) attn_bwd_dst_tile_kernel<true><<<blocks, 256, sm, st>>>(dout, ldo, k, v, ld, rowptr, col, alpha, scale, dq, ds, ldd, dsig, colsum_partial, N, H, wlo, whi);
   else attn_bwd_dst_tile_kernel<false><<<blocks, 256, sm, st>>>(dout, ldo, k, v, ld, rowptr, col, alpha, scale, dq, ds, ldd, dsig, colsum_partial, N, H, wlo, whi);
   return finish_launch();
@@ -913,16 +896,11 @@ extern "C" int ercg_attn_window_bwd_src(const float* dout, int64_t ldo, const fl
   const size_t sm = attn_tile_smem(H, wlo, whi, 0, 2);
   const unsigned blocks = (unsigned)((N + WT - 1) / WT);
   if (attn_use_blk(H, wlo, whi)) {
-    static DeviceOnce once;
-    if (!blk_attr(attn_bwd_src_blk_kernel<BTH_SRC>, once)) return ERCG_ECUDA;
+    if (!smem_limit<attn_bwd_src_blk_kernel<BTH_SRC>>(ATTN_SMEM_LIMIT)) return ERCG_ECUDA;
     attn_bwd_src_blk_kernel<BTH_SRC><<<blocks, BTH_SRC, attn_blk_smem(H, wlo, whi, 2), (cudaStream_t)stream>>>(dout, ldo, q, ld, t_rowptr, t_col, t_eid, alpha, dsig, scale, dk, dv, ldd, colsum_partial, N, H, wlo, whi);
     return finish_launch();
   }
-  static DeviceOnce attr;
-  if (attr.need()) {
-    cudaFuncSetAttribute(attn_bwd_src_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
-    attr.mark();
-  }
+  if (!smem_limit<attn_bwd_src_tile_kernel>(ATTN_SMEM_LIMIT)) return ERCG_ECUDA;
   attn_bwd_src_tile_kernel<<<blocks, 256, sm, (cudaStream_t)stream>>>(dout, ldo, q, ld, t_rowptr, t_col, t_eid, alpha, dsig, scale, dk, dv, ldd, colsum_partial, N, H, wlo, whi);
   return finish_launch();
 }

@@ -131,38 +131,121 @@ __device__ __forceinline__ bool dropout_drop(uint64_t h, int lane4, unsigned thr
 
 constexpr int kNumSMs = 148;   // B200
 constexpr int kMaxDevices = 64; // per-device caches of launch attributes are indexed by the CUDA device id
+constexpr int kMaxSmemPerBlock = 227 * 1024;   // B200: the most dynamic shared memory one block may opt in to
 
-// Per-device one-time setup (cudaFuncSetAttribute is per device context) and per-device attribute caches.  Function-local
-// `static bool done` flags made the second GPU of a process launch with the first GPU's setup; these are indexed by the
-// CUDA device id and safe to race on (worst case: the setup runs twice).
+// ---- launch set-up shared by every kernel that needs more than a plain <<<>>> launch: a dynamic shared-memory limit above
+// 48 KB, a cluster shape, or a cooperative (co-resident) grid.  Everything below is per device: kernel attributes belong to
+// the device context, and the answers are computed once so that a launch inside a CUDA-graph capture makes no set-up call.
 inline int current_device() {
   int d = 0;
   cudaGetDevice(&d);
   return d;
 }
-struct DeviceOnce {
-  std::atomic<unsigned char> done[kMaxDevices];
-  bool need() const {
+
+// A value computed once per CUDA device id (one process may drive several GPUs, each needs its own set-up).  A result < 1
+// means "unavailable" and is cached as such (read back as 0).  Safe to race on: at worst compute() runs twice.  Device ids
+// >= kMaxDevices are not cached.
+struct PerDevice {
+  std::atomic<int> v[kMaxDevices];
+  template <class F>
+  int get(F compute) {
     const int d = current_device();
-    return d < 0 || d >= kMaxDevices || !done[d].load(std::memory_order_acquire);
-  }
-  void mark() {
-    const int d = current_device();
-    if (d >= 0 && d < kMaxDevices) done[d].store(1, std::memory_order_release);
+    const bool slot = d >= 0 && d < kMaxDevices;
+    if (slot) {
+      const int c = v[d].load(std::memory_order_acquire);
+      if (c != 0) return c > 0 ? c : 0;
+    }
+    const int n = compute();
+    if (slot) v[d].store(n > 0 ? n : -1, std::memory_order_release);
+    return n > 0 ? n : 0;
   }
 };
+
 inline int device_sm_count() {
-  static std::atomic<int> cache[kMaxDevices];
-  const int d = current_device();
-  if (d >= 0 && d < kMaxDevices) {
-    const int c = cache[d].load(std::memory_order_acquire);
-    if (c > 0) return c;
+  static PerDevice sms;
+  return sms.get([] {
+    int n = 0;
+    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, current_device());
+    return n > 0 ? n : kNumSMs;
+  });
+}
+
+// Raises kernel K's dynamic shared-memory limit to `bytes` on the current device, once per device.  Every caller of one K
+// passes the same bytes.  false (with no error left pending) when the runtime refuses; the caller returns ERCG_ECUDA.
+template <auto K>
+bool smem_limit(int bytes) {
+  static PerDevice done;
+  return done.get([&] {
+    if (cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) == cudaSuccess) return 1;
+    cudaGetLastError();
+    return 0;
+  }) > 0;
+}
+
+// cudaLaunchKernelEx configuration of `grid` blocks in 1-D clusters of C
+struct ClusterConfig {
+  cudaLaunchConfig_t cfg = {};
+  cudaLaunchAttribute attr[1];
+  ClusterConfig(int C, int grid, int threads, size_t smem, cudaStream_t st) {
+    cfg.gridDim = dim3(grid, 1, 1);
+    cfg.blockDim = dim3(threads, 1, 1);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = C;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
   }
-  int n = 0;
-  cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, d);
-  if (n < 1) n = kNumSMs;
-  if (d >= 0 && d < kMaxDevices) cache[d].store(n, std::memory_order_release);
-  return n;
+  ClusterConfig(const ClusterConfig&) = delete;      // cfg.attrs points into this object
+};
+
+// How many of kernel K can be resident at once: blocks per SM for C = 1, clusters of C blocks on the device for C > 1.
+// Asked once per device at `smem`, the largest dynamic shared memory K may launch with (which becomes K's limit), so the
+// answer is a lower bound for every launch.  0: K cannot be scheduled this way.
+template <auto K, int C = 1>
+int resident_capacity(int threads, int smem) {
+  static PerDevice cap;
+  return cap.get([&] {
+    if (smem > 0 && !smem_limit<K>(smem)) return 0;
+    int n = 0;
+    cudaError_t err;
+    if constexpr (C == 1) {
+      err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, K, threads, smem);
+    } else {
+      err = C > 8 ? cudaFuncSetAttribute(K, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) : cudaSuccess;
+      ClusterConfig c(C, C, threads, smem, 0);
+      if (err == cudaSuccess) err = cudaOccupancyMaxActiveClusters(&n, K, &c.cfg);
+    }
+    if (err != cudaSuccess) {
+      cudaGetLastError();
+      n = 0;
+    }
+    return n;
+  });
+}
+
+// Result of a launch made with cudaLaunchKernelEx / cudaLaunchCooperativeKernel.  A failed launch leaves its error
+// pending, and finish_launch() of the next unrelated launch would report it as its own, so it is cleared here.
+inline int launch_status(cudaError_t err) {
+  if (err == cudaSuccess) return finish_launch();
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  cudaGetLastError();
+  return ERCG_ECUDA;
+}
+
+template <typename... KArgs, typename... Args>
+int launch_cluster(void (*kernel)(KArgs...), int C, int grid, int threads, size_t smem, cudaStream_t st, Args&&... args) {
+  ClusterConfig c(C, grid, threads, smem, st);
+  return launch_status(cudaLaunchKernelEx(&c.cfg, kernel, static_cast<Args&&>(args)...));
+}
+
+// For kernels that call grid.sync(): the caller first checks that the grid fits resident_capacity.
+template <typename P>
+int launch_cooperative(void (*kernel)(P), int grid, int threads, size_t smem, cudaStream_t st, P p) {
+  void* args[] = {&p};
+  return launch_status(cudaLaunchCooperativeKernel(kernel, dim3(grid), dim3(threads), args, smem, st));
 }
 
 }  // namespace ercg

@@ -489,19 +489,22 @@ static DagParams dag_params(const ercg_dag_layer* a, int UN) {
   return p;
 }
 
+// One cooperative launch of K.  The grid has at most one CTA per SM, so one CTA of K resident per SM, asked once per device
+// at the largest shared memory K may use, makes every size co-schedulable; no set-up call is made per launch, so a layer
+// can be captured in a CUDA graph.
+template <auto K>
+static int dag_launch(const ercg_dag_layer* a, int UN, int grid, size_t smem, void* stream) {
+  if (smem > (size_t)kMaxSmemPerBlock) return ERCG_ERANGE;
+  if (resident_capacity<K>(DT, kMaxSmemPerBlock) < 1) return ERCG_ECUDA;
+  return launch_cooperative(K, grid, DT, smem, (cudaStream_t)stream, dag_params(a, UN));
+}
+
 extern "C" int ercg_dag_layer_fwd(const ercg_dag_layer* args, void* stream) {
   int rc = dag_check(args, 0);
   if (rc <= 0) return rc;
   int grid = 0;
   const int UN = dag_units(args->D, &grid);
-  const size_t smem = dag_fwd_smem(args->D, UN);
-  if (smem > 227 * 1024) return ERCG_ERANGE;
-  if (cudaFuncSetAttribute(dag_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return ERCG_ECUDA;
-  DagParams p = dag_params(args, UN);
-  void* kargs[] = {&p};
-  cudaError_t err = cudaLaunchCooperativeKernel((const void*)dag_fwd_kernel, dim3(grid), dim3(DT), kargs, smem, (cudaStream_t)stream);
-  ++g_launches;
-  return err == cudaSuccess ? ERCG_OK : ERCG_ECUDA;
+  return dag_launch<dag_fwd_kernel>(args, UN, grid, dag_fwd_smem(args->D, UN), stream);
 }
 
 extern "C" int ercg_dag_layer_bwd(const ercg_dag_layer* args, void* stream) {
@@ -509,12 +512,5 @@ extern "C" int ercg_dag_layer_bwd(const ercg_dag_layer* args, void* stream) {
   if (rc <= 0) return rc;
   int grid = 0;
   const int UN = dag_units(args->D, &grid);
-  const size_t smem = dag_bwd_smem(args->D, UN);
-  if (smem > 227 * 1024) return ERCG_ERANGE;
-  if (cudaFuncSetAttribute(dag_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return ERCG_ECUDA;
-  DagParams p = dag_params(args, UN);
-  void* kargs[] = {&p};
-  cudaError_t err = cudaLaunchCooperativeKernel((const void*)dag_bwd_kernel, dim3(grid), dim3(DT), kargs, smem, (cudaStream_t)stream);
-  ++g_launches;
-  return err == cudaSuccess ? ERCG_OK : ERCG_ECUDA;
+  return dag_launch<dag_bwd_kernel>(args, UN, grid, dag_bwd_smem(args->D, UN), stream);
 }

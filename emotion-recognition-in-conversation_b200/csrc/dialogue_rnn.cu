@@ -509,38 +509,14 @@ static DrnnParams drnn_params(const ercg_dialogue_rnn* a) {
   return p;
 }
 
-constexpr int DRNN_SMEM_LIMIT = 227 * 1024;
-
-// CTAs of `kernel` resident per SM at the largest shared memory it may use, so a lower bound for every size; set up and
-// queried once per device (not per call, which may be inside a CUDA-graph capture).  0: it cannot be co-scheduled.
-static int drnn_capacity(const void* kernel, std::atomic<int>* cache) {
-  const int d = current_device();
-  if (d >= 0 && d < kMaxDevices) {
-    const int c = cache[d].load(std::memory_order_acquire);
-    if (c != 0) return c > 0 ? c : 0;
-  }
-  int n = 0;
-  if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, DRNN_SMEM_LIMIT) != cudaSuccess ||
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, RT, DRNN_SMEM_LIMIT) != cudaSuccess)
-    n = 0;
-  if (n == 0) cudaGetLastError();
-  if (d >= 0 && d < kMaxDevices) cache[d].store(n > 0 ? n : -1, std::memory_order_release);
-  return n;
-}
-
-static int drnn_launch(const void* kernel, std::atomic<int>* cache, const ercg_dialogue_rnn* a, size_t smem, int G,
-                       void* stream) {
-  if (smem > (size_t)DRNN_SMEM_LIMIT) return ERCG_ERANGE;
-  if (drnn_capacity(kernel, cache) < 1) return ERCG_ECUDA;
-  DrnnParams p = drnn_params(a);
-  void* kargs[] = {&p};
-  const cudaError_t err = cudaLaunchCooperativeKernel(kernel, dim3(G), dim3(RT), kargs, smem, (cudaStream_t)stream);
-  ++g_launches;
-  if (err != cudaSuccess) {
-    cudaGetLastError();
-    return ERCG_ECUDA;
-  }
-  return ERCG_OK;
+// CTAs of K resident per SM are asked at the largest shared memory it may use, so the answer is a lower bound for every
+// size; set up and queried once per device (not per call, which may be inside a CUDA-graph capture).  The grid has at most
+// one CTA per SM, so one resident CTA per SM makes it co-schedulable.
+template <auto K>
+static int drnn_launch(const ercg_dialogue_rnn* a, size_t smem, int G, void* stream) {
+  if (smem > (size_t)kMaxSmemPerBlock) return ERCG_ERANGE;
+  if (resident_capacity<K>(RT, kMaxSmemPerBlock) < 1) return ERCG_ECUDA;
+  return launch_cooperative(K, G, RT, smem, (cudaStream_t)stream, drnn_params(a));
 }
 
 }  // namespace ercg
@@ -551,14 +527,12 @@ extern "C" int ercg_dialogue_rnn_fwd(const ercg_dialogue_rnn* args, void* stream
   const int rc = drnn_check(args, 0);
   if (rc <= 0) return rc;
   const int G = drnn_grid(args);
-  static std::atomic<int> cache[kMaxDevices];
-  return drnn_launch((const void*)drnn_fwd_kernel, cache, args, drnn_fwd_smem(args, G), G, stream);
+  return drnn_launch<drnn_fwd_kernel>(args, drnn_fwd_smem(args, G), G, stream);
 }
 
 extern "C" int ercg_dialogue_rnn_bwd(const ercg_dialogue_rnn* args, void* stream) {
   const int rc = drnn_check(args, 1);
   if (rc <= 0) return rc;
   const int G = drnn_grid(args);
-  static std::atomic<int> cache[kMaxDevices];
-  return drnn_launch((const void*)drnn_bwd_kernel, cache, args, drnn_bwd_smem(args, G), G, stream);
+  return drnn_launch<drnn_bwd_kernel>(args, drnn_bwd_smem(args, G), G, stream);
 }

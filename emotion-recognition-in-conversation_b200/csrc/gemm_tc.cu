@@ -230,7 +230,7 @@ struct NnCfg {
   static constexpr int ACC_FULL = Q_FREE + Q;        // [2]
   static constexpr int ACC_EMPTY = ACC_FULL + 2;     // [2]
   static constexpr int COUNT = ACC_EMPTY + 2;
-  static_assert(SMEM_BYTES <= 232448, "shared memory budget");
+  static_assert(SMEM_BYTES <= kMaxSmemPerBlock, "shared memory budget");
   static_assert(COUNT * 8 + 8 <= 512, "barrier area");
 };
 constexpr uint32_t TC_SMEM_BYTES = NnCfg<false>::SMEM_BYTES;
@@ -876,7 +876,7 @@ struct TnCfg {
   static constexpr int W_FULL = 0, W_FREE = W_FULL + R, TA_FULL = W_FREE + R, TA_FREE = TA_FULL + TN_TA,
                        B_FULL = TA_FREE + TN_TA, B_SPLIT = B_FULL + Q, B_FREE = B_SPLIT + Q, ACC_FULL = B_FREE + Q,
                        ACC_EMPTY = ACC_FULL + 2, BARS = ACC_EMPTY + 2;
-  static_assert(SMEM_BYTES <= 232448, "shared memory budget");
+  static_assert(SMEM_BYTES <= kMaxSmemPerBlock, "shared memory budget");
   static_assert(BARS * 8 + 8 <= 512, "barrier area");
 };
 constexpr int TN_THREADS = 352;   // 4 splitter + 4 epilogue warps, W producer, MMA, narrow-operand producer
@@ -1282,34 +1282,10 @@ static bool tn_pairs_enabled() {
   static const bool on = [] { const char* e = getenv("ERCG_TN_PAIRS"); return !e || atoi(e) != 0; }();   // read once
   return on;
 }
-// CTA pairs that can be resident at once (1 CTA / SM, both SMs of a TPC): per-device, queried once.  A grid with more
-// clusters than this runs in two waves.
+// CTA pairs that can be resident at once (1 CTA / SM, both SMs of a TPC).  A grid with more clusters than this runs in
+// two waves.
 static int tn_pair_capacity() {
-  static std::atomic<int> cache[kMaxDevices];
-  const int d = current_device();
-  if (d >= 0 && d < kMaxDevices) {
-    const int c = cache[d].load(std::memory_order_acquire);
-    if (c != 0) return c > 0 ? c : 0;
-  }
-  int n = 0;
-  if (cudaFuncSetAttribute(gemm_tc_tn_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TnCfg<true>::SMEM_BYTES) == cudaSuccess) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(kNumSMs / 2 * 2, 1, 1);
-    cfg.blockDim = dim3(TN_THREADS, 1, 1);
-    cfg.dynamicSmemBytes = TnCfg<true>::SMEM_BYTES;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    if (cudaOccupancyMaxActiveClusters(&n, gemm_tc_tn_kernel<false, true>, &cfg) != cudaSuccess) { cudaGetLastError(); n = 0; }
-  } else {
-    cudaGetLastError();
-  }
-  if (d >= 0 && d < kMaxDevices) cache[d].store(n > 0 ? n : -1, std::memory_order_release);
-  return n;
+  return resident_capacity<gemm_tc_tn_kernel<false, true>, 2>(TN_THREADS, TnCfg<true>::SMEM_BYTES);
 }
 
 static void tn_tc_plan(int64_t M, int K1, int N1, bool& swap, int& w_tiles, int& n_tiles, int& bn, int& S, long long& rps,
@@ -1338,13 +1314,9 @@ static void tn_tc_plan(int64_t M, int K1, int N1, bool& swap, int& w_tiles, int&
 template <bool WBF16>
 static int tn_launch(bool two, const CUtensorMap& tmW, const CUtensorMap& tmN, float* P, long long M, int Wc, int Nc, int bn,
                      int wt, int nt, int S, long long rps, long long* tr, cudaStream_t st) {
-  static DeviceOnce attr_set;
-  if (attr_set.need()) {
-    if (cudaFuncSetAttribute(gemm_tc_tn_kernel<WBF16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TnCfg<false>::SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(gemm_tc_tn_kernel<WBF16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TnCfg<true>::SMEM_BYTES) != cudaSuccess)
-      return ERCG_ECUDA;
-    attr_set.mark();
-  }
+  if (!smem_limit<gemm_tc_tn_kernel<WBF16, false>>(TnCfg<false>::SMEM_BYTES) ||
+      !smem_limit<gemm_tc_tn_kernel<WBF16, true>>(TnCfg<true>::SMEM_BYTES))
+    return ERCG_ECUDA;
   if (!two) {
     const long long units = (long long)wt * nt * S;
     const int grid = (int)(units < kNumSMs ? units : kNumSMs);
@@ -1354,23 +1326,8 @@ static int tn_launch(bool two, const CUtensorMap& tmW, const CUtensorMap& tmN, f
   const long long units = (long long)(wt / 2) * nt * S;
   const int cap = tn_pair_capacity();
   const int pairs = (int)(units < cap ? units : cap);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * pairs, 1, 1);
-  cfg.blockDim = dim3(TN_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = TnCfg<true>::SMEM_BYTES;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  if (cudaLaunchKernelEx(&cfg, gemm_tc_tn_kernel<WBF16, true>, tmW, tmN, P, M, Wc, Nc, bn, wt, nt, S, rps, tr) != cudaSuccess) {
-    cudaGetLastError();
-    return ERCG_ECUDA;
-  }
-  return finish_launch();
+  return launch_cluster(gemm_tc_tn_kernel<WBF16, true>, 2, 2 * pairs, TN_THREADS, TnCfg<true>::SMEM_BYTES, st, tmW, tmN, P, M,
+                        Wc, Nc, bn, wt, nt, S, rps, tr);
 }
 
 // B[K,N] (row-major, ldb) -> Bt_hi [N, Kp] fp32 (K-major, tf32-rounded) and B16 [N, Kc, 64] bf16 (Kc = chunks of 32 k):
@@ -1478,33 +1435,18 @@ static bool nn_pairs_enabled() {
 }
 // CTA pairs of the NN kernel that can be resident at once (per device, queried once)
 static int nn_pair_capacity() {
-  static std::atomic<int> cache[kMaxDevices];
-  const int d = current_device();
-  if (d >= 0 && d < kMaxDevices) {
-    const int c = cache[d].load(std::memory_order_acquire);
-    if (c != 0) return c > 0 ? c : 0;
-  }
-  int n = 0;
-  auto kern = gemm_tc_nn_kernel<0, false, false, true, true>;
-  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, NnCfg<true>::SMEM_BYTES) == cudaSuccess) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(kNumSMs / 2 * 2, 1, 1);
-    cfg.blockDim = dim3(TC_THREADS, 1, 1);
-    cfg.dynamicSmemBytes = NnCfg<true>::SMEM_BYTES;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess) { cudaGetLastError(); n = 0; }
-  } else {
-    cudaGetLastError();
-  }
-  if (n > kNumSMs / 2) n = kNumSMs / 2;
-  if (d >= 0 && d < kMaxDevices) cache[d].store(n > 0 ? n : -1, std::memory_order_release);
-  return n;
+  const int n = resident_capacity<gemm_tc_nn_kernel<0, false, false, true, true>, 2>(TC_THREADS, NnCfg<true>::SMEM_BYTES);
+  return n < kNumSMs / 2 ? n : kNumSMs / 2;
+}
+
+// dynamic shared memory of every NN kernel of activation ACT (the tables in ercg_gemm_nn_tc)
+template <int ACT>
+static bool nn_smem_limits() {
+  return smem_limit<gemm_tc_nn_kernel<ACT, false, false>>(TC_SMEM_BYTES) &&
+         smem_limit<gemm_tc_nn_kernel<ACT, true, false>>(TC_SMEM_BYTES) &&
+         smem_limit<gemm_tc_nn_kernel<ACT, false, false, true, true>>(NnCfg<true, false>::SMEM_BYTES) &&
+         smem_limit<gemm_tc_nn_kernel<ACT, true, false, true>>(NnCfg<true, true>::SMEM_BYTES) &&
+         smem_limit<gemm_tc_nn_kernel<ACT, false, false, true>>(NnCfg<true, true>::SMEM_BYTES);
 }
 
 extern "C" size_t ercg_gemm_nn_tc_workspace_bytes(int N, int K) {
@@ -1570,19 +1512,7 @@ extern "C" int ercg_gemm_nn_tc(const float* A, int64_t lda, const float* B, int6
       {gemm_tc_nn_kernel<2, false, false, true, true>, gemm_tc_nn_kernel<2, true, false, true>, gemm_tc_nn_kernel<2, false, false, true>},
       {gemm_tc_nn_kernel<3, false, false, true, true>, gemm_tc_nn_kernel<3, true, false, true>, gemm_tc_nn_kernel<3, false, false, true>}};
   const int pair_kind = smallk ? 1 : ((K + TC_BK - 1) / TC_BK > 16 ? 0 : 2);
-  static DeviceOnce attr_set;            // cudaFuncSetAttribute is per device context: once per DEVICE, not per process
-  if (attr_set.need()) {
-    for (int i = 0; i < 4; ++i) {
-      for (int k = 0; k < 2; ++k)
-        if (cudaFuncSetAttribute(kernels[i][k], cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES) != cudaSuccess)
-          return ERCG_ECUDA;
-      if (cudaFuncSetAttribute(pair_kernels[i][0], cudaFuncAttributeMaxDynamicSharedMemorySize, NnCfg<true, false>::SMEM_BYTES) != cudaSuccess ||
-          cudaFuncSetAttribute(pair_kernels[i][1], cudaFuncAttributeMaxDynamicSharedMemorySize, NnCfg<true, true>::SMEM_BYTES) != cudaSuccess ||
-          cudaFuncSetAttribute(pair_kernels[i][2], cudaFuncAttributeMaxDynamicSharedMemorySize, NnCfg<true, true>::SMEM_BYTES) != cudaSuccess)
-        return ERCG_ECUDA;
-    }
-    attr_set.mark();
-  }
+  if (!nn_smem_limits<0>() || !nn_smem_limits<1>() || !nn_smem_limits<2>() || !nn_smem_limits<3>()) return ERCG_ECUDA;
   const int num_sms = device_sm_count();
   const int grid = two ? 2 * pair_cap : (int)(tiles < num_sms ? tiles : num_sms);
   static int dbg = -1;
@@ -1599,31 +1529,15 @@ extern "C" int ercg_gemm_nn_tc(const float* A, int64_t lda, const float* B, int6
   ep.seed_dev = reinterpret_cast<const unsigned long long*>(seed_dev);
   float* partial = colsum_out ? reinterpret_cast<float*>(b16 + (size_t)N * Kc * 64) : nullptr;   // [grid][4][128], after the B copies
   if (two) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid, 1, 1);
-    cfg.blockDim = dim3(TC_THREADS, 1, 1);
-    cfg.dynamicSmemBytes = pair_kind == 0 ? NnCfg<true, false>::SMEM_BYTES : NnCfg<true, true>::SMEM_BYTES;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    const long long ldc_ll = ldc, M_ll = M;
-    if (cudaLaunchKernelEx(&cfg, pair_kernels[act][pair_kind], tmA, tmBh, tmBl, tmC, C, ldc_ll, M_ll, N, K, bn, ep, partial) != cudaSuccess) {
-      cudaGetLastError();
-      return ERCG_ECUDA;
-    }
+    const int pair_smem = pair_kind == 0 ? NnCfg<true, false>::SMEM_BYTES : NnCfg<true, true>::SMEM_BYTES;
+    rc = launch_cluster(pair_kernels[act][pair_kind], 2, grid, TC_THREADS, pair_smem, st, tmA, tmBh, tmBl, tmC, C, ldc, M, N,
+                        K, bn, ep, partial);
   } else {
     kernels[act][smallk]<<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(tmA, tmBh, tmBl, tmC, C, ldc, M, N, K, bn, ep, partial);
-  }
-  if (colsum_out) {
     rc = finish_launch();
-    if (rc) return rc;
-    tc_colsum_final_kernel<<<fin_blocks(N), 256, 0, st>>>(partial, grid * 4, 128, N, colsum_out);
   }
+  if (rc || !colsum_out) return rc;
+  tc_colsum_final_kernel<<<fin_blocks(N), 256, 0, st>>>(partial, grid * 4, 128, N, colsum_out);
   return finish_launch();
 }
 
@@ -1752,12 +1666,8 @@ extern "C" int ercg_gemm_nn_tc_bf16a(const void* A_bf16, int64_t lda, const floa
   typedef void (*NnKernel)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, float*, long long, long long, int, int, int,
                            TcEpilogue, float*);
   static const NnKernel kernels[2] = {gemm_tc_nn_kernel<0, false, true>, gemm_tc_nn_kernel<0, true, true>};
-  static DeviceOnce attr_set;
-  if (attr_set.need()) {
-    for (int k = 0; k < 2; ++k)
-      if (cudaFuncSetAttribute(kernels[k], cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES) != cudaSuccess) return ERCG_ECUDA;
-    attr_set.mark();
-  }
+  if (!smem_limit<gemm_tc_nn_kernel<0, false, true>>(TC_SMEM_BYTES) || !smem_limit<gemm_tc_nn_kernel<0, true, true>>(TC_SMEM_BYTES))
+    return ERCG_ECUDA;
   const int num_sms = device_sm_count();
   const long long tiles = (M + TC_BM - 1) / TC_BM;
   const int grid = (int)(tiles < num_sms ? tiles : num_sms);

@@ -420,29 +420,13 @@ extern "C" int ercg_graphify_csr(const void* lengths_dev, int lengths_is_i64, in
   p.speakers = speakers_dev; p.spk64 = speakers_is_i64; p.spk_ld = spk_ld;
   p.wp = wp; p.wf = wf; p.n_speakers = n_speakers; p.N = N; p.E = E; p.o = *out;
   p.tile_agg = reinterpret_cast<long long*>(workspace);
-  // launch geometry is a property of the CURRENT device: cached per device id (read-mostly atomics, any thread may fill it)
-  static std::atomic<int> cache_bps[kMaxDevices], cache_sms[kMaxDevices];
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const int slot = (dev >= 0 && dev < kMaxDevices) ? dev : 0;
-  int max_blocks_per_sm = cache_bps[slot].load(std::memory_order_acquire);
-  int num_sms = cache_sms[slot].load(std::memory_order_acquire);
-  if (!max_blocks_per_sm || !num_sms || slot != dev) {
-    cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&max_blocks_per_sm, graphify_kernel, 256, 0);
-    if (max_blocks_per_sm < 1) max_blocks_per_sm = 1;
-    if (num_sms < 1) num_sms = kNumSMs;
-    cache_sms[slot].store(num_sms, std::memory_order_release);
-    cache_bps[slot].store(max_blocks_per_sm, std::memory_order_release);
-  }
+  const int num_sms = device_sm_count();
+  const int max_blocks_per_sm = resident_capacity<graphify_kernel>(256, 0);
+  if (max_blocks_per_sm < 1) return ERCG_ECUDA;
   long long want = (B + 7) / 8;                       // one warp per dialogue
   long long cap = (long long)max_blocks_per_sm * num_sms;
   int grid = (int)(want < 1 ? 1 : (want > cap ? cap : want));
-  void* args[] = {&p};
-  cudaError_t err = cudaLaunchCooperativeKernel((const void*)graphify_kernel, dim3(grid), dim3(256), args, 0,
-                                                (cudaStream_t)stream);
-  ++g_launches;
-  if (err != cudaSuccess) return ERCG_ECUDA;
+  if (int rc = launch_cooperative(graphify_kernel, grid, 256, 0, (cudaStream_t)stream, p)) return rc;
   if (out->rel_info) {
     if (E > 0) {
       const long long want_c = (E / 16 + 255) / 256;

@@ -27,7 +27,7 @@ namespace ercg {
 
 constexpr int RC_NB = 8;                 // lanes (dialogues) per cluster advanced in lockstep
 constexpr int RC_THREADS = 512;
-constexpr int RC_SMEM_LIMIT = 227 * 1024 - 1024;   // dynamic shared memory per CTA we allow (227 KB less the static part)
+constexpr int RC_SMEM_LIMIT = kMaxSmemPerBlock - 1024;   // dynamic shared memory per CTA we allow (less the static part)
 
 __device__ __forceinline__ float rc_sigmoid(float x) { return 1.f / (1.f + expf(-x)); }
 __device__ __forceinline__ uint32_t rc_smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -335,95 +335,47 @@ static int rc_cluster_size(int G, int Hd) {
   return rc_geom(G, Hd, 8, false, g) <= (size_t)RC_SMEM_LIMIT && rc_geom(G, Hd, 8, true, g) <= (size_t)RC_SMEM_LIMIT ? 8 : 16;
 }
 
-// Clusters of C CTAs of `kern` that can be resident at once, queried once per device (and per C) at the largest shared
-// memory the kernel is allowed, so it is a lower bound for every Hd.  0: this cluster shape cannot be scheduled.
-template <typename K>
-static int rc_capacity(K kern, int C, std::atomic<int>* cache) {
-  const int d = current_device();
-  if (d >= 0 && d < kMaxDevices) {
-    const int c = cache[d].load(std::memory_order_acquire);
-    if (c != 0) return c > 0 ? c : 0;
-  }
-  int n = 0;
-  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, RC_SMEM_LIMIT) == cudaSuccess &&
-      cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(C * 2, 1, 1);
-    cfg.blockDim = dim3(RC_THREADS, 1, 1);
-    cfg.dynamicSmemBytes = RC_SMEM_LIMIT;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = C;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess) n = 0;
-  }
-  if (n == 0) cudaGetLastError();
-  if (d >= 0 && d < kMaxDevices) cache[d].store(n > 0 ? n : -1, std::memory_order_release);
-  return n;
-}
-
 // One launch: the grid holds an even number of clusters (half per direction), at most what is resident at once and at
-// most one lane per dialogue.
-template <typename K, typename... Args>
-static int rc_launch(K kern, std::atomic<int> (*cache)[kMaxDevices], int G, int Hd, int B, bool bwd, cudaStream_t st,
-                     Args... args) {
+// most one lane per dialogue.  The resident count is asked at the largest shared memory the kernel is allowed, so it is a
+// lower bound for every Hd.
+template <auto K, typename... Args>
+static int rc_launch(int G, int Hd, int B, bool bwd, cudaStream_t st, Args... args) {
   RcGeom g;
   const int C = rc_cluster_size(G, Hd);
   const size_t smem = rc_geom(G, Hd, C, bwd, g);
   if (smem > (size_t)RC_SMEM_LIMIT) return ERCG_EINVAL;
-  const int cap = rc_capacity(kern, C, cache[C == 16]);
+  const int cap = C == 16 ? resident_capacity<K, 16>(RC_THREADS, RC_SMEM_LIMIT)
+                          : resident_capacity<K, 8>(RC_THREADS, RC_SMEM_LIMIT);
   if (cap < 1) return ERCG_ECUDA;
   const long long want = 2LL * ((B + RC_NB - 1) / RC_NB);
   int ncl = (int)(want < cap ? want : cap) & ~1;
   if (ncl < 2) ncl = 2;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(ncl * C, 1, 1);
-  cfg.blockDim = dim3(RC_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = C;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  if (cudaLaunchKernelEx(&cfg, kern, args..., g) != cudaSuccess) {
-    cudaGetLastError();
-    return ERCG_ECUDA;
-  }
-  return finish_launch();
+  return launch_cluster(K, C, ncl * C, RC_THREADS, smem, st, args..., g);
 }
-
-static std::atomic<int> g_cap_lstm_fwd[2][kMaxDevices], g_cap_lstm_bwd[2][kMaxDevices];
-static std::atomic<int> g_cap_gru_fwd[2][kMaxDevices], g_cap_gru_bwd[2][kMaxDevices];
 
 int lstm_cluster_fwd(const float* gx, long long ldgx, const float* whh, const int* node_off, int B, int Hd, float* out,
                      long long ldo, float* gates, float* cells, float* hprev, cudaStream_t st) {
-  return rc_launch(rnn_cluster_fwd_kernel<0>, g_cap_lstm_fwd, 4, Hd, B, false, st, gx, ldgx, whh, (const float*)nullptr,
-                   node_off, B, out, ldo, gates, cells, hprev);
+  return rc_launch<rnn_cluster_fwd_kernel<0>>(4, Hd, B, false, st, gx, ldgx, whh, (const float*)nullptr, node_off, B, out,
+                                              ldo, gates, cells, hprev);
 }
 
 int lstm_cluster_bwd(const float* dout, long long ldo, const float* gates, const float* cells, const float* whh,
                      const int* node_off, int B, int Hd, float* dgx, long long lddgx, cudaStream_t st) {
-  return rc_launch(rnn_cluster_bwd_kernel<0>, g_cap_lstm_bwd, 4, Hd, B, true, st, dout, ldo, gates, cells,
-                   (const float*)nullptr, whh, node_off, B, dgx, lddgx, (float*)nullptr, 0LL);
+  return rc_launch<rnn_cluster_bwd_kernel<0>>(4, Hd, B, true, st, dout, ldo, gates, cells, (const float*)nullptr, whh,
+                                              node_off, B, dgx, lddgx, (float*)nullptr, 0LL);
 }
 
 int gru_cluster_fwd(const float* gx, long long ldgx, const float* whh, const float* bhh, const int* node_off, int B, int Hd,
                     float* out, long long ldo, float* gates, float* hprev, cudaStream_t st) {
-  return rc_launch(rnn_cluster_fwd_kernel<1>, g_cap_gru_fwd, 3, Hd, B, false, st, gx, ldgx, whh, bhh, node_off, B, out, ldo,
-                   gates, (float*)nullptr, hprev);
+  return rc_launch<rnn_cluster_fwd_kernel<1>>(3, Hd, B, false, st, gx, ldgx, whh, bhh, node_off, B, out, ldo, gates,
+                                              (float*)nullptr, hprev);
 }
 
 int gru_cluster_bwd(const float* dout, long long ldo, const float* gates, const float* hprev, const float* whh,
                     const int* node_off, int B, int Hd, float* dgx, long long lddgx, float* dgh, long long lddgh,
                     cudaStream_t st) {
-  return rc_launch(rnn_cluster_bwd_kernel<1>, g_cap_gru_bwd, 3, Hd, B, true, st, dout, ldo, gates, (const float*)nullptr,
-                   hprev, whh, node_off, B, dgx, lddgx, dgh, lddgh);
+  return rc_launch<rnn_cluster_bwd_kernel<1>>(3, Hd, B, true, st, dout, ldo, gates, (const float*)nullptr, hprev, whh,
+                                              node_off, B, dgx, lddgx, dgh, lddgh);
 }
 
 }  // namespace ercg

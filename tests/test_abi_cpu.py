@@ -60,6 +60,23 @@ def test_ctypes_table_mirrors_the_header():
     assert fields == re.findall(r"\*\s*(\w+)\s*;", body)
 
 
+def test_launch_setup_only_in_common_cuh():
+    """Shared-memory limits, residency queries and cluster / cooperative launches go through the helpers of
+    csrc/common.cuh, so every kernel sets them up once per device, clears the error of a failed launch and counts it."""
+    csrc = os.path.join(ROOT, "emotion-recognition-in-conversation_b200", "csrc")
+    setup = re.compile(r"\b(cudaFuncSetAttribute|cudaOccupancyMaxActiveBlocksPerMultiprocessor|cudaOccupancyMaxActiveClusters|"
+                       r"cudaLaunchKernelEx|cudaLaunchCooperativeKernel)\b|\[\s*kMaxDevices\s*\]")
+    found = {}
+    for name in sorted(os.listdir(csrc)):
+        if not name.endswith((".cu", ".cuh")):
+            continue
+        src = open(os.path.join(csrc, name)).read()
+        src = re.sub(r"//[^\n]*", " ", re.sub(r"/\*.*?\*/", " ", src, flags=re.S))
+        found[name] = {m.group(0) for m in setup.finditer(src)}
+    assert found["common.cuh"] >= {"cudaFuncSetAttribute", "cudaOccupancyMaxActiveClusters", "cudaLaunchKernelEx"}
+    assert not {n: sorted(f) for n, f in found.items() if f and n != "common.cuh"}
+
+
 def test_host_only_entry_points():
     import erc_b200
     from erc_b200 import _lib

@@ -182,3 +182,42 @@ def test_gat_dialoggcn_v1_standalone_forward_backward_vs_oracle(B, N, D):
         out.update({"d" + n: p.grad.cpu().numpy() for n, p in mod.named_parameters()})
         res.append(out)
     parity_check("dagerc/gat_standalone/B%d_N%d_D%d" % (B, N, D), res[2], res[0], res[1])
+
+
+def test_dag_layer_graph_capture_bit_equal_to_eager():
+    """One K10 layer forward + backward captured in a CUDA graph and replayed: the output and every gradient are bit-equal
+    to the eager run (the layer's launch set-up is done once per device, not inside the capture)."""
+    import erc_b200  # noqa: F401
+    from erc_b200 import ops_dagerc
+    from erc_b200.graph import build_graph
+    from erc_b200.track_mm.dagerc_models import GAT_dialoggcn_v1
+    gen = torch.Generator().manual_seed(7)
+    lengths = torch.tensor([30, 17, 1, 44, 8])
+    D, N = 300, int(lengths.sum())
+    spk = torch.randint(0, 2, (lengths.numel(), int(lengths.max())), generator=gen)
+    g = build_graph(lengths, spk.cuda(), 0, 0, 2, reference_layout=False, mean_weight=False)
+    dag = ops_dagerc.DagStructure(g, lengths, 1)                   # holds the one host sync: built before the capture
+    torch.manual_seed(7)
+    gat, gru_c, gru_p = GAT_dialoggcn_v1(D).cuda(), torch.nn.GRUCell(D, D).cuda(), torch.nn.GRUCell(D, D).cuda()
+    H = torch.randn(N, D, generator=gen).cuda().requires_grad_()
+    dout = torch.randn(N, D, generator=gen).cuda()
+    wrt = [H, *gat.parameters(), *gru_c.parameters(), *gru_p.parameters()]
+
+    def fwd_bwd():
+        out = ops_dagerc.dag_layer(H, gat, gru_c, gru_p, dag)
+        return (out.detach(), *torch.autograd.grad(out, wrt, dout))
+
+    a = fwd_bwd()
+    assert all(torch.isfinite(x).all() for x in a)
+    s = torch.cuda.Stream()
+    s.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(s):
+        fwd_bwd()
+    torch.cuda.current_stream().wait_stream(s)
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        c = fwd_bwd()
+    graph.replay()
+    torch.cuda.synchronize()
+    assert len(c) == len(wrt) + 1
+    assert all(torch.equal(x, y) for x, y in zip(a, c))
