@@ -6,56 +6,88 @@
 // K5 = EdgeAtt of DialogueGCN (track_mm/dgcn_models.py:121-152): the same score/softmax machinery
 //   normalised over the OUT-edges of each source (by-source traversal), no value aggregation.
 //
-// One warp per node, lane c owns float4 chunk(s) of the H-wide rows.  Scores of up to 32 edges are
-// kept one-per-lane in a register (deg <= 11 / 21 for the reference's windows); longer rows fall back
-// to an online (running max / rescale) chunked loop.  Score, softmax and aggregation are one kernel:
-// k_j and v_j rows are read once per edge from L1/L2, q_i/s_i/out_i once per node from HBM.
+// Warp-per-node kernels (any graph, any even H <= 1024, 8-byte aligned rows): one warp per node, lane l holds its part of
+// an H-wide row as NC chunks of type V, chunk c = elements [CW * (l + 32c), CW * (l + 32c) + CW).  V = float4 (CW = 4) when
+// H % 4 == 0 and every row is 16-byte aligned with ld % 4 == 0, float2 (CW = 2) otherwise (e.g. the key half of dgcnv2's
+// [xt | e] at odd hidden sizes); ERCG_LAUNCH_NC picks V and NC from H and the operands.  Scores of up to 32 edges are
+// kept one-per-lane in a register (deg <= 11 / 21 for the reference's windows); longer rows fall back to an online
+// (running max / rescale) chunked loop.  Score, softmax and aggregation are one kernel: k_j and v_j rows are read once per
+// edge from L1/L2, q_i/s_i/out_i once per node from HBM.  All sums keep a fixed order (per lane over chunks, then the
+// butterfly), so results are bit-reproducible and independent of the grid.
 // Algorithmic HBM bytes per node (SURVEY.md 8d): 5*4H (q,k,v,s,out) + 4 (rowptr) + 8*deg (col, alpha).
-// The float4 kernels here take H <= 384, H % 4 == 0 and 16-byte aligned rows; attn_wide.cuh runs the same algorithm for
-// every other even H <= 1024 and for 8-byte aligned rows (float4 or float2 chunks, chosen from H and the operands).
+// The ercg_attn_window_* entry points run CTA tile kernels instead: attn_blk.cuh's for windows of up to 16 candidates, the
+// round-1 tile kernels below for wider ones.
 #include "common.cuh"
 #include "attn_blk.cuh"
 #include <math.h>
 #include <stdlib.h>
+#include <type_traits>
 
 namespace ercg {
 
 constexpr int AW = 8;
+// Minimum resident CTAs per SM the warp-per-node kernels are compiled for: the float4 NC <= 3 instantiations were tuned
+// without a block count (0), the wider ones spill without one (ptxas held some at 48-64 registers; with 2, none spills).
+template <typename V, int NC>
+constexpr int node_min_blocks = std::is_same<V, float4>::value && NC <= 3 ? 0 : 2;
 
-template <int NC>
-__device__ __forceinline__ void load_row(const float* p, int nch, int lane, float4 r[NC]) {
+template <typename V> struct Chunk;
+template <> struct Chunk<float4> { static constexpr int SH = 2; };
+template <> struct Chunk<float2> { static constexpr int SH = 1; };
+template <typename V> __device__ __forceinline__ V ldv(const float* p);
+template <> __device__ __forceinline__ float4 ldv<float4>(const float* p) { return ld4(p); }
+template <> __device__ __forceinline__ float2 ldv<float2>(const float* p) { return *reinterpret_cast<const float2*>(p); }
+template <typename V> __device__ __forceinline__ V zerov();
+template <> __device__ __forceinline__ float4 zerov<float4>() { return make_float4(0.f, 0.f, 0.f, 0.f); }
+template <> __device__ __forceinline__ float2 zerov<float2>() { return make_float2(0.f, 0.f); }
+__device__ __forceinline__ void stv(float* p, float4 v) { st4(p, v); }
+__device__ __forceinline__ void stv(float* p, float2 v) { *reinterpret_cast<float2*>(p) = v; }
+__device__ __forceinline__ float dotv(const float4& a, const float4& b) { return dot4(a, b); }
+__device__ __forceinline__ float dotv(const float2& a, const float2& b) { return fmaf(a.x, b.x, a.y * b.y); }
+__device__ __forceinline__ void fmav(float4& a, float s, const float4& b) { fma4(a, s, b); }
+__device__ __forceinline__ void fmav(float2& a, float s, const float2& b) { a.x = fmaf(s, b.x, a.x); a.y = fmaf(s, b.y, a.y); }
+__device__ __forceinline__ void scalev(float4& a, float s) { a.x *= s; a.y *= s; a.z *= s; a.w *= s; }
+__device__ __forceinline__ void scalev(float2& a, float s) { a.x *= s; a.y *= s; }
+__device__ __forceinline__ void addv(float4& a, const float4& b) { a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w; }
+__device__ __forceinline__ void addv(float2& a, const float2& b) { a.x += b.x; a.y += b.y; }
+
+template <typename V, int NC>
+__device__ __forceinline__ void load_row(const float* p, int nch, int lane, V r[NC]) {
+  constexpr int CW = 1 << Chunk<V>::SH;
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
     const int ch = lane + 32 * c;
-    r[c] = ch < nch ? ld4(p + 4 * ch) : make_float4(0.f, 0.f, 0.f, 0.f);
+    r[c] = ch < nch ? ldv<V>(p + CW * ch) : zerov<V>();
   }
 }
-template <int NC>
-__device__ __forceinline__ float row_dot(const float4 a[NC], const float* p, int nch, int lane) {
+template <typename V, int NC>
+__device__ __forceinline__ float row_dot(const V a[NC], const float* p, int nch, int lane) {
+  constexpr int CW = 1 << Chunk<V>::SH;
   float s = 0.f;
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
     const int ch = lane + 32 * c;
-    if (ch < nch) s += dot4(a[c], ld4(p + 4 * ch));
+    if (ch < nch) s += dotv(a[c], ldv<V>(p + CW * ch));
   }
   return warp_sum(s);
 }
 
 // <a, row_q> for 4 rows at once: the 4 row loads are issued back to back, the 4 reductions interleave.
 // Rows with live[q] == false are not read (warp-uniform) and yield 0.
-template <int NC>
-__device__ __forceinline__ void row_dot4(const float4 a[NC], const float* const p[4], const bool live[4], int nch, int lane,
+template <typename V, int NC>
+__device__ __forceinline__ void row_dot4(const V a[NC], const float* const p[4], const bool live[4], int nch, int lane,
                                          float out[4]) {
+  constexpr int CW = 1 << Chunk<V>::SH;
   float s[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
     const int ch = lane + 32 * c;
     if (ch < nch) {
-      float4 v[4];
+      V v[4];
 #pragma unroll
-      for (int q = 0; q < 4; ++q) v[q] = live[q] ? ld4(p[q] + 4 * ch) : make_float4(0.f, 0.f, 0.f, 0.f);
+      for (int q = 0; q < 4; ++q) v[q] = live[q] ? ldv<V>(p[q] + CW * ch) : zerov<V>();
 #pragma unroll
-      for (int q = 0; q < 4; ++q) s[q] += dot4(a[c], v[q]);
+      for (int q = 0; q < 4; ++q) s[q] += dotv(a[c], v[q]);
     }
   }
 #pragma unroll
@@ -67,36 +99,38 @@ __device__ __forceinline__ void row_dot4(const float4 a[NC], const float* const 
   for (int q = 0; q < 4; ++q) out[q] = s[q];
 }
 // acc += sum_q w[q] * row_q (4 rows in flight)
-template <int NC>
-__device__ __forceinline__ void row_axpy4(float4 acc[NC], const float w[4], const float* const p[4], const bool live[4],
+template <typename V, int NC>
+__device__ __forceinline__ void row_axpy4(V acc[NC], const float w[4], const float* const p[4], const bool live[4],
                                           int nch, int lane) {
+  constexpr int CW = 1 << Chunk<V>::SH;
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
     const int ch = lane + 32 * c;
     if (ch < nch) {
-      float4 v[4];
+      V v[4];
 #pragma unroll
-      for (int q = 0; q < 4; ++q) v[q] = live[q] ? ld4(p[q] + 4 * ch) : make_float4(0.f, 0.f, 0.f, 0.f);
+      for (int q = 0; q < 4; ++q) v[q] = live[q] ? ldv<V>(p[q] + CW * ch) : zerov<V>();
 #pragma unroll
-      for (int q = 0; q < 4; ++q) fma4(acc[c], w[q], v[q]);
+      for (int q = 0; q < 4; ++q) fmav(acc[c], w[q], v[q]);
     }
   }
 }
 
-template <int NC>
-__global__ void __launch_bounds__(AW * 32)
+template <typename V, int NC>
+__global__ void __launch_bounds__(AW * 32, node_min_blocks<V, NC>)
 attn_fwd_kernel(const float* __restrict__ q, const float* __restrict__ k, const float* __restrict__ v,
                 const float* __restrict__ s, long long ld, const int* __restrict__ rowptr,
                 const int* __restrict__ col, float scale, float* __restrict__ out, long long ldo,
                 float* __restrict__ alpha, float* __restrict__ dact, long long N, int H) {
+  constexpr int CW = 1 << Chunk<V>::SH;
   const int lane = threadIdx.x & 31;
   const long long node = (long long)blockIdx.x * AW + (threadIdx.x >> 5);
   if (node >= N) return;
-  const int nch = H >> 2;
-  float4 qi[NC], acc[NC];
-  load_row<NC>(q + node * ld, nch, lane, qi);
+  const int nch = H >> Chunk<V>::SH;
+  V qi[NC], acc[NC];
+  load_row<V, NC>(q + node * ld, nch, lane, qi);
 #pragma unroll
-  for (int c = 0; c < NC; ++c) acc[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int c = 0; c < NC; ++c) acc[c] = zerov<V>();
   const int beg = rowptr[node], end = rowptr[node + 1];
   float run_max = -INFINITY, run_sum = 0.f;
   for (int cb = beg; cb < end; cb += 32) {
@@ -112,7 +146,7 @@ attn_fwd_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
         live[qq] = u + qq < cn;
         p[qq] = k + (long long)__shfl_sync(0xffffffffu, mc, min(u + qq, cn - 1)) * ld;
       }
-      row_dot4<NC>(qi, p, live, nch, lane, d);
+      row_dot4<V, NC>(qi, p, live, nch, lane, d);
 #pragma unroll
       for (int qq = 0; qq < 4; ++qq)
         if (lane == u + qq) my = d[qq] * scale;
@@ -127,7 +161,7 @@ attn_fwd_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
     const float ex = lane < cn ? expf(my - new_max) : 0.f;
     run_sum = run_sum * resc + warp_sum(ex);
 #pragma unroll
-    for (int c = 0; c < NC; ++c) { acc[c].x *= resc; acc[c].y *= resc; acc[c].z *= resc; acc[c].w *= resc; }
+    for (int c = 0; c < NC; ++c) scalev(acc[c], resc);
     if (alpha && lane < cn) alpha[cb + lane] = ex;        // un-normalised, relative to new_max; fixed below
     if (alpha && cb > beg && resc != 1.f) {               // rescale earlier chunks (rare: deg > 32)
       for (int e2 = beg + lane; e2 < cb; e2 += 32) alpha[e2] *= resc;
@@ -143,7 +177,7 @@ attn_fwd_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
         a[qq] = __shfl_sync(0xffffffffu, ex, l);
         p[qq] = v + (long long)__shfl_sync(0xffffffffu, mc, l) * ld;
       }
-      row_axpy4<NC>(acc, a, p, live, nch, lane);
+      row_axpy4<V, NC>(acc, a, p, live, nch, lane);
     }
     run_max = new_max;
   }
@@ -156,32 +190,30 @@ attn_fwd_kernel(const float* __restrict__ q, const float* __restrict__ k, const 
   for (int c = 0; c < NC; ++c) {
     const int ch = lane + 32 * c;
     if (ch < nch) {
-      float4 r = acc[c];
-      r.x *= inv; r.y *= inv; r.z *= inv; r.w *= inv;
-      if (s) {
-        const float4 sk = ld4(s + node * ld + 4 * ch);
-        r.x += sk.x; r.y += sk.y; r.z += sk.z; r.w += sk.w;
-      }
-      st4(out + node * ldo + 4 * ch, r);
+      V r = acc[c];
+      scalev(r, inv);
+      if (s) addv(r, ldv<V>(s + node * ld + CW * ch));
+      stv(out + node * ldo + CW * ch, r);
     }
   }
 }
 
 // by-destination backward: dalpha_e = <dout_i, v_j>, D = sum alpha dalpha, dsig_e = alpha_e (dalpha_e - D),
 // dq_i = scale * sum dsig_e k_j, ds_i = dout_i
-template <int NC>
-__global__ void __launch_bounds__(AW * 32)
+template <typename V, int NC>
+__global__ void __launch_bounds__(AW * 32, node_min_blocks<V, NC>)
 attn_bwd_dst_kernel(const float* __restrict__ dout, long long ldo, const float* __restrict__ k,
                     const float* __restrict__ v, long long ld, const int* __restrict__ rowptr,
                     const int* __restrict__ col, const float* __restrict__ alpha, float scale,
                     float* __restrict__ dq, float* __restrict__ ds, long long ldd, float* __restrict__ dsig,
                     const float* __restrict__ dact, long long N, int H) {
+  constexpr int CW = 1 << Chunk<V>::SH;
   const int lane = threadIdx.x & 31;
   const long long node = (long long)blockIdx.x * AW + (threadIdx.x >> 5);
   if (node >= N) return;
-  const int nch = H >> 2;
-  float4 go[NC], acc[NC];
-  load_row<NC>(dout + node * ldo, nch, lane, go);
+  const int nch = H >> Chunk<V>::SH;
+  V go[NC], acc[NC];
+  load_row<V, NC>(dout + node * ldo, nch, lane, go);
   const int beg = rowptr[node], end = rowptr[node + 1];
   if (end - beg <= 32) {
     // common case: every per-edge scalar of the row lives in one lane; no round trip through the dsig buffer
@@ -198,7 +230,7 @@ attn_bwd_dst_kernel(const float* __restrict__ dout, long long ldo, const float* 
         live[qq] = u + qq < cn;
         p[qq] = v + (long long)__shfl_sync(0xffffffffu, mc, min(u + qq, cn - 1)) * ld;
       }
-      row_dot4<NC>(go, p, live, nch, lane, d);
+      row_dot4<V, NC>(go, p, live, nch, lane, d);
 #pragma unroll
       for (int qq = 0; qq < 4; ++qq)
         if (lane == u + qq) my = d[qq];
@@ -208,7 +240,7 @@ attn_bwd_dst_kernel(const float* __restrict__ dout, long long ldo, const float* 
     if (dact && lane < cn) g *= dact[beg + lane];
     if (lane < cn) dsig[beg + lane] = g;
 #pragma unroll
-    for (int c = 0; c < NC; ++c) acc[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+    for (int c = 0; c < NC; ++c) acc[c] = zerov<V>();
     for (int u = 0; u < cn; u += 4) {
       const float* p[4];
       bool live[4];
@@ -220,14 +252,14 @@ attn_bwd_dst_kernel(const float* __restrict__ dout, long long ldo, const float* 
         gw[qq] = __shfl_sync(0xffffffffu, g, l) * scale;
         p[qq] = k + (long long)__shfl_sync(0xffffffffu, mc, l) * ld;
       }
-      row_axpy4<NC>(acc, gw, p, live, nch, lane);
+      row_axpy4<V, NC>(acc, gw, p, live, nch, lane);
     }
 #pragma unroll
     for (int c = 0; c < NC; ++c) {
       const int ch = lane + 32 * c;
       if (ch < nch) {
-        st4(dq + node * ldd + 4 * ch, acc[c]);
-        if (ds) st4(ds + node * ldd + 4 * ch, go[c]);
+        stv(dq + node * ldd + CW * ch, acc[c]);
+        if (ds) stv(ds + node * ldd + CW * ch, go[c]);
       }
     }
     return;
@@ -238,7 +270,7 @@ attn_bwd_dst_kernel(const float* __restrict__ dout, long long ldo, const float* 
     const int cn = min(32, end - cb);
     float my = 0.f;
     for (int u = 0; u < cn; ++u) {
-      const float d = row_dot<NC>(go, v + (long long)col[cb + u] * ld, nch, lane);
+      const float d = row_dot<V, NC>(go, v + (long long)col[cb + u] * ld, nch, lane);
       if (lane == u) my = d;
     }
     const float a = lane < cn ? alpha[cb + lane] : 0.f;
@@ -247,7 +279,7 @@ attn_bwd_dst_kernel(const float* __restrict__ dout, long long ldo, const float* 
   }
   __syncwarp();
 #pragma unroll
-  for (int c = 0; c < NC; ++c) acc[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int c = 0; c < NC; ++c) acc[c] = zerov<V>();
   for (int cb = beg; cb < end; cb += 32) {
     const int cn = min(32, end - cb);
     float g = 0.f;
@@ -262,7 +294,7 @@ attn_bwd_dst_kernel(const float* __restrict__ dout, long long ldo, const float* 
 #pragma unroll
       for (int c = 0; c < NC; ++c) {
         const int ch = lane + 32 * c;
-        if (ch < nch) fma4(acc[c], gu, ld4(pk + 4 * ch));
+        if (ch < nch) fmav(acc[c], gu, ldv<V>(pk + CW * ch));
       }
     }
   }
@@ -270,26 +302,27 @@ attn_bwd_dst_kernel(const float* __restrict__ dout, long long ldo, const float* 
   for (int c = 0; c < NC; ++c) {
     const int ch = lane + 32 * c;
     if (ch < nch) {
-      st4(dq + node * ldd + 4 * ch, acc[c]);
-      if (ds) st4(ds + node * ldd + 4 * ch, go[c]);
+      stv(dq + node * ldd + CW * ch, acc[c]);
+      if (ds) stv(ds + node * ldd + CW * ch, go[c]);
     }
   }
 }
 
 // by-source backward: dk_j = scale * sum_i dsig[j->i] q_i,  dv_j = sum_i alpha[j->i] dout_i
-template <int NC>
-__global__ void __launch_bounds__(AW * 32)
+template <typename V, int NC>
+__global__ void __launch_bounds__(AW * 32, node_min_blocks<V, NC>)
 attn_bwd_src_kernel(const float* __restrict__ dout, long long ldo, const float* __restrict__ q, long long ld,
                     const int* __restrict__ t_rowptr, const int* __restrict__ t_col, const int* __restrict__ t_eid,
                     const float* __restrict__ alpha, const float* __restrict__ dsig, float scale,
                     float* __restrict__ dk, float* __restrict__ dv, long long ldd, long long N, int H) {
+  constexpr int CW = 1 << Chunk<V>::SH;
   const int lane = threadIdx.x & 31;
   const long long node = (long long)blockIdx.x * AW + (threadIdx.x >> 5);
   if (node >= N) return;
-  const int nch = H >> 2;
-  float4 ak[NC], av[NC];
+  const int nch = H >> Chunk<V>::SH;
+  V ak[NC], av[NC];
 #pragma unroll
-  for (int c = 0; c < NC; ++c) { ak[c] = make_float4(0.f, 0.f, 0.f, 0.f); av[c] = ak[c]; }
+  for (int c = 0; c < NC; ++c) { ak[c] = zerov<V>(); av[c] = ak[c]; }
   const int beg = t_rowptr[node], end = t_rowptr[node + 1];
   for (int e = beg; e < end; ++e) {
     const int i = t_col[e], id = t_eid[e];
@@ -300,8 +333,8 @@ attn_bwd_src_kernel(const float* __restrict__ dout, long long ldo, const float* 
     for (int c = 0; c < NC; ++c) {
       const int ch = lane + 32 * c;
       if (ch < nch) {
-        fma4(ak[c], g, ld4(pq + 4 * ch));
-        fma4(av[c], a, ld4(pd + 4 * ch));
+        fmav(ak[c], g, ldv<V>(pq + CW * ch));
+        fmav(av[c], a, ldv<V>(pd + CW * ch));
       }
     }
   }
@@ -309,8 +342,8 @@ attn_bwd_src_kernel(const float* __restrict__ dout, long long ldo, const float* 
   for (int c = 0; c < NC; ++c) {
     const int ch = lane + 32 * c;
     if (ch < nch) {
-      st4(dk + node * ldd + 4 * ch, ak[c]);
-      st4(dv + node * ldd + 4 * ch, av[c]);
+      stv(dk + node * ldd + CW * ch, ak[c]);
+      stv(dv + node * ldd + CW * ch, av[c]);
     }
   }
 }
@@ -320,7 +353,7 @@ attn_bwd_src_kernel(const float* __restrict__ dout, long long ldo, const float* 
 // per node at 63 % issue utilisation and 55 % occupancy -- issue- and latency-bound, DRAM at 20-30 %.  For the graphs
 // K1 builds, the neighbours of node i are the contiguous rows [i - wlo, i + whi] of its dialogue, so a CTA that owns 32
 // consecutive nodes needs only the 32 + wlo + whi rows around them.  These kernels stage those rows of k / v (and q or
-// dout) in shared memory with plain coalesced loads (all global latency is paid once, in parallel), then
+// dout) in shared memory with coalesced cp.async copies (blk_stage_rows; all global latency is paid once, in parallel), then
 //   * scores / dalpha: ONE LANE PER EDGE walks the 25 float4 chunks of "its" neighbour row in shared memory -- no
 //     shuffle reduction at all; two nodes share a warp (16 lanes each) when wlo + whi + 1 <= 16,
 //   * aggregation: one lane per float4 chunk, per-edge scalars broadcast by shuffle.
@@ -330,40 +363,6 @@ attn_bwd_src_kernel(const float* __restrict__ dout, long long ldo, const float* 
 #define ATTN_WT_ 32
 #endif
 constexpr int WT = ATTN_WT_;  // nodes per CTA tile
-
-// Rows go global -> shared with 16-byte cp.async (LDGSTS): a lane issues all of its ~15 row chunks back to back, no
-// registers are tied up and nobody waits until stage_wait(), so the whole tile's HBM latency is paid once and the CSR
-// metadata loads issued right after overlap with it.  (The first version staged through registers -- ptxas kept only four
-// loads in flight per lane -- and ran at 35-40 % of the HBM peak.)
-__device__ __forceinline__ void stage_rows(float4* dst, const float* __restrict__ src, long long ld, long long r0, int rows,
-                                           int nch) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (lane < nch)
-    for (int r = warp; r < rows; r += 8) {
-      const uint32_t d = (uint32_t)__cvta_generic_to_shared(dst + r * nch + lane);
-      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(src + (r0 + r) * ld + 4 * lane) : "memory");
-    }
-}
-__device__ __forceinline__ void stage_wait() {
-  asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
-  __syncthreads();
-}
-template <bool PAIR>
-__device__ __forceinline__ float half_max(float v) {
-  if (!PAIR) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 16));
-  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 8));
-  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 4));
-  v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 2));
-  return fmaxf(v, __shfl_xor_sync(0xffffffffu, v, 1));
-}
-template <bool PAIR>
-__device__ __forceinline__ float half_sum(float v) {
-  if (!PAIR) v += __shfl_xor_sync(0xffffffffu, v, 16);
-  v += __shfl_xor_sync(0xffffffffu, v, 8);
-  v += __shfl_xor_sync(0xffffffffu, v, 4);
-  v += __shfl_xor_sync(0xffffffffu, v, 2);
-  return v + __shfl_xor_sync(0xffffffffu, v, 1);
-}
 
 // per-CTA column sums of two H-wide outputs: lane = float4 chunk, warps reduced in warp order through the staging buffer
 // (8 KB of it, reused once every warp is done with the staged rows -- no extra shared memory, so occupancy is unchanged)
@@ -399,9 +398,9 @@ attn_fwd_tile_kernel(const float* __restrict__ q, const float* __restrict__ k, c
   float4* sq = attn_sm;
   float4* sk = sq + WT * nch;
   float4* sv = sk + Rmax * nch;
-  stage_rows(sq, q, ld, t0, tn, nch);
-  stage_rows(sk, k, ld, r0, R, nch);
-  stage_rows(sv, v, ld, r0, R, nch);
+  blk_stage_rows<256>(sq, q, ld, t0, tn, nch);
+  blk_stage_rows<256>(sk, k, ld, r0, R, nch);
+  blk_stage_rows<256>(sv, v, ld, r0, R, nch);
   constexpr int NPW = WT / 8;                 // nodes per warp
   constexpr int G = PAIR ? 2 : 1;             // nodes handled together in the score phase
   constexpr int IT = NPW / G;
@@ -432,7 +431,7 @@ attn_fwd_tile_kernel(const float* __restrict__ q, const float* __restrict__ k, c
     const int nl = warp * NPW + h;
     skip[h] = (s && nl < tn && lane < nch) ? ld4(s + (t0 + nl) * ld + 4 * lane) : make_float4(0.f, 0.f, 0.f, 0.f);
   }
-  stage_wait();
+  cp_wait_all();
 #pragma unroll
   for (int it = 0; it < IT; ++it) {
     const int p = it * G;
@@ -447,9 +446,10 @@ attn_fwd_tile_kernel(const float* __restrict__ q, const float* __restrict__ k, c
       for (int c = 0; c < nch; ++c) d += dot4(qi[c], kr[c]);
     }
     d *= scale;
-    const float mx = half_max<PAIR>(live ? d : -INFINITY);
+    const float x = live ? d : -INFINITY;
+    const float mx = PAIR ? h16_max(x) : warp_max(x);
     const float ex = live ? expf(d - mx) : 0.f;
-    const float inv = 1.f / (half_sum<PAIR>(ex) + 1e-16f);
+    const float inv = 1.f / ((PAIR ? h16_sum(ex) : warp_sum(ex)) + 1e-16f);
     const float al = ex * inv;
     if (live && alpha) alpha[beg + e] = al;
     // aggregation: lanes = float4 chunks, one node after the other
@@ -491,9 +491,9 @@ attn_bwd_dst_tile_kernel(const float* __restrict__ dout, long long ldo, const fl
   float4* sd = attn_sm;
   float4* sk = sd + WT * nch;
   float4* sv = sk + Rmax * nch;
-  stage_rows(sd, dout, ldo, t0, tn, nch);
-  stage_rows(sk, k, ld, r0, R, nch);
-  stage_rows(sv, v, ld, r0, R, nch);
+  blk_stage_rows<256>(sd, dout, ldo, t0, tn, nch);
+  blk_stage_rows<256>(sk, k, ld, r0, R, nch);
+  blk_stage_rows<256>(sv, v, ld, r0, R, nch);
   constexpr int NPW = WT / 8;
   constexpr int G = PAIR ? 2 : 1;
   constexpr int IT = NPW / G;
@@ -518,7 +518,7 @@ attn_bwd_dst_tile_kernel(const float* __restrict__ dout, long long ldo, const fl
       als[it] = alpha[begs[it] + e];
     }
   }
-  stage_wait();
+  cp_wait_all();
 #pragma unroll
   for (int it = 0; it < IT; ++it) {
     const int p = it * G;
@@ -533,7 +533,8 @@ attn_bwd_dst_tile_kernel(const float* __restrict__ dout, long long ldo, const fl
 #pragma unroll 5
       for (int c = 0; c < nch; ++c) da += dot4(gi[c], vr[c]);
     }
-    const float D = half_sum<PAIR>(al * da);
+    const float ad = al * da;
+    const float D = PAIR ? h16_sum(ad) : warp_sum(ad);
     const float g = al * (da - D);
     if (live) dsig[beg + e] = g;
     const float gs = g * scale;
@@ -579,8 +580,8 @@ attn_bwd_src_tile_kernel(const float* __restrict__ dout, long long ldo, const fl
   const int R = (int)(r1 - r0), Rmax = WT + wlo + whi;
   float4* sq = attn_sm;
   float4* sd = sq + Rmax * nch;
-  stage_rows(sq, q, ld, r0, R, nch);
-  stage_rows(sd, dout, ldo, r0, R, nch);
+  blk_stage_rows<256>(sq, q, ld, r0, R, nch);
+  blk_stage_rows<256>(sd, dout, ldo, r0, R, nch);
   constexpr int NPW = WT / 8;
   int degs[NPW], rows[NPW];                    // per-edge metadata of this warp's nodes, requested before the wait
   float as_[NPW], gs_[NPW];
@@ -602,7 +603,7 @@ attn_bwd_src_tile_kernel(const float* __restrict__ dout, long long ldo, const fl
       gs_[p] = dsig[id] * scale;
     }
   }
-  stage_wait();
+  cp_wait_all();
 #pragma unroll
   for (int p = 0; p < NPW; ++p) {
     const int nl = warp * NPW + p;
@@ -631,17 +632,17 @@ attn_bwd_src_tile_kernel(const float* __restrict__ dout, long long ldo, const fl
 
 // ---------------------------------------------------------------------------------- K5 EdgeAtt
 // by-source softmax of <x_j, u_k> over k in out(j); result stored at the by-destination edge id.
-template <int NC>
-__global__ void __launch_bounds__(AW * 32)
+template <typename V, int NC>
+__global__ void __launch_bounds__(AW * 32, node_min_blocks<V, NC>)
 edgeatt_fwd_kernel(const float* __restrict__ x, long long ldx, const float* __restrict__ u, long long ldu,
                    const int* __restrict__ t_rowptr, const int* __restrict__ t_col, const int* __restrict__ t_eid,
                    float* __restrict__ nu, long long N, int H) {
   const int lane = threadIdx.x & 31;
   const long long node = (long long)blockIdx.x * AW + (threadIdx.x >> 5);
   if (node >= N) return;
-  const int nch = H >> 2;
-  float4 xj[NC];
-  load_row<NC>(x + node * ldx, nch, lane, xj);
+  const int nch = H >> Chunk<V>::SH;
+  V xj[NC];
+  load_row<V, NC>(x + node * ldx, nch, lane, xj);
   const int beg = t_rowptr[node], end = t_rowptr[node + 1];
   // pass 1: raw scores -> nu[t_eid], running max
   float mx = -INFINITY;
@@ -649,7 +650,7 @@ edgeatt_fwd_kernel(const float* __restrict__ x, long long ldx, const float* __re
     const int cn = min(32, end - cb);
     float my = -INFINITY;
     for (int uu = 0; uu < cn; ++uu) {
-      const float d = row_dot<NC>(xj, u + (long long)t_col[cb + uu] * ldu, nch, lane);
+      const float d = row_dot<V, NC>(xj, u + (long long)t_col[cb + uu] * ldu, nch, lane);
       if (lane == uu) my = d;
     }
     if (lane < cn) nu[t_eid[cb + lane]] = my;
@@ -669,16 +670,17 @@ edgeatt_fwd_kernel(const float* __restrict__ x, long long ldx, const float* __re
 }
 
 // by-source backward: dsig[e] = nu_e (dnu_e - sum nu dnu),  dx_j = sum_k dsig u_k   (dx is WRITTEN, not accumulated)
-template <int NC>
-__global__ void __launch_bounds__(AW * 32)
+template <typename V, int NC>
+__global__ void __launch_bounds__(AW * 32, node_min_blocks<V, NC>)
 edgeatt_bwd_src_kernel(const float* __restrict__ dnu, const float* __restrict__ nu, const float* __restrict__ u,
                        long long ldu, const int* __restrict__ t_rowptr, const int* __restrict__ t_col,
                        const int* __restrict__ t_eid, float* __restrict__ dsig, float* __restrict__ dx, long long lddx,
                        long long N, int H) {
+  constexpr int CW = 1 << Chunk<V>::SH;
   const int lane = threadIdx.x & 31;
   const long long node = (long long)blockIdx.x * AW + (threadIdx.x >> 5);
   if (node >= N) return;
-  const int nch = H >> 2;
+  const int nch = H >> Chunk<V>::SH;
   const int beg = t_rowptr[node], end = t_rowptr[node + 1];
   float D = 0.f;
   for (int e = beg + lane; e < end; e += 32) {
@@ -686,9 +688,9 @@ edgeatt_bwd_src_kernel(const float* __restrict__ dnu, const float* __restrict__ 
     D += nu[id] * dnu[id];
   }
   D = warp_sum(D);
-  float4 acc[NC];
+  V acc[NC];
 #pragma unroll
-  for (int c = 0; c < NC; ++c) acc[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int c = 0; c < NC; ++c) acc[c] = zerov<V>();
   for (int e = beg; e < end; ++e) {
     const int id = t_eid[e];
     const float g = nu[id] * (dnu[id] - D);
@@ -697,29 +699,30 @@ edgeatt_bwd_src_kernel(const float* __restrict__ dnu, const float* __restrict__ 
 #pragma unroll
     for (int c = 0; c < NC; ++c) {
       const int ch = lane + 32 * c;
-      if (ch < nch) fma4(acc[c], g, ld4(pu + 4 * ch));
+      if (ch < nch) fmav(acc[c], g, ldv<V>(pu + CW * ch));
     }
   }
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
     const int ch = lane + 32 * c;
-    if (ch < nch) st4(dx + node * lddx + 4 * ch, acc[c]);
+    if (ch < nch) stv(dx + node * lddx + CW * ch, acc[c]);
   }
 }
 
 // by-destination backward: du_k = sum_{j in in(k)} dsig[j->k] x_j
-template <int NC>
-__global__ void __launch_bounds__(AW * 32)
+template <typename V, int NC>
+__global__ void __launch_bounds__(AW * 32, node_min_blocks<V, NC>)
 edgeatt_bwd_dst_kernel(const float* __restrict__ dsig, const float* __restrict__ x, long long ldx,
                        const int* __restrict__ rowptr, const int* __restrict__ col, float* __restrict__ du,
                        long long lddu, long long N, int H) {
+  constexpr int CW = 1 << Chunk<V>::SH;
   const int lane = threadIdx.x & 31;
   const long long node = (long long)blockIdx.x * AW + (threadIdx.x >> 5);
   if (node >= N) return;
-  const int nch = H >> 2;
-  float4 acc[NC];
+  const int nch = H >> Chunk<V>::SH;
+  V acc[NC];
 #pragma unroll
-  for (int c = 0; c < NC; ++c) acc[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int c = 0; c < NC; ++c) acc[c] = zerov<V>();
   const int beg = rowptr[node], end = rowptr[node + 1];
   for (int e = beg; e < end; ++e) {
     const float g = dsig[e];
@@ -727,19 +730,17 @@ edgeatt_bwd_dst_kernel(const float* __restrict__ dsig, const float* __restrict__
 #pragma unroll
     for (int c = 0; c < NC; ++c) {
       const int ch = lane + 32 * c;
-      if (ch < nch) fma4(acc[c], g, ld4(px + 4 * ch));
+      if (ch < nch) fmav(acc[c], g, ldv<V>(px + CW * ch));
     }
   }
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
     const int ch = lane + 32 * c;
-    if (ch < nch) st4(du + node * lddu + 4 * ch, acc[c]);
+    if (ch < nch) stv(du + node * lddu + CW * ch, acc[c]);
   }
 }
 
-#include "attn_wide.cuh"
-
-// window (tile) kernels and the NC = 1..3 kernels above: 16-byte aligned rows, H % 4 == 0, H <= 384
+// window (tile) kernels: 16-byte aligned rows, H % 4 == 0, H <= 384
 static int chk(const void* p, long long ld, int H) {
   if ((H & 3) || H <= 0 || H > 384) return ERCG_EINVAL;
   if (!p) return ERCG_EINVAL;
@@ -763,22 +764,23 @@ using namespace ercg;
 
 #define ERCG_CHK(p, ld) do { int rc_ = chk(p, ld, H); if (rc_) return rc_; } while (0)
 #define ERCG_CHK_ROW(p, ld) do { int rc_ = chk_row(p, ld, H, &v4_); if (rc_) return rc_; } while (0)
-// float4 chunks NC = 1..3 where every row allows them and H <= 384 (the original kernels); float4 NC = 4..8 for wider
-// rows; float2 chunks when H % 4 == 2 or a row is only 8-byte aligned.  The choice depends on H and the operands only.
-#define ERCG_LAUNCH_NC(kernel, wide, ...)                                                               \
+// One warp per node, 8 per CTA.  Chunk type and count from H and the operands only: float4 chunks where every row allows
+// them (NC = 1, 2, 3, 4, 6, 8 up to H = 128, 256, 384, 512, 768, 1024), float2 chunks when H % 4 == 2 or a row is only
+// 8-byte aligned (NC = 4, 8, 12, 16 up to H = 256, 512, 768, 1024).
+#define ERCG_LAUNCH_NC(kernel, ...)                                                                     \
   do {                                                                                                  \
     const unsigned blocks_ = (unsigned)((N + AW - 1) / AW);                                             \
     cudaStream_t st_ = (cudaStream_t)stream;                                                            \
-    if (v4_ && H <= 128) kernel<1><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                          \
-    else if (v4_ && H <= 256) kernel<2><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                     \
-    else if (v4_ && H <= 384) kernel<3><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                     \
-    else if (v4_ && H <= 512) wide<float4, 4><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);               \
-    else if (v4_ && H <= 768) wide<float4, 6><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);               \
-    else if (v4_) wide<float4, 8><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                           \
-    else if (H <= 256) wide<float2, 4><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                      \
-    else if (H <= 512) wide<float2, 8><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                      \
-    else if (H <= 768) wide<float2, 12><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                     \
-    else wide<float2, 16><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                                   \
+    if (v4_ && H <= 128) kernel<float4, 1><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                  \
+    else if (v4_ && H <= 256) kernel<float4, 2><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);             \
+    else if (v4_ && H <= 384) kernel<float4, 3><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);             \
+    else if (v4_ && H <= 512) kernel<float4, 4><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);             \
+    else if (v4_ && H <= 768) kernel<float4, 6><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);             \
+    else if (v4_) kernel<float4, 8><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                         \
+    else if (H <= 256) kernel<float2, 4><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                    \
+    else if (H <= 512) kernel<float2, 8><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                    \
+    else if (H <= 768) kernel<float2, 12><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                   \
+    else kernel<float2, 16><<<blocks_, AW * 32, 0, st_>>>(__VA_ARGS__);                                 \
     return finish_launch();                                                                             \
   } while (0)
 
@@ -791,7 +793,7 @@ extern "C" int ercg_attn_fwd(const float* q, const float* k, const float* v, con
   bool v4_ = (H & 3) == 0;
   ERCG_CHK_ROW(q, ld); ERCG_CHK_ROW(k, ld); ERCG_CHK_ROW(v, ld); ERCG_CHK_ROW(out, ldo);
   if (s) ERCG_CHK_ROW(s, ld);
-  ERCG_LAUNCH_NC(attn_fwd_kernel, attn_fwd_wide_kernel, q, k, v, s, ld, rowptr, col, scale, out, ldo, alpha, dact, N, H);
+  ERCG_LAUNCH_NC(attn_fwd_kernel, q, k, v, s, ld, rowptr, col, scale, out, ldo, alpha, dact, N, H);
 }
 
 extern "C" int ercg_attn_bwd_dst(const float* dout, int64_t ldo, const float* k, const float* v, int64_t ld,
@@ -804,7 +806,7 @@ extern "C" int ercg_attn_bwd_dst(const float* dout, int64_t ldo, const float* k,
   bool v4_ = (H & 3) == 0;
   ERCG_CHK_ROW(dout, ldo); ERCG_CHK_ROW(k, ld); ERCG_CHK_ROW(v, ld); ERCG_CHK_ROW(dq, ldd);
   if (ds) ERCG_CHK_ROW(ds, ldd);
-  ERCG_LAUNCH_NC(attn_bwd_dst_kernel, attn_bwd_dst_wide_kernel, dout, ldo, k, v, ld, rowptr, col, alpha, scale, dq, ds, ldd, dsig, dact, N, H);
+  ERCG_LAUNCH_NC(attn_bwd_dst_kernel, dout, ldo, k, v, ld, rowptr, col, alpha, scale, dq, ds, ldd, dsig, dact, N, H);
 }
 
 extern "C" int ercg_attn_bwd_src(const float* dout, int64_t ldo, const float* q, int64_t ld,
@@ -816,7 +818,7 @@ extern "C" int ercg_attn_bwd_src(const float* dout, int64_t ldo, const float* q,
   if (!t_rowptr || !t_col || !t_eid || !alpha || !dsig) return ERCG_EINVAL;
   bool v4_ = (H & 3) == 0;
   ERCG_CHK_ROW(dout, ldo); ERCG_CHK_ROW(q, ld); ERCG_CHK_ROW(dk, ldd); ERCG_CHK_ROW(dv, ldd);
-  ERCG_LAUNCH_NC(attn_bwd_src_kernel, attn_bwd_src_wide_kernel, dout, ldo, q, ld, t_rowptr, t_col, t_eid, alpha, dsig, scale, dk, dv, ldd, N, H);
+  ERCG_LAUNCH_NC(attn_bwd_src_kernel, dout, ldo, q, ld, t_rowptr, t_col, t_eid, alpha, dsig, scale, dk, dv, ldd, N, H);
 }
 
 // ---- window-graph variants (contract: the in-neighbours of node i lie in [i - wlo, i + whi]; violated -> trap)
@@ -913,7 +915,7 @@ extern "C" int ercg_edgeatt_fwd(const float* x, int64_t ldx, const float* u, int
   if (!t_rowptr || !t_col || !t_eid || !nu) return ERCG_EINVAL;
   bool v4_ = (H & 3) == 0;
   ERCG_CHK_ROW(x, ldx); ERCG_CHK_ROW(u, ldu);
-  ERCG_LAUNCH_NC(edgeatt_fwd_kernel, edgeatt_fwd_wide_kernel, x, ldx, u, ldu, t_rowptr, t_col, t_eid, nu, N, H);
+  ERCG_LAUNCH_NC(edgeatt_fwd_kernel, x, ldx, u, ldu, t_rowptr, t_col, t_eid, nu, N, H);
 }
 
 extern "C" int ercg_edgeatt_bwd_src(const float* dnu, const float* nu, const float* u, int64_t ldu,
@@ -924,7 +926,7 @@ extern "C" int ercg_edgeatt_bwd_src(const float* dnu, const float* nu, const flo
   if (!dnu || !nu || !t_rowptr || !t_col || !t_eid || !dsig) return ERCG_EINVAL;
   bool v4_ = (H & 3) == 0;
   ERCG_CHK_ROW(u, ldu); ERCG_CHK_ROW(dx, lddx);
-  ERCG_LAUNCH_NC(edgeatt_bwd_src_kernel, edgeatt_bwd_src_wide_kernel, dnu, nu, u, ldu, t_rowptr, t_col, t_eid, dsig, dx, lddx, N, H);
+  ERCG_LAUNCH_NC(edgeatt_bwd_src_kernel, dnu, nu, u, ldu, t_rowptr, t_col, t_eid, dsig, dx, lddx, N, H);
 }
 
 extern "C" int ercg_edgeatt_bwd_dst(const float* dsig, const float* x, int64_t ldx,
@@ -935,5 +937,5 @@ extern "C" int ercg_edgeatt_bwd_dst(const float* dsig, const float* x, int64_t l
   if (!dsig || !rowptr || !col) return ERCG_EINVAL;
   bool v4_ = (H & 3) == 0;
   ERCG_CHK_ROW(x, ldx); ERCG_CHK_ROW(du, lddu);
-  ERCG_LAUNCH_NC(edgeatt_bwd_dst_kernel, edgeatt_bwd_dst_wide_kernel, dsig, x, ldx, rowptr, col, du, lddu, N, H);
+  ERCG_LAUNCH_NC(edgeatt_bwd_dst_kernel, dsig, x, ldx, rowptr, col, du, lddu, N, H);
 }

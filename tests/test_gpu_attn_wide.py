@@ -1,5 +1,5 @@
-"""K4 / K5 attention at the widths the float4 NC = 1..3 kernels do not take (csrc/attn_wide.cuh): any even H up to 1024 and
-rows that are only 8-byte aligned.  Op level against torch on the CPU in fp32 and fp64, the DialogueGCN and dgcnv2 modules at
+"""K4 / K5 warp-per-node attention (csrc/attn.cu) beyond float4 chunks with NC = 1..3: any even H up to 1024 and rows that
+are only 8-byte aligned.  Op level against torch on the CPU in fp32 and fp64, the DialogueGCN and dgcnv2 modules at
 those hidden sizes against the oracles, bit reproducibility and CUDA-graph capture, and the argument checks.
 
 Every tensor is measured against its own scale (parity_check with zero_floor_frac=1e-12)."""

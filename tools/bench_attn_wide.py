@@ -1,10 +1,10 @@
-"""Micro-benchmark of the K4 / K5 attention kernels at the widths csrc/attn_wide.cuh adds, forward + backward, against the
-reference's PyTorch formulation in eager mode on the same GPU.
+"""Micro-benchmark of the K4 / K5 warp-per-node attention kernels (csrc/attn.cu) at widths past H = 384 and at float2
+chunks, forward + backward, against the reference's PyTorch formulation in eager mode on the same GPU.
 
     python tools/bench_attn_wide.py [--rounds 11] [--out result.json]
 
 4096 IEMOCAP-shaped dialogues (synth.iemocap_lengths, seed 1; ~200 k utterances), fp32, TF32 off.
-  * K5 EdgeAtt (DialogueGCN), g in {300 (float4 NC = 3, the original kernels), 302 (float2), 512, 768}: ops.edge_att(x, u) on
+  * K5 EdgeAtt (DialogueGCN), g in {300 (float4 NC = 3), 302 (float2), 512, 768}: ops.edge_att(x, u) on
     the 10 / 10 window graph, gradients of x and u, against the oracle's formulation (oracle/modules.py EdgeAttOracle after
     its u = x W^T: gather both ends of every edge, per-source scatter softmax).
   * K4 nodal MatchingAttention 'general2' (dgcnv2), width in {356 (h = 128, float4 NC = 3), 358 (h = 129, float2), 868
