@@ -9,8 +9,15 @@ What is kept from the reference
     mean cross entropy (class-weighted for 6-way DialogueGCN, masked for DAG-ERC + clip_grad_norm_(5)), Adam / AdamW with the
     reference's learning rates, a test pass after every epoch (EvalCallback(test_per_epoch=1), mmbase.py:136) with accuracy,
     weighted / micro / macro F1, balanced accuracy and the confusion matrix (sklearn, mmbase.py:262-283), seed marking per
-    epoch, ``best_model.ckpt`` / ``last_model.ckpt`` as plain ``state_dict`` files (mmbase.py:325-333) whose keys are the
-    reference modules' keys.
+    epoch, ``best_model.ckpt`` / ``last_model.ckpt`` whose model keys are the reference modules' keys.
+Checkpoints
+  * ``--ckpt_layout=state_dict`` (default): each file is the model's plain ``state_dict``, written once per improvement /
+    after the last epoch.  The reference's files are NOT this: mmbase.py:325-333 saves lumo's ``Trainer.state_dict()``.
+  * ``--ckpt_layout=reference``: that layout (lumo/trainer/trainer.py:623-632), ``{'models': {'model': sd}, 'optims':
+    {'optim': <torch.optim Adam / AdamW state_dict>}, 'others': {'train_mm': {epoch, best, history, run parameters, every
+    rank's CPU generator state}}, 'thtensor': {}, 'nptensor': {}}``; ``last_model.ckpt`` is rewritten after every epoch.
+  * ``--resume=<ckpt>`` continues a run from such a file (refused when a run-defining parameter differs);
+    ``--load=<ckpt>`` starts from the weights alone, of either layout (a reference checkpoint included).
 What is different
   * the model runs in libercgraph kernels; the batch is collated onto the device in the packed layout (collate.DeviceCollate);
     the optimizer is the flat-buffer Adam kernel (optim.FlatAdam);
@@ -40,6 +47,9 @@ import numpy as np
 import torch
 
 MODULES = ("cogmen", "dgcn", "dgcnv2", "mmgcn", "dagerc")
+CKPT_LAYOUTS = ("state_dict", "reference")
+# the parameters a resumed run must share with the run that wrote the checkpoint (besides the number of processes)
+RUN_KEYS = ("module", "dataset", "modality", "seed", "batch_size", "n_classes", "n_speakers", "optim")
 
 
 # ------------------------------------------------------------------------------------------------ parameters
@@ -81,7 +91,8 @@ def resolve_params(args):
     if module not in MODULES:
         raise SystemExit("--module= one of %s" % (MODULES,))
     p = dict(seed=1, dataset="iemocap-cogmen-6", modality="atv", n_speakers=2, device=0, reimplement=False, data=None,
-             train_dialogues=120, test_dialogues=31, save_dir=None, log_every=0, max_len=None)
+             train_dialogues=120, test_dialogues=31, save_dir=None, log_every=0, max_len=None, ckpt_layout="state_dict",
+             resume=None, load=None)
     per_module = {
         "cogmen": dict(epoch=55, batch_size=32, optim="Adam", lr=1e-4, weight_decay=1e-8, num_heads=17),          # cogmen.py:36-52
         "dgcn": dict(epoch=55, batch_size=32, optim="Adam", lr=3e-4, weight_decay=0.0, loss_weights=True),        # dgcn.py:24-44
@@ -94,6 +105,10 @@ def resolve_params(args):
     for k, v in args.items():
         k = {"train.batch_size": "batch_size", "optim.lr": "lr", "optim.weight_decay": "weight_decay"}.get(k, k)
         p[k] = v
+    if p["ckpt_layout"] not in CKPT_LAYOUTS:
+        raise SystemExit("--ckpt_layout= one of %s" % (CKPT_LAYOUTS,))
+    if p["resume"] and p["load"]:
+        raise SystemExit("--resume and --load exclude each other (--resume also loads the weights)")
     ds = p["dataset"]
     if "n_classes" not in p:
         tail = ds.rsplit("-", 1)[-1]
@@ -227,6 +242,94 @@ def build_model(p, dev):
     return m.to(dev)
 
 
+# ------------------------------------------------------------------------------------------------ checkpoints
+def load_checkpoint(path):
+    return torch.load(path, map_location="cpu", weights_only=True)
+
+
+def is_reference_layout(ckpt):
+    """The reference trainer's Trainer.state_dict() layout (lumo/trainer/trainer.py:623-632): {'models': {'model': sd},
+    'optims': ..., 'others': ..., 'thtensor': ..., 'nptensor': ...}; anything else is a plain model state_dict."""
+    return isinstance(ckpt, dict) and isinstance(ckpt.get("models"), dict) and "model" in ckpt["models"]
+
+
+def load_model_weights(model, ckpt, log=print):
+    """Weights and buffers of a checkpoint of either layout into ``model``.  A leading ``module.`` (DDP, accelerate) is
+    stripped; every key of ``model`` must be present; keys ``model`` does not have (COGMEN's dead encoder in a build
+    without it) are ignored and logged.  Returns the ignored keys."""
+    sd = ckpt["models"]["model"] if is_reference_layout(ckpt) else ckpt
+    sd = {(k[len("module."):] if k.startswith("module.") else k): v for k, v in sd.items()}
+    own = model.state_dict()
+    missing = [k for k in own if k not in sd]
+    if missing:
+        raise SystemExit("train_mm: the checkpoint lacks %d of the module's keys: %s" % (len(missing), ", ".join(missing)))
+    ignored = [k for k in sd if k not in own]
+    if ignored:
+        log("train_mm: ignoring %d checkpoint keys this build does not have: %s" % (len(ignored), ", ".join(ignored)))
+    model.load_state_dict({k: sd[k] for k in own}, strict=True)
+    return ignored
+
+
+def reference_param_names(p):
+    """Names of the reference module's parameters() in order -- what the indices of its torch.optim state count.  For
+    COGMEN that list includes the dead TransformerEncoder, which this build leaves out unless --dead_encoder."""
+    with torch.device("meta"):
+        m = build_model(dict(p, dead_encoder=True), torch.device("meta"))
+    return [k for k, _ in m.named_parameters()]
+
+
+def load_reference_optim(optim, ckpt, p, names, log=print):
+    """The Adam state of a reference-layout checkpoint train_mm did not write into ``optim`` (FlatAdam; ``names``: its
+    parameters' names).  Without 'param_names' its indices are mapped to names through the reference module's parameter
+    list.  Returns False, after saying so in the log, when the state cannot be mapped (the weights alone are loaded)."""
+    optims = ckpt.get("optims") or {}
+    sd = optims.get("optim", next(iter(optims.values())) if len(optims) == 1 else None)
+    if not isinstance(sd, dict) or not sd.get("param_groups"):
+        log("train_mm: the checkpoint holds no optimizer state; loading the weights only")
+        return False
+    g = sd["param_groups"]
+    if len(g) == 1 and "param_names" not in g[0]:
+        ref = reference_param_names(p)
+        if len(g[0]["params"]) == len(ref):
+            sd = dict(sd, param_groups=[dict(g[0], param_names=ref)])
+    try:
+        optim.load_state_dict(sd, names)
+    except (ValueError, KeyError) as e:
+        log("train_mm: the checkpoint's optimizer state does not map onto this module's parameters (%s); loading the "
+            "weights only" % e)
+        return False
+    return True
+
+
+def run_params(p, world):
+    return dict({k: p[k] for k in RUN_KEYS}, world=world)
+
+
+def check_resumable(ckpt, p, world, path):
+    """SystemExit unless ``ckpt`` can continue this run: reference layout, and, when train_mm wrote it, the same
+    run-defining parameters (RUN_KEYS and the number of processes)."""
+    if not is_reference_layout(ckpt):
+        raise SystemExit("train_mm: --resume=%s is a plain state_dict; resuming needs a checkpoint written with "
+                         "--ckpt_layout=reference (--load reads the weights alone)" % path)
+    mine = (ckpt.get("others") or {}).get("train_mm")
+    if mine is None:
+        return
+    want = run_params(p, world)
+    diff = ["%s=%r (checkpoint: %r)" % (k, want[k], mine["params"].get(k)) for k in want if mine["params"].get(k) != want[k]]
+    if diff:
+        raise SystemExit("train_mm: --resume=%s comes from a different run; it cannot continue with %s"
+                         % (path, ", ".join(diff)))
+
+
+def _plain(x):
+    """numpy scalars (sklearn's metrics) -> Python numbers, so the checkpoint loads with torch.load(weights_only=True)."""
+    if isinstance(x, dict):
+        return {k: _plain(v) for k, v in x.items()}
+    if isinstance(x, (list, tuple)):
+        return [_plain(v) for v in x]
+    return x.item() if isinstance(x, np.generic) else x
+
+
 class Trainer:
     def __init__(self, p, rank=0, world=1, log=print):
         """rank / world from init_distributed; world > 1 needs the process group initialised."""
@@ -253,7 +356,24 @@ class Trainer:
         self.class_weight = None
         if p["module"] in ("dgcn", "dgcnv2") and p.get("loss_weights") and p["n_classes"] == 6:
             self.class_weight = torch.tensor(DGCN_LOSS_WEIGHTS, device=self.dev)
-        self.best = {}
+        self.param_names = [k for k, _ in self.model.named_parameters()]     # the order of model.parameters()
+        self.best, self.history, self.start_epoch = {}, [], 1
+
+    def resume(self, ckpt, path):
+        """--resume (after check_resumable): weights, buffers and Adam state; for a checkpoint train_mm wrote also the
+        best record, the history, this rank's CPU generator and the epoch counter."""
+        load_model_weights(self.model, ckpt, self.log)
+        mine = (ckpt.get("others") or {}).get("train_mm")
+        if mine is None:
+            self.log("train_mm: %s was not written by train_mm: its weights and optimizer state are loaded, training starts "
+                     "at epoch 1 and the run parameters cannot be checked" % path)
+            load_reference_optim(self.optim, ckpt, self.p, self.param_names, self.log)
+            return
+        self.optim.load_state_dict(ckpt["optims"]["optim"], self.param_names)     # applied when the optimizer attaches
+        self.best, self.history = mine["best"], list(mine["history"])
+        torch.set_rng_state(mine["rng"][self.rank])
+        self.start_epoch = int(mine["epoch"]) + 1
+        self.log("train_mm: resuming %s after epoch %d" % (path, mine["epoch"]))
 
     def _logits(self, batch):
         m = self.p["module"]
@@ -371,20 +491,46 @@ class Trainer:
                 "maf1": metrics.f1_score(true, pred, average="macro"),
                 "cm": metrics.confusion_matrix(true, pred, labels=range(self.p["n_classes"])).tolist(), "C": n}
 
-    def save(self, name):
+    def _rng_states(self):
+        """The CPU generator state of every rank (the dropout seeds are drawn from it, by MMGCN in the test pass too, and
+        the ranks evaluate unequal numbers of test batches), gathered on every rank."""
+        st = torch.get_rng_state()
+        if self.world == 1:
+            return [st]
+        import torch.distributed as dist
+        out = [None] * self.world
+        dist.all_gather_object(out, st)
+        return out
+
+    def save(self, name, epoch=None, rngs=None):
+        """``state_dict`` layout: the model's state_dict (mmbase.py:325-333).  ``reference`` layout (``rngs`` from
+        _rng_states): the reference trainer's Trainer.state_dict() with torch.optim's Adam state, plus what --resume
+        needs under others.train_mm.  Written to a temporary file and renamed, so a kill never leaves a truncated file."""
         d = self.p.get("save_dir")
         if not d or self.rank != 0:
             return None
         os.makedirs(d, exist_ok=True)
         path = os.path.join(d, name)
-        torch.save({k: v.detach().cpu().clone() for k, v in self.model.state_dict().items()}, path)   # mmbase.py:325-333
+        obj = {k: v.detach().cpu().clone() for k, v in self.model.state_dict().items()}
+        if self.p["ckpt_layout"] == "reference":
+            osd = self.optim.torch_state_dict(self.param_names)
+            osd["state"] = {i: {k: v.detach().cpu() for k, v in st.items()} for i, st in osd["state"].items()}
+            obj = {"models": {"model": obj}, "optims": {"optim": osd},
+                   "others": {"train_mm": {"epoch": epoch, "best": _plain(self.best), "history": _plain(self.history),
+                                           "params": run_params(self.p, self.world), "rng": rngs}},
+                   "thtensor": {}, "nptensor": {}}
+        tmp = path + ".tmp"
+        torch.save(obj, tmp)
+        os.replace(tmp, path)
         return path
 
     def train(self, train, test, log=print):
         p = self.p
+        ref = p["ckpt_layout"] == "reference"
         self.model.train()
-        history = []
-        for epoch in range(1, int(p["epoch"]) + 1):
+        history = self.history
+        epoch = self.start_epoch - 1
+        for epoch in range(self.start_epoch, int(p["epoch"]) + 1):
             rng = np.random.default_rng(p["seed"] * 100003 + epoch)                                  # rnd.mark(seed) per epoch, mmbase.py:207-208
             order = rng.permutation(len(train))
             t0 = time.perf_counter()
@@ -405,12 +551,16 @@ class Trainer:
             rec = {"epoch": epoch, "train_Lall": lsum / nb, "train_Acc": asum / nb, "utt_per_s": utts / dt,
                    **{"test_" + k: v for k, v in te.items() if k != "cm"}}
             history.append(rec)
+            rngs = self._rng_states() if ref else None                  # collective: before the rank-0-only writes
             if te["f1"] >= self.best.get("f1", -1.0):
                 self.best = {"f1": te["f1"], "acc": te["acc"], "epoch": epoch, "cm": te["cm"]}
-                self.save("best_model.ckpt")
+                self.save("best_model.ckpt", epoch, rngs)
+            if ref:
+                self.save("last_model.ckpt", epoch, rngs)              # every epoch: an interrupted run can be resumed
             log("epoch %3d  train Lall %.4f Acc %.3f  |  test Lall %.4f acc %.3f f1 %.3f  |  %.0f utt/s" % (
                 epoch, rec["train_Lall"], rec["train_Acc"], te["Lall"], te["acc"], te["f1"], rec["utt_per_s"]))
-        self.save("last_model.ckpt")
+        if not ref or self.start_epoch > int(p["epoch"]):
+            self.save("last_model.ckpt", epoch, self._rng_states() if ref else None)
         return history
 
 
@@ -424,7 +574,16 @@ def main(argv=None, log=print):
         train, test, what = load_data(p)
         log("train_mm: module=%s dataset=%s modality=%s hidden_all=%d n_classes=%d n_speakers=%d | %s: %d / %d dialogues" % (
             p["module"], p["dataset"], p["modality"], p["hidden_all"], p["n_classes"], p["n_speakers"], what, len(train), len(test)))
+        ckpt = None
+        if p["resume"]:
+            ckpt = load_checkpoint(p["resume"])                     # every rank reads it
+            check_resumable(ckpt, p, world, p["resume"])
         tr = Trainer(p, rank, world, log=log)
+        if ckpt is not None:
+            tr.resume(ckpt, p["resume"])
+        elif p["load"]:
+            load_model_weights(tr.model, load_checkpoint(p["load"]), log)
+            log("train_mm: weights loaded from %s" % p["load"])
         if p.get("eval_first"):
             log("eval_first:", {k: v for k, v in tr.test(test).items() if k != "cm"})
         hist = tr.train(train, test, log=log)
