@@ -145,6 +145,12 @@ SIGNATURES = {
     # K12 (DialogueRNN)
     "ercg_dialogue_rnn_fwd": (I, [POINTER(DialogueRnnArgs), P]),
     "ercg_dialogue_rnn_bwd": (I, [POINTER(DialogueRnnArgs), P]),
+    # K13 (dense masked MatchingAttention), the sequence reversal and log-softmax of the sequence classifiers
+    "ercg_match_att_fwd": (I, [P, L, I, I, I, I, P, L, P, I, P, L, P, P, P]),
+    "ercg_match_att_bwd": (I, [P, L, I, I, I, I, P, L, P, I, P, P, P, L, P, P, L, P, L, P]),
+    "ercg_reverse_seq": (I, [P, L, I, I, I, P, P, L, I, P]),
+    "ercg_log_softmax_fwd": (I, [P, L, P, L, L, I, P]),
+    "ercg_log_softmax_bwd": (I, [P, L, P, L, P, L, L, I, P]),
 }
 
 _lib = None

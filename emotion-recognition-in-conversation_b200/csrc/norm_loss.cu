@@ -542,6 +542,36 @@ cls_tail_final_kernel(const float* __restrict__ partial, int nb, int width, int 
   else db3[c - CK - K] = (float)s;
 }
 
+// ---------------------------------------------------------------------------------- log-softmax over the columns of a row
+// F.log_softmax(x, dim=-1) of the sequence classifiers' heads: y = x - max - log(sum exp(x - max)); backward
+// dx = dy - exp(y) * sum dy.  One warp per row, lanes over the columns (any C), fixed-order warp sums.
+__global__ void __launch_bounds__(256)
+log_softmax_fwd_kernel(const float* __restrict__ x, long long ldx, float* __restrict__ y, long long ldy, long long rows, int C) {
+  const long long r = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (r >= rows) return;
+  const int lane = threadIdx.x & 31;
+  const float* xr = x + r * ldx;
+  float m = -INFINITY;
+  for (int c = lane; c < C; c += 32) m = fmaxf(m, xr[c]);
+  m = warp_max(m);
+  float s = 0.f;
+  for (int c = lane; c < C; c += 32) s += expf(xr[c] - m);
+  const float ls = logf(warp_sum(s));
+  for (int c = lane; c < C; c += 32) y[r * ldy + c] = xr[c] - m - ls;
+}
+
+__global__ void __launch_bounds__(256)
+log_softmax_bwd_kernel(const float* __restrict__ y, long long ldy, const float* __restrict__ dy, long long lddy,
+                       float* __restrict__ dx, long long lddx, long long rows, int C) {
+  const long long r = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (r >= rows) return;
+  const int lane = threadIdx.x & 31;
+  float s = 0.f;
+  for (int c = lane; c < C; c += 32) s += dy[r * lddy + c];
+  s = warp_sum(s);
+  for (int c = lane; c < C; c += 32) dx[r * lddx + c] = dy[r * lddy + c] - expf(y[r * ldy + c]) * s;
+}
+
 }  // namespace ercg
 
 using namespace ercg;
@@ -787,5 +817,22 @@ extern "C" int ercg_cls_tail_bwd(const float* h, int64_t ldh, const float* dlogi
   int rc = finish_launch();
   if (rc) return rc;
   cls_tail_final_kernel<<<fin_blocks(width), 256, 0, st>>>(part, grid, width, C * K, K, C, dW3, db0, db3);
+  return finish_launch();
+}
+
+extern "C" int ercg_log_softmax_fwd(const float* x, int64_t ldx, float* y, int64_t ldy, int64_t rows, int C, void* stream) {
+  if (rows < 0 || C < 1 || ldx < C || ldy < C) return ERCG_EINVAL;
+  if (rows == 0) return ERCG_OK;
+  if (!x || !y) return ERCG_EINVAL;
+  log_softmax_fwd_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, (cudaStream_t)stream>>>(x, ldx, y, ldy, rows, C);
+  return finish_launch();
+}
+
+extern "C" int ercg_log_softmax_bwd(const float* y, int64_t ldy, const float* dy, int64_t lddy, float* dx, int64_t lddx,
+                                    int64_t rows, int C, void* stream) {
+  if (rows < 0 || C < 1 || ldy < C || lddy < C || lddx < C) return ERCG_EINVAL;
+  if (rows == 0) return ERCG_OK;
+  if (!y || !dy || !dx) return ERCG_EINVAL;
+  log_softmax_bwd_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, (cudaStream_t)stream>>>(y, ldy, dy, lddy, dx, lddx, rows, C);
   return finish_launch();
 }

@@ -1,5 +1,6 @@
-"""torch.autograd wrappers for K11 (MaskedEdgeAttention 'attn1' in closed form, csrc/dgcnv2.cu) and K12 (the DialogueRNN
-recurrence, csrc/dialogue_rnn.cu); include/ercgraph.h."""
+"""torch.autograd wrappers for K11 (MaskedEdgeAttention 'attn1' in closed form, csrc/dgcnv2.cu), K12 (the DialogueRNN
+recurrence, csrc/dialogue_rnn.cu), K13 (dense masked MatchingAttention) with the sequence reversal (csrc/seq_attn.cu), and the
+log-softmax of the sequence classifiers (csrc/norm_loss.cu); include/ercgraph.h."""
 import ctypes
 
 import torch
@@ -128,3 +129,106 @@ def dialogue_rnn(U, qmask, g_cell, p_cell, e_cell, att_weight, att_type, drop_p=
                                   e_cell.weight_hh, e_cell.bias_ih, e_cell.bias_hh, (L, B, Dg, Dp, De, P), float(drop_p),
                                   tuple(int(s) for s in seeds))
     return e.view(L, B, De), [alpha[B * t * (t - 1) // 2:B * t * (t + 1) // 2].view(B, t) for t in range(1, L)]
+
+
+# ------------------------------------------------------------------------------------------- K13 dense MatchingAttention
+MATCH_KINDS = {"general": 0, "general2": 1}
+
+
+class _MatchAtt(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, M, xq, mask, kind, L, B, Q):
+        M, ldm = _rows(M)
+        xq, ldq = _rows(xq)
+        D, dev = M.size(1), M.device
+        pool = torch.empty((Q * B, D), dtype=torch.float32, device=dev)
+        alpha = torch.empty((Q, B, L), dtype=torch.float32, device=dev)
+        score = torch.empty((Q, B, L), dtype=torch.float32, device=dev)
+        check(lib().ercg_match_att_fwd(_p(M), ldm, L, B, D, Q, _p(xq), ldq, _p(mask), kind, _p(pool), D, _p(alpha), _p(score),
+                                       _stream()), "ercg_match_att_fwd")
+        ctx.dims = (kind, L, B, Q, ldm, ldq)
+        ctx.save_for_backward(M, xq, mask, alpha, score)
+        ctx.mark_non_differentiable(alpha)
+        return pool, alpha
+
+    @staticmethod
+    def backward(ctx, dpool, _dalpha):
+        M, xq, mask, alpha, score = ctx.saved_tensors
+        kind, L, B, Q, ldm, ldq = ctx.dims
+        dpool, lddp = _rows(dpool)
+        D, dev = M.size(1), M.device
+        w = torch.empty((Q, B, L), dtype=torch.float32, device=dev)
+        dxq = torch.empty((Q * B, D), dtype=torch.float32, device=dev)
+        dM = torch.empty((L * B, D), dtype=torch.float32, device=dev)
+        check(lib().ercg_match_att_bwd(_p(M), ldm, L, B, D, Q, _p(xq), ldq, _p(mask), kind, _p(alpha), _p(score), _p(dpool),
+                                       lddp, _p(w), _p(dxq), D, _p(dM), D, _stream()), "ercg_match_att_bwd")
+        return dM, dxq, None, None, None, None, None
+
+
+def match_attention(M, xq, mask, att_type):
+    """MatchingAttention over B dialogues (K13): M [L, B, D] memory (seq-first), xq [Q, B, D] or [B, D] (Q = 1) transformed
+    queries, mask [B, L] float or None (ignored for 'general') -> (pool [Q, B, D] (or [B, D]), alpha [Q, B, L]); alpha is not
+    differentiable.  Q = L with xq = transform(M) is the att2 loop over every position."""
+    L, B, D = M.shape
+    squeeze = xq.dim() == 2
+    xq3 = xq.unsqueeze(0) if squeeze else xq
+    Q = xq3.size(0)
+    kind = MATCH_KINDS[att_type]
+    m = None
+    if kind == 1 and mask is not None:
+        m = mask.to(torch.float32).contiguous()
+    pool, alpha = _MatchAtt.apply(M.reshape(L * B, D), xq3.reshape(Q * B, D), m, kind, L, B, Q)
+    return (pool.view(B, D) if squeeze else pool.view(Q, B, D)), alpha
+
+
+# ------------------------------------------------------------------------------------------- sequence reversal, log-softmax
+class _ReverseSeq(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, counts, Lout):
+        Lin, B, D = x.shape
+        x2, ldx = _rows(x.reshape(Lin * B, D))
+        out = torch.empty((Lout, B, D), dtype=torch.float32, device=x.device)
+        check(lib().ercg_reverse_seq(_p(x2), ldx, Lin, B, D, _p(counts), _p(out), D, Lout, _stream()), "ercg_reverse_seq")
+        ctx.save_for_backward(counts)
+        ctx.Lin = Lin
+        return out
+
+    @staticmethod
+    def backward(ctx, dout):
+        (counts,) = ctx.saved_tensors
+        Lout, B, D = dout.shape
+        dout = dout.contiguous()
+        dx = torch.empty((ctx.Lin, B, D), dtype=torch.float32, device=dout.device)
+        check(lib().ercg_reverse_seq(_p(dout), D, Lout, B, D, _p(counts), _p(dx), D, ctx.Lin, _stream()), "ercg_reverse_seq")
+        return dx, None, None
+
+
+def reverse_seq(x, counts, Lout):
+    """x [L, B, D] -> [Lout, B, D]: the first counts[b] rows of dialogue b in reverse order, zero rows after them
+    (pad_sequence of flip(x[:c_b]) when Lout = max c_b).  counts: int32 CUDA tensor [B]."""
+    return _ReverseSeq.apply(x.to(torch.float32), counts, int(Lout))
+
+
+class _LogSoftmax(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x):
+        x, ldx = _rows(x)
+        R, C = x.shape
+        y = torch.empty((R, C), dtype=torch.float32, device=x.device)
+        check(lib().ercg_log_softmax_fwd(_p(x), ldx, _p(y), C, R, C, _stream()), "ercg_log_softmax_fwd")
+        ctx.save_for_backward(y)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        (y,) = ctx.saved_tensors
+        dy, lddy = _rows(dy)
+        R, C = y.shape
+        dx = torch.empty((R, C), dtype=torch.float32, device=y.device)
+        check(lib().ercg_log_softmax_bwd(_p(y), C, _p(dy), lddy, _p(dx), C, R, C, _stream()), "ercg_log_softmax_bwd")
+        return dx
+
+
+def log_softmax(x):
+    """F.log_softmax(x, dim=-1) for a 2-D fp32 CUDA tensor [rows, C]."""
+    return _LogSoftmax.apply(x)

@@ -1,7 +1,8 @@
 """Drop-in for track_mm/dgcnv2_models.py (SURVEY.md 8f-2): the DialogueGCN part (reference :517-773) -- ``MatchingAttention``
-('general2'), ``MaskedEdgeAttention`` ('attn1'), ``edge_perms``, ``batch_graphify`` and ``GraphNetwork`` -- and the DialogueRNN
-recurrence (:235-348) -- ``SimpleAttention``, ``DialogueRNNCell``, ``DialogueRNN`` -- with the reference's constructor
-arguments, signatures and state_dict keys.
+('general2'), ``MaskedEdgeAttention`` ('attn1'), ``edge_perms``, ``batch_graphify`` and ``GraphNetwork`` --, the DialogueRNN
+recurrence (:235-348) -- ``SimpleAttention``, ``DialogueRNNCell``, ``DialogueRNN`` -- and the declare-lab sequence classifiers
+``LSTMModel``, ``GRUModel`` and ``DialogRNNModel`` with ``MatchingAttention.forward(M, x, mask)``, with the reference's
+constructor arguments, signatures and state_dict keys.
 
 Kernel mapping
   MaskedEdgeAttention.scalar (Linear 2D -> 110)   K2 over the dialogue-major full-length rows
@@ -15,9 +16,17 @@ Kernel mapping
                                                   over all L*B rows; the three GRUCells, the attention over the global-state
                                                   history and the party-state update: K12 (csrc/dialogue_rnn.cu), one
                                                   persistent kernel forward and one backward
+  MatchingAttention.forward(M, x, mask)           transform = K2, then K13 (csrc/seq_attn.cu): 'general' / masked 'general2'
+                                                  attention of one query per dialogue, forward and backward
+  LSTMModel / GRUModel                            2-layer BiLSTM / BiGRU over the unpacked batch (birnn_forward: K2 + K6 / K6b)
+  DialogRNNModel                                  DialogueRNN (K12) forward and over the reversed dialogues (_reverse_seq:
+                                                  ercg_reverse_seq, its backward the same permutation); dropout_rec =
+                                                  ops.dropout
+  att2 head of the three (the per-position loop)  K13 with Q = L: all positions of all dialogues in one launch
+  linear -> ReLU -> dropout -> smax_fc            ops.mlp_head, then ercg_log_softmax_fwd / bwd
 The unused attention variants of the file (Attention 'mlp', MatchingAttention 'dot' / 'concat') are parameter holders or
-NotImplementedError: DGCNModule with 'attn1' and nodal 'general2' never executes them.  DialogueRNN runs stand-alone;
-DGCNModule("DialogRNN") still raises NotImplementedError.
+NotImplementedError: DGCNModule with 'attn1' and nodal 'general2' never executes them.  DialogueRNN runs stand-alone and
+inside DialogRNNModel; DGCNModule("DialogRNN") still raises NotImplementedError.
 """
 import torch
 from torch import nn
@@ -27,7 +36,8 @@ from ..graph import build_graph, speakers_from_edge_dict
 from ..models.rgcn import RGCNConv
 from ..pyg_nn import GraphConv
 from .cogmen_utils import edge_perms  # noqa: F401  (same function in the reference, dgcnv2_models.py:612-635)
-from .dgcn_models import _fresh_seed
+from .dgcn_models import _fresh_seed, birnn_forward
+from .mmgcn_utils import lengths_graph
 
 
 class MatchingAttention(nn.Module):
@@ -45,11 +55,25 @@ class MatchingAttention(nn.Module):
         return ops.matching_attention(xt, emotions, graph_full)
 
     def forward(self, M, x, mask=None):
-        """Reference signature (M [L,B,D], x [B,D], mask [B,L]) -> one query per dialogue.  Only the unused LSTMModel /
-        DialogRNNModel classes and the per-position loop of attentive_node_features (:709-712) call it that way; the product
-        path evaluates all positions of all dialogues at once (``pooled``)."""
-        raise NotImplementedError("MatchingAttention.forward(M, x, mask): use pooled(emotions, graph_full) -- every node of "
-                                  "every dialogue in one launch (same arithmetic as the reference's loop over positions)")
+        """Reference signature: M [L,B,mem_dim] (seq-first), x [B,cand_dim], mask [B,L] float or None -> (pool [B,mem_dim],
+        alpha [B,1,L]); one query per dialogue on K13.  'general' ignores the mask; 'general2' with mask None uses all ones,
+        and a dialogue whose mask is all zero gets NaN, as in the reference."""
+        dev = self.transform.weight.device
+        if M.dim() != 3 or x.dim() != 2 or M.size(2) != self.mem_dim or x.size(1) != self.cand_dim or x.size(0) != M.size(1):
+            raise ValueError("M [L, B, %d] and x [B, %d] expected, got %s and %s" % (self.mem_dim, self.cand_dim, tuple(M.shape),
+                                                                                 tuple(x.shape)))
+        _check_mask(mask, M.size(1), M.size(0), dev)
+        _check_cuda_f32(dev, M=M, x=x)
+        L, B, _ = M.shape
+        pool, alpha = ops_dgcnv2.match_attention(M, ops.linear(x, self.transform.weight, self.transform.bias), mask, self.att_type)
+        return pool, alpha.view(B, 1, L)
+
+    def all_positions(self, M, mask=None):
+        """The att2 loop of the sequence classifiers in one K13 launch: query t of dialogue b is transform(M[t, b]) against all
+        of M[:, b] -> (pool [L,B,mem_dim] = the stacked forward(M, M[t], mask)[0], alpha [L,B,L]: alpha[t] = forward(...)[1][:, 0])."""
+        L, B, D = M.shape
+        xq = ops.linear(M.reshape(L * B, D), self.transform.weight, self.transform.bias).view(L, B, D)
+        return ops_dgcnv2.match_attention(M, xq, mask, self.att_type)
 
 
 class SimpleAttention(nn.Module):
@@ -207,3 +231,142 @@ class GraphNetwork(nn.Module):
                             reference_layout=False, mean_weight=False)
         logits = self.packed_logits(x, edge_index, edge_norm, edge_type, gfull, nodal_attn)
         return ops.unpack_rows(logits, gfull, int(lens.max()), seq_first=True)
+
+
+# ------------------------------------------------------------------------------------------- sequence classifiers
+def _check_cuda_f32(dev, **tensors):
+    for name, t in tensors.items():
+        if t.device != dev or dev.type != "cuda":
+            raise ValueError("%s (%s) and the parameters (%s) must be on the same CUDA device" % (name, t.device, dev))
+        if t.dtype != torch.float32:
+            raise ValueError("%s must be float32, got %s" % (name, t.dtype))
+
+
+def _check_mask(mask, B, L, dev):
+    if mask is None:
+        return
+    if mask.dim() != 2 or tuple(mask.shape) != (B, L):
+        raise ValueError("mask must be [B, L] = [%d, %d], got %s" % (B, L, tuple(mask.shape)))
+    if mask.device != dev:
+        raise ValueError("mask (%s) and the parameters (%s) must be on the same CUDA device" % (mask.device, dev))
+
+
+def _check_seq_inputs(m, U, qmask, umask, D_m):
+    """U [L,B,D_m] float32, qmask [L,B,P], umask [B,L] on the parameters' CUDA device."""
+    dev = m.linear.weight.device
+    if U.dim() != 3 or U.size(2) != D_m:
+        raise ValueError("U must be [L, B, %d], got %s" % (D_m, tuple(U.shape)))
+    if qmask.dim() != 3 or qmask.shape[:2] != U.shape[:2]:
+        raise ValueError("qmask must be [L, B, P] with U's L, B = %s, got %s" % (tuple(U.shape[:2]), tuple(qmask.shape)))
+    if umask is None:
+        raise ValueError("umask [B, L] is required")
+    _check_mask(umask, U.size(1), U.size(0), dev)
+    _check_cuda_f32(dev, U=U)
+    if qmask.device != dev:
+        raise ValueError("qmask (%s) and the parameters (%s) must be on the same CUDA device" % (qmask.device, dev))
+
+
+def _classify(m, emotions, umask, att2):
+    """The shared head of LSTMModel / GRUModel / DialogRNNModel: att2 = masked 'general2' MatchingAttention of every
+    position over its dialogue (K13), then relu(linear) -> dropout -> smax_fc (ops.mlp_head) -> log_softmax over the classes.
+    -> (log_prob [L,B,C], alpha: L tensors [B,L] with att2, else [])."""
+    L, B, D = emotions.shape
+    alpha = []
+    if att2:
+        emotions, a = m.matchatt.all_positions(emotions, umask)
+        alpha = list(a.unbind(0))
+    p = m.dropout.p if m.training else 0.0
+    logits = ops.mlp_head(emotions.reshape(L * B, D), m.linear.weight, m.linear.bias, m.smax_fc.weight, m.smax_fc.bias, p,
+                          _fresh_seed() if p > 0 else 0)
+    return ops_dgcnv2.log_softmax(logits).view(L, B, -1), alpha
+
+
+class LSTMModel(nn.Module):
+    """declare-lab LSTMModel: a 2-layer bidirectional nn.LSTM over the unpacked batch (every dialogue runs all L steps;
+    hoisted input GEMM + K6 through birnn_forward), then the head of ``_classify``.  forward(U [L,B,D_m], qmask [L,B,P],
+    umask [B,L], att2=True) -> (log_prob [L,B,n_classes], alpha, [], []); padded positions get outputs too."""
+    rnn_type = nn.LSTM
+
+    def __init__(self, D_m, D_e, D_h, n_classes=7, dropout=0.5):
+        super().__init__()
+        self.n_classes = n_classes
+        self.dropout = nn.Dropout(dropout)
+        setattr(self, self._rnn_name(), self.rnn_type(input_size=D_m, hidden_size=D_e, num_layers=2, bidirectional=True,
+                                                      dropout=dropout))
+        self.matchatt = MatchingAttention(2 * D_e, 2 * D_e, att_type="general2")
+        self.linear = nn.Linear(2 * D_e, D_h)
+        self.smax_fc = nn.Linear(D_h, n_classes)
+
+    @classmethod
+    def _rnn_name(cls):
+        return "lstm" if cls.rnn_type is nn.LSTM else "gru"
+
+    def forward(self, U, qmask, umask, att2=True):
+        rnn = getattr(self, self._rnn_name())
+        _check_seq_inputs(self, U, qmask, umask, rnn.input_size)
+        L, B, D_m = U.shape
+        dev = U.device
+        gf = lengths_graph(torch.full((B,), L, dtype=torch.int64), dev)
+        h = birnn_forward(rnn, ops.pack_rows(U, gf, seq_first=True), gf, None, self.training)     # dialogue-major rows
+        emotions = ops.unpack_rows(h, gf, L, seq_first=True)
+        log_prob, alpha = _classify(self, emotions, umask, att2)
+        return log_prob, alpha, [], []
+
+
+class GRUModel(LSTMModel):
+    """declare-lab GRUModel: LSTMModel with ``gru = nn.GRU(...)`` (K6b)."""
+    rnn_type = nn.GRU
+
+
+class DialogRNNModel(nn.Module):
+    """declare-lab DialogRNNModel: a forward and a reversed DialogueRNN (K12 each), ``dropout_rec`` (p = dropout + 0.15, the
+    declare-lab value) on both, their concatenation, then the head of ``_classify``.  forward(U [L,B,D_m], qmask [L,B,P],
+    umask [B,L], att2=True) -> (log_prob [L,B,n_classes], alpha or [], alpha_f, alpha_b).  The reversed direction reads each
+    dialogue's first int(sum(umask[b])) rows in reverse order (``_reverse_seq``); the longest such count must equal L (the
+    reference's concatenation fails otherwise: ValueError here).
+    K12's limits hold: D_g, D_p, D_e <= 256, P <= 16, at most one non-zero entry per qmask row, listener_state=False,
+    context_attention 'simple' or 'general'."""
+
+    def __init__(self, D_m, D_g, D_p, D_e, D_h, D_a=100, n_classes=7, listener_state=False, context_attention="simple",
+                 dropout_rec=0.5, dropout=0.5):
+        super().__init__()
+        self.D_m, self.D_g, self.D_p, self.D_e, self.D_h, self.n_classes = D_m, D_g, D_p, D_e, D_h, n_classes
+        self.dropout = nn.Dropout(dropout)
+        self.dropout_rec = nn.Dropout(dropout + 0.15)
+        self.dialog_rnn_f = DialogueRNN(D_m, D_g, D_p, D_e, listener_state, context_attention, D_a, dropout_rec)
+        self.dialog_rnn_r = DialogueRNN(D_m, D_g, D_p, D_e, listener_state, context_attention, D_a, dropout_rec)
+        self.linear = nn.Linear(2 * D_e, 2 * D_h)
+        self.smax_fc = nn.Linear(2 * D_h, n_classes)
+        self.matchatt = MatchingAttention(2 * D_e, 2 * D_e, att_type="general2")
+
+    @staticmethod
+    def _counts(mask):
+        return mask.sum(1).int()                      # the reference's torch.sum(mask, 1).int()
+
+    def _reverse_seq(self, X, mask, counts=None):
+        """pad_sequence([flip(X[:c_b, b]) for each b]), c_b = int(sum(mask[b])): [max c_b, B, D]."""
+        counts = self._counts(mask) if counts is None else counts
+        Lout = int(counts.max()) if counts.numel() else 0
+        return ops_dgcnv2.reverse_seq(X, counts, max(Lout, 0))
+
+    def _drop_rec(self, x):
+        p = self.dropout_rec.p if self.training else 0.0
+        return ops.dropout(x, p, _fresh_seed()) if p > 0 else x
+
+    def forward(self, U, qmask, umask, att2=True):
+        _check_seq_inputs(self, U, qmask, umask, self.D_m)
+        L, B, _ = U.shape
+        counts = self._counts(umask)
+        maxc = int(counts.max()) if B else L
+        if maxc != L:
+            raise ValueError("the longest dialogue in umask has %d positions, U has L = %d: the forward and reversed "
+                             "directions cannot be concatenated" % (maxc, L))
+        emotions_f, alpha_f = self.dialog_rnn_f(U, qmask)
+        emotions_f = self._drop_rec(emotions_f)
+        rev_U = self._reverse_seq(U, umask, counts)
+        rev_qmask = self._reverse_seq(qmask, umask, counts)
+        emotions_b, alpha_b = self.dialog_rnn_r(rev_U, rev_qmask)
+        emotions_b = self._drop_rec(self._reverse_seq(emotions_b, umask, counts))
+        emotions = torch.cat([emotions_f, emotions_b], dim=-1)
+        log_prob, alpha = _classify(self, emotions, umask, att2)
+        return log_prob, alpha, alpha_f, alpha_b

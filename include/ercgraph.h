@@ -659,6 +659,37 @@ typedef struct ercg_dialogue_rnn {
 int ercg_dialogue_rnn_fwd(const ercg_dialogue_rnn* args, void* stream);
 int ercg_dialogue_rnn_bwd(const ercg_dialogue_rnn* args, void* stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * K13  dense masked MatchingAttention of the declare-lab sequence classifiers (MatchingAttention.forward(M, x, mask) and the
+ * att2 loop of LSTMModel / GRUModel / DialogRNNModel, track_mm/dgcnv2_models.py).  B dialogues of L memory rows M (seq-first:
+ * row j*B + b, row stride ldm); Q queries per dialogue, query q of dialogue b = row r = q*B + b of xq (= transform(x), ldq).
+ *   kind ERCG_MATCH_GENERAL : alpha_j = softmax_j <xq_r, M_j>   (mask ignored)
+ *   kind ERCG_MATCH_GENERAL2: s_j = m_j <xq_r, m_j M_j>, p = softmax_j tanh(s_j) over all L, alpha_j = p_j m_j / sum_k p_k m_k
+ *        (m = mask[b*L + j], [B, L] contiguous; NULL = all ones; a row whose mask is all zero gives NaN, as the reference)
+ *   pool_r = sum_j alpha_j M_j
+ * fwd writes pool [Q*B, D] (row stride ldp), alpha [Q, B, L] and score [Q, B, L] (s_j, kept for the backward).
+ * bwd reads dpool (row stride lddp) and writes dxq [Q*B, D] and dM [L*B, D] (both overwritten); w [Q, B, L] is workspace.
+ * D in 1..1024 (any row alignment), L and Q in 1..4096, ld* >= D, B >= 0; other sizes or kinds: ERCG_EINVAL before any
+ * launch; B*Q or B*L above 2^31 - 1: ERCG_ERANGE.  B == 0: no-op.  Fixed-order fp32, no atomics: bit-reproducible.
+ * ------------------------------------------------------------------------------------------- */
+#define ERCG_MATCH_GENERAL 0
+#define ERCG_MATCH_GENERAL2 1
+int ercg_match_att_fwd(const float* M, int64_t ldm, int L, int B, int D, int Q, const float* xq, int64_t ldq,
+                       const float* mask, int kind, float* pool, int64_t ldp, float* alpha, float* score, void* stream);
+int ercg_match_att_bwd(const float* M, int64_t ldm, int L, int B, int D, int Q, const float* xq, int64_t ldq,
+                       const float* mask, int kind, const float* alpha, const float* score, const float* dpool,
+                       int64_t lddp, float* w, float* dxq, int64_t lddxq, float* dM, int64_t lddm, void* stream);
+/* DialogRNNModel._reverse_seq (pad_sequence of flip(x[:c_b]) per dialogue): x [Lin*B, D] seq-first (row stride ldx) ->
+ * out [Lout*B, D] (row stride ldo), out[t*B + b] = x[(c_b - 1 - t)*B + b] for t < c_b and 0 for c_b <= t < Lout, with
+ * c_b = counts[b] (device int32) clamped to [0, Lin].  Its backward is the same call with Lin and Lout swapped. */
+int ercg_reverse_seq(const float* x, int64_t ldx, int Lin, int B, int D, const int32_t* counts, float* out, int64_t ldo,
+                     int Lout, void* stream);
+/* y = log_softmax(x) over the C columns of each row (F.log_softmax(., 2) of the classifiers' heads); bwd: dx = dy - exp(y) *
+ * sum_c dy.  Any C >= 1; rows == 0: no-op. */
+int ercg_log_softmax_fwd(const float* x, int64_t ldx, float* y, int64_t ldy, int64_t rows, int C, void* stream);
+int ercg_log_softmax_bwd(const float* y, int64_t ldy, const float* dy, int64_t lddy, float* dx, int64_t lddx, int64_t rows,
+                         int C, void* stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
