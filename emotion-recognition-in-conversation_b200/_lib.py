@@ -93,6 +93,7 @@ SIGNATURES = {
     "ercg_lstm_fwd": (I, [P, L, P, P, I, I, P, L, P, P, P, P]),
     "ercg_lstm_bwd": (I, [P, L, P, P, P, P, I, I, P, L, P]),
     "ercg_dropout": (I, [P, P, L, F, U64, P]),
+    "ercg_dropout_dev": (I, [P, P, L, F, U64, P, P]),
     "ercg_gru_fwd": (I, [P, L, P, P, P, I, I, P, L, P, P, P]),
     "ercg_gru_bwd": (I, [P, L, P, P, P, P, I, I, P, L, P, L, P]),
     "ercg_bn_workspace_bytes": (SZ, [L, I]),

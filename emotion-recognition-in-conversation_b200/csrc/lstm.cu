@@ -129,6 +129,13 @@ __global__ void dropout_kernel(const float* __restrict__ x, float* __restrict__ 
   if (i < n) out[i] = hash_uniform(seed, (unsigned long long)i) < p ? 0.f : x[i] * scale;
 }
 
+// dropout_kernel with the seed offset read from device memory (a step counter that a captured graph advances)
+__global__ void dropout_dev_kernel(const float* __restrict__ x, float* __restrict__ out, long long n, float p, float scale,
+                                   unsigned long long seed, const unsigned long long* __restrict__ seed_dev) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = hash_uniform(seed + __ldg(seed_dev), (unsigned long long)i) < p ? 0.f : x[i] * scale;
+}
+
 }  // namespace ercg
 
 using namespace ercg;
@@ -182,5 +189,15 @@ extern "C" int ercg_dropout(const float* x, float* out, int64_t n, float p, uint
   if (n == 0) return ERCG_OK;
   if (!x || !out) return ERCG_EINVAL;
   dropout_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, out, n, p, 1.f / (1.f - p), seed);
+  return finish_launch();
+}
+
+extern "C" int ercg_dropout_dev(const float* x, float* out, int64_t n, float p, uint64_t seed, const uint64_t* seed_dev,
+                                void* stream) {
+  if (!seed_dev || n < 0 || !(p >= 0.f && p < 1.f)) return ERCG_EINVAL;
+  if (n == 0) return ERCG_OK;
+  if (!x || !out) return ERCG_EINVAL;
+  dropout_dev_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      x, out, n, p, 1.f / (1.f - p), seed, reinterpret_cast<const unsigned long long*>(seed_dev));
   return finish_launch();
 }

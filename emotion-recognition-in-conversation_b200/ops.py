@@ -713,20 +713,28 @@ def gru_layer(gx, whh, bhh, graph):
     return _GruLayer.apply(gx, whh, bhh, graph)
 
 
+def _dropout_call(x, out, p, seed, seed_dev):
+    if seed_dev is None:
+        check(lib().ercg_dropout(_p(x), _p(out), x.numel(), p, seed & (2 ** 64 - 1), _stream()), "ercg_dropout")
+    else:
+        check(lib().ercg_dropout_dev(_p(x), _p(out), x.numel(), p, seed & (2 ** 64 - 1), _p(seed_dev), _stream()),
+              "ercg_dropout_dev")
+
+
 class _Dropout(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, p, seed):
         x = x.contiguous()
         out = torch.empty_like(x)
-        check(lib().ercg_dropout(_p(x), _p(out), x.numel(), p, seed & (2 ** 64 - 1), _stream()), "ercg_dropout")
-        ctx.p, ctx.seed = p, seed
+        ctx.p, ctx.seed, ctx.seed_dev = p, seed, SEED_DEV       # the backward reads the same device word
+        _dropout_call(x, out, p, seed, ctx.seed_dev)
         return out
 
     @staticmethod
     def backward(ctx, dout):
         dout = dout.contiguous()
         dx = torch.empty_like(dout)
-        check(lib().ercg_dropout(_p(dout), _p(dx), dout.numel(), ctx.p, ctx.seed & (2 ** 64 - 1), _stream()), "ercg_dropout")
+        _dropout_call(dout, dx, ctx.p, ctx.seed, ctx.seed_dev)
         return dx, None, None
 
 

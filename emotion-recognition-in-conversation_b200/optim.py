@@ -20,6 +20,14 @@ from ._lib import lib, check
 from .ops import _p, _stream, _ws
 
 
+ALIGN = 64      # every parameter starts on a 256-byte boundary of the flat buffers: the kernels read weights / biases as
+                # float4 and through TMA
+
+
+def _slot(numel):
+    return (numel + ALIGN - 1) // ALIGN * ALIGN
+
+
 def _step_tensor(step):
     """torch.optim's Adam 'step': a CPU scalar of the default float type (float64 only when that is the default)."""
     return torch.tensor(float(step), dtype=torch.float64 if torch.get_default_dtype() == torch.float64 else torch.float32)
@@ -53,8 +61,7 @@ class FlatAdam:
         if order is not None:
             live = sorted(live, key=order)            # stable: lets a caller put early-available gradients first
         dev = live[0].device
-        ALIGN = 64                                     # every parameter starts on a 256-byte boundary of the flat buffers: the
-        n = sum((p.numel() + ALIGN - 1) // ALIGN * ALIGN for p in live)    # kernels read weights / biases as float4 and through TMA
+        n = sum(_slot(p.numel()) for p in live)
         self.n = n
         self.flat_p = torch.zeros(n, dtype=torch.float32, device=dev)     # padding stays 0 under Adam (g = 0, p = 0)
         self.flat_g = torch.zeros(n + self.extra_slots, dtype=torch.float32, device=dev)
@@ -73,13 +80,18 @@ class FlatAdam:
                 p.data = view                          # the parameter now LIVES in the flat buffer (same Parameter object)
                 self.g_views.append(self.flat_g[off:off + k].view_as(p))
                 self.offsets.append(off)
-                off += (k + ALIGN - 1) // ALIGN * ALIGN
+                off += _slot(k)
         self.live = live
         self._live_ids = {id(p) for p in live}
         if self._pending is not None:                  # state loaded before the live set was known
             pending, self._pending = self._pending, None
             self._apply(*pending)
         return self
+
+    def flat_bytes(self):
+        """Bytes of the flat gradient buffer if every parameter were live: an upper bound known before the first backward
+        (what a communicator that all-reduces that buffer has to hold)."""
+        return 4 * (sum(_slot(p.numel()) for p in self.params) + self.extra_slots)
 
     @property
     def extra(self):

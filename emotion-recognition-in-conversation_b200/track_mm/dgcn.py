@@ -35,3 +35,18 @@ class DGCNModule(nn.Module):
         logits = self.clf(torch.cat([features, graph_out], dim=-1), text_length)
         g.check_inputs()          # K1's input-error flags (length > padded width, speaker id out of range) -> ValueError
         return logits, graph_out
+
+    def forward_packed(self, x_packed, speaker_packed, text_length, graph=None):
+        """Resident-data entry point: utterance rows already packed [N, hidden_all] (16-byte aligned rows, as
+        collate.DeviceCollate / synth.packed_batch lay them out), packed speakers [N].  Same values as ``forward``.
+        The BiLSTM's layer-0 input transform is a plain product on the packed rows (no row gather), so it runs on the
+        tensor-core kernels; the rows get no gradient.  K1's input flags are NOT read here (that would wait for the
+        host): call ``graph.check_inputs()`` after the step, as the train step's ``check()`` does."""
+        g = graph if graph is not None else build_graph(text_length, speaker_packed, self.wp, self.wf, self.n_speakers,
+                                                        device=x_packed.device, mean_weight=False)
+        features = self.rnn.packed_forward(x_packed, g)
+        edge_norm = self.edge_att.edge_weights(features, g)
+        g.attach()
+        graph_out = self.gcn(features, g.edge_index, edge_norm, g.edge_type)
+        logits = self.clf(torch.cat([features, graph_out], dim=-1), text_length)
+        return logits, graph_out

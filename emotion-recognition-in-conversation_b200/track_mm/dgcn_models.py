@@ -31,15 +31,19 @@ def birnn_forward(rnn, x2d, graph, a_rows, training):
     for layer in range(rnn.num_layers):
         sfx = "_l%d" % layer
         w_ih = torch.cat([getattr(rnn, "weight_ih" + sfx), getattr(rnn, "weight_ih" + sfx + "_reverse")], 0)
-        w_hh = torch.stack([getattr(rnn, "weight_hh" + sfx), getattr(rnn, "weight_hh" + sfx + "_reverse")], 0)
         b_ih = (getattr(rnn, "bias_ih" + sfx), getattr(rnn, "bias_ih" + sfx + "_reverse"))
         b_hh = (getattr(rnn, "bias_hh" + sfx), getattr(rnn, "bias_hh" + sfx + "_reverse"))
         rows = a_rows if layer == 0 else None
         if gru:           # b_hn is scaled by the reset gate, so b_hh stays out of the hoisted GEMM
             gx = ops.linear(h, w_ih, torch.cat(b_ih, 0), a_rows=rows)
-            h = ops.gru_layer(gx, w_hh, torch.stack(b_hh, 0), graph)
         else:
             gx = ops.linear(h, w_ih, torch.cat([b_ih[0] + b_hh[0], b_ih[1] + b_hh[1]], 0), a_rows=rows)
+        # W_hh is stacked after the input transform: autograd runs the later node first, so W_hh's gradient is complete
+        # before the input transform's weight-gradient GEMM (what the train step's early gradient bucket waits for)
+        w_hh = torch.stack([getattr(rnn, "weight_hh" + sfx), getattr(rnn, "weight_hh" + sfx + "_reverse")], 0)
+        if gru:
+            h = ops.gru_layer(gx, w_hh, torch.stack(b_hh, 0), graph)
+        else:
             h = ops.lstm_layer(gx, w_hh, graph)
         if training and rnn.dropout > 0 and layer + 1 < rnn.num_layers:
             h = ops.dropout(h, rnn.dropout, _fresh_seed())

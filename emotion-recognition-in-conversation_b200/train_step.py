@@ -1,90 +1,85 @@
-"""The COGMEN train step as ONE replayable unit (SURVEY.md 8e / 8f-3; reference: CogmenTrainer.train_step,
-track_mm/cogmen.py:179-195, under accelerate/DDP, lumo/trainer/trainer.py:62-64,315-327).
+"""The COGMEN and DialogueGCN train steps as ONE replayable unit each (SURVEY.md 8e / 8f-3; reference:
+CogmenTrainer.train_step, track_mm/cogmen.py:179-195, and the DialogueGCN step, dgcn.py:117-134, under accelerate/DDP,
+lumo/trainer/trainer.py:62-64,315-327).
 
     graph build (K1) -> forward_packed -> cross entropy -> backward -> gradient all-reduce -> Adam
 
 * Nothing in the step touches the host: sizes and the possible relation ids come from the host-side batch description,
-  the loss normaliser is the host-known global utterance count, the optimizer's step counter and the dropout seed live on
-  the device.  ``capture()`` records the step once into a CUDA graph (collectives included) and ``replay()`` relaunches
-  it: ~50 kernel launches + autograd bookkeeping per step become one graph launch -- what makes 2^20 utterances split over
-  8 GPUs (1.7 ms of kernels per rank) scale.
-* Collectives per step with world > 1: BatchNorm statistics (2H+1 doubles, forward), their backward sums (2H floats) --
-  both only in ``bn_sync="global"`` mode; ``"local"`` is the reference's DDP behaviour (per-rank statistics) -- and the flat
-  gradient buffer.  The loss numerator rides in the tail of the gradient buffer; there is no separate loss collective.
+  the loss normaliser is host-known (COGMEN: the global utterance count) or reduced on the device (DialogueGCN's weighted
+  mean), the optimizer's step counter and the dropout seed live on the device.  ``capture()`` records the step once into a
+  CUDA graph (collectives included) and ``replay()`` relaunches it: ~50 kernel launches + autograd bookkeeping per step
+  become one graph launch -- what makes 2^20 utterances split over 8 GPUs (1.7 ms of kernels per rank) scale.
+* Collectives per step with world > 1: COGMEN's BatchNorm statistics (2H+1 doubles, forward), their backward sums (2H
+  floats) -- both only in ``bn_sync="global"`` mode; ``"local"`` is the reference's DDP behaviour (per-rank statistics) --,
+  DialogueGCN's loss (numerator, denominator: 2 floats, forward), and the flat gradient buffer.  COGMEN's loss numerator
+  rides in the tail of the gradient buffer; there is no separate loss collective.
 * Transport: libercgraph's peer-memory kernels over NVLink (p2p.PeerComm: ercg_p2p_allreduce for the gradient buckets,
   ercg_p2p_bn_stats / ercg_p2p_bn_act_bwd_reduce = the BatchNorm reductions fused with their exchange) when every rank can set
   them up, else torch.distributed on ``group`` -- the results are the same to the last bit (rank-ordered sums).
-* The gradient all-reduce is bucketed in two: everything except the input projection is reduced on a side stream as soon as
-  those gradients exist, under the projection's weight-gradient GEMM (the longest kernel of the step); the projection's own
-  gradient follows on the main stream.
+* The gradient all-reduce is bucketed in two: everything except the parameters of the input transform is reduced on a side
+  stream as soon as those gradients exist, under the input transform's weight-gradient GEMM (the longest kernel of the
+  step); the input transform's own gradients follow on the main stream.
 """
-import os
-
 import torch
-import torch.distributed as dist
 
 from . import ops
 from .graph import build_graph, graph_sizes, relation_ids_for_speakers
 from .optim import FlatAdam
 
 
-class CogmenTrainStep:
-    def __init__(self, model, lengths, speakers_present=(0,), lr=1e-4, weight_decay=1e-8, world=1, global_utterances=None,
-                 bn_sync="global", overlap=True, group=None, transport="auto"):
+class _FlatTrainStep:
+    """What the train steps share: communicators, the flat optimizer layout with the two gradient buckets, the bucketed
+    all-reduce + Adam tail, capture / replay and the deferred input check.  A subclass passes its FlatAdam and provides
+    ``_forward_backward(x, spk, labels)`` (which ends in ``self._backward(loss)``), ``_late_params()`` (the parameters
+    whose gradients come last: the input transform's) and ``global_loss()``."""
+
+    def __init__(self, model, lengths, speakers_present, opt, comm_bytes, world, group, transport, overlap):
         """lengths: CPU int64 [B] dialogue lengths of THIS rank's batch (a step re-run on new data of the same lengths reuses
         the capture; new lengths need a new capture).  speakers_present: the speaker ids the data set uses.
         transport: "p2p" = peer-memory all-reduce kernels (ercg_p2p_allreduce, one NVSwitch node), "nccl" = torch.distributed
-        on ``group``, "auto" = p2p when every rank can set it up, else torch.distributed."""
-        from .dist import StatSync
+        on ``group``, "auto" = p2p when every rank can set it up, else torch.distributed.  opt: the step's FlatAdam.
+        comm_bytes: payload size of the peer-memory communicators; the first step, and every step without overlap,
+        all-reduces the whole flat gradient buffer in one call, so it must hold that buffer."""
         from .p2p import PeerComm, Reducer
         self.model, self.world, self.group = model, world, group
         self.dev = next(model.parameters()).device
         comms = None
         if world > 1 and transport in ("auto", "p2p") and self.dev.type == "cuda":
             # two communicators: the early gradient bucket runs on a side stream next to the main stream's collectives
-            comms = PeerComm.create(group, self.dev, max_bytes=8 << 20, n=2)
+            comms = PeerComm.create(group, self.dev, max_bytes=comm_bytes, n=2)
             if comms is None and transport == "p2p":
-                raise RuntimeError("CogmenTrainStep: transport='p2p' but the peer-memory communicator could not be set up")
-        self.comms = comms
+                raise RuntimeError("%s: transport='p2p' but the peer-memory communicator could not be set up" % type(self).__name__)
+        self.comms, self.comm_bytes = comms, comm_bytes
         self.reduce_main = Reducer(group, comms[0] if comms else None)
         self.reduce_side = Reducer(group, comms[1] if comms else None)
         self.lengths = lengths.to(torch.int64).cpu().contiguous()
         self.sizes = graph_sizes(self.lengths, model.wp, model.wf)
         self.lengths_dev = self.lengths.to(self.dev)
         self.rel_ids = relation_ids_for_speakers(speakers_present, model.n_speakers)
-        self.global_utts = int(global_utterances if global_utterances is not None else self.sizes[0])
-        self.opt = FlatAdam(model.parameters(), lr=lr, weight_decay=weight_decay, extra_slots=1)
+        self.opt = opt
         self.overlap = bool(overlap) and world > 1
         self.side = torch.cuda.Stream(device=self.dev) if self.overlap else None
-        if world > 1 and bn_sync == "global":
-            model.gcn.stat_sync = StatSync(group=group, global_count=self.global_utts, reduce=self.reduce_main)
         self._graph = None
         self._static = None
+        self._graph_loss = None      # the captured step's loss (rewritten by every replay)
+        self._last_loss = None       # the loss of the last step run, eager or replayed
         self._pending = 0
         self._n_early = None
         self._hooks = []
-        self.loss_share = None
+        self._late_ids = None
 
     # ------------------------------------------------------------------------------------------ one step, eager
-    def _forward_backward(self, x, spk, labels):
-        m = self.model
-        g = build_graph(self.lengths_dev, spk, m.wp, m.wf, m.n_speakers, device=self.dev, sizes=self.sizes,
-                        relation_ids=self.rel_ids)
-        logits, _ = m.forward_packed(x, spk, self.lengths_dev, graph=g)
-        num_out = self.opt.extra if self.opt.live is not None else None
-        loss = ops.cross_entropy(logits, labels, denom=self.global_utts if self.world > 1 else None, num_out=num_out)
+    def _backward(self, loss):
         self.opt.zero_grad()
         self._pending = self._n_early if self._n_early is not None else -1
         loss.backward()
-        self._last_graph = g
-        return loss
 
     def _late_first(self, p):
-        # flat layout: gradients that exist EARLY in the backward first, the input projection (computed last) at the end
-        proj = self.model.rnn[1]
-        return 1 if (p is proj.weight or p is proj.bias) else 0
+        # flat layout: gradients that exist EARLY in the backward first, the input transform's (computed last) at the end
+        return 1 if id(p) in self._late_ids else 0
 
     def _attach(self):
+        self._late_ids = {id(p) for p in self._late_params()}
         self.opt.attach(order=self._late_first)
         live = self.opt.live
         self._n_early = sum(1 for p in live if self._late_first(p) == 0)
@@ -93,8 +88,8 @@ class CogmenTrainStep:
                 self._hooks.append(p.register_post_accumulate_grad_hook(self._on_grad))
 
     def _on_grad(self, _p):
-        """post-accumulate hook of every non-projection parameter: when the last one has its gradient, reduce that bucket on
-        the side stream while the main stream goes on to the projection's weight gradient."""
+        """post-accumulate hook of every early parameter: when the last one has its gradient, reduce that bucket on the side
+        stream while the main stream goes on to the input transform's weight gradient."""
         self._pending -= 1
         if self._pending != 0:
             return
@@ -106,23 +101,27 @@ class CogmenTrainStep:
         with torch.cuda.stream(self.side):
             self.reduce_side(opt.span(0, self._n_early))
 
+    def _first_step(self, loss):
+        """Called once, right after the flat layout exists (before the first un-bucketed all-reduce)."""
+
     def step(self, x, spk, labels):
-        """One eager step.  Returns this rank's share of the global mean loss (device scalar)."""
+        """One eager step.  Returns the loss (device scalar): COGMEN, this rank's share of the global mean; DialogueGCN,
+        the global weighted mean."""
         loss = self._forward_backward(x, spk, labels)
         if self.opt.live is None:
             self._attach()                                   # first step: decide the flat layout, then finish it un-bucketed
-            if self.world > 1:
-                self.opt.extra.copy_(loss.detach().reshape(1) * float(self.global_utts))
+            self._first_step(loss)
             self.opt.gather()
             if self.world > 1:
                 self.reduce_main(self.opt.flat_g)
             self.opt.update()
-            return loss.detach()
+            self._last_loss = loss.detach()
+            return self._last_loss
         opt = self.opt
         if self.world > 1:
             if self.overlap:
                 opt.gather(self._n_early, None)
-                self.reduce_main(opt.flat_g[opt.offsets[self._n_early]:])                    # projection bucket + loss slot
+                self.reduce_main(opt.flat_g[opt.offsets[self._n_early]:])                    # late bucket + loss slots
                 torch.cuda.current_stream(self.dev).wait_stream(self.side)
             else:
                 opt.gather()
@@ -130,11 +129,8 @@ class CogmenTrainStep:
         else:
             opt.gather()
         opt.update()
-        return loss.detach()
-
-    def global_loss(self):
-        """Global mean loss of the last step (valid after the gradient all-reduce; world == 1: the local loss)."""
-        return self.opt.extra[0] / float(self.global_utts)
+        self._last_loss = loss.detach()
+        return self._last_loss
 
     # ------------------------------------------------------------------------------------------ capture / replay
     def capture(self, x, spk, labels, warmup=3):
@@ -150,13 +146,14 @@ class CogmenTrainStep:
         ops.SEED_DEV = self.opt.step_dev                     # dropout seed = host seed + device step counter: fresh mask per replay
         self._graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self._graph):
-            self._loss = self.step(x, spk, labels)
+            self._graph_loss = self.step(x, spk, labels)
         ops.SEED_DEV = None
         return self
 
     def replay(self):
         self._graph.replay()
-        return self._loss
+        self._last_loss = self._graph_loss
+        return self._graph_loss
 
     def check(self):
         """Raise if K1 flagged the batch of the last step (bad lengths / speaker ids / relation id outside the hint), or if
@@ -168,3 +165,77 @@ class CogmenTrainStep:
     @property
     def transport(self):
         return self.reduce_main.transport
+
+
+class CogmenTrainStep(_FlatTrainStep):
+    def __init__(self, model, lengths, speakers_present=(0,), lr=1e-4, weight_decay=1e-8, world=1, global_utterances=None,
+                 bn_sync="global", overlap=True, group=None, transport="auto"):
+        """See _FlatTrainStep.  global_utterances: the utterance count of the GLOBAL batch (the loss normaliser; default
+        this rank's).  bn_sync: "global" = BatchNorm statistics over all ranks, "local" = per rank (the reference's DDP)."""
+        from .dist import StatSync
+        opt = FlatAdam(model.parameters(), lr=lr, weight_decay=weight_decay, extra_slots=1)
+        # 8 MB holds the live gradient (1.1 MB at width 1443); the dead encoder's parameters never get one
+        super().__init__(model, lengths, speakers_present, opt, 8 << 20, world, group, transport, overlap)
+        self.global_utts = int(global_utterances if global_utterances is not None else self.sizes[0])
+        if world > 1 and bn_sync == "global":
+            model.gcn.stat_sync = StatSync(group=group, global_count=self.global_utts, reduce=self.reduce_main)
+        self.loss_share = None
+
+    def _forward_backward(self, x, spk, labels):
+        m = self.model
+        g = build_graph(self.lengths_dev, spk, m.wp, m.wf, m.n_speakers, device=self.dev, sizes=self.sizes,
+                        relation_ids=self.rel_ids)
+        logits, _ = m.forward_packed(x, spk, self.lengths_dev, graph=g)
+        num_out = self.opt.extra if self.opt.live is not None else None
+        loss = ops.cross_entropy(logits, labels, denom=self.global_utts if self.world > 1 else None, num_out=num_out)
+        self._backward(loss)
+        self._last_graph = g
+        return loss
+
+    def _late_params(self):
+        proj = self.model.rnn[1]
+        return proj.weight, proj.bias
+
+    def _first_step(self, loss):
+        if self.world > 1:                                   # the loss slot was not attached during the first forward
+            self.opt.extra.copy_(loss.detach().reshape(1) * float(self.global_utts))
+
+    def global_loss(self):
+        """Global mean loss of the last step (valid after the gradient all-reduce; world == 1: the local loss)."""
+        return self.opt.extra[0] / float(self.global_utts)
+
+
+class DgcnTrainStep(_FlatTrainStep):
+    def __init__(self, model, lengths, speakers_present=None, lr=3e-4, weight_decay=0.0, class_weight=None, world=1,
+                 group=None, transport="auto", overlap=True):
+        """DialogueGCN (track_mm.dgcn.DGCNModule) step.  See _FlatTrainStep.  speakers_present: default every speaker id of
+        the model.  lr / weight_decay: dgcn.py's Adam defaults.  class_weight: the cross entropy's class weights
+        (track_mm.dgcn.LOSS_WEIGHTS for the 6-way IEMOCAP setting, dgcn.py:109-110) or None.  The loss is the weighted mean
+        over the GLOBAL batch: with world > 1 its (numerator, denominator) is all-reduced in the forward, so a batch sharded
+        by dialogue takes the same step as one GPU on the whole batch."""
+        if speakers_present is None:
+            speakers_present = range(model.n_speakers)
+        opt = FlatAdam(model.parameters(), lr=lr, weight_decay=weight_decay)
+        # every parameter but the classifier's unused emotion_att gets a gradient: 8.6 MB at width 1380
+        super().__init__(model, lengths, speakers_present, opt, max(8 << 20, opt.flat_bytes()), world, group, transport, overlap)
+        self.class_weight = None
+        if class_weight is not None:
+            self.class_weight = torch.as_tensor(class_weight, dtype=torch.float32).to(self.dev).contiguous()
+
+    def _forward_backward(self, x, spk, labels):
+        m = self.model
+        g = build_graph(self.lengths_dev, spk, m.wp, m.wf, m.n_speakers, device=self.dev, mean_weight=False, sizes=self.sizes,
+                        relation_ids=self.rel_ids)
+        logits, _ = m.forward_packed(x, spk, self.lengths_dev, graph=g)
+        loss = ops.cross_entropy(logits, labels, self.class_weight, reduce_sync=self.reduce_main if self.world > 1 else None)
+        self._backward(loss)
+        self._last_graph = g
+        return loss
+
+    def _late_params(self):
+        rnn = self.model.rnn.rnn
+        return tuple(getattr(rnn, n + "_l0" + d) for n in ("weight_ih", "bias_ih", "bias_hh") for d in ("", "_reverse"))
+
+    def global_loss(self):
+        """Global weighted mean loss of the last step (eager or replayed)."""
+        return self._last_loss

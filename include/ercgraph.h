@@ -316,6 +316,12 @@ int ercg_lstm_bwd(const float* dout, int64_t ldo, const float* gates, const floa
 /* inverted dropout with a counter-hash mask (same (seed, index) -> same mask, so the backward re-applies it):
  * out[i] = hash(seed, i) < p ? 0 : x[i] / (1 - p).  nn.LSTM(dropout=.4) between layers, dgcn_models.py:17. */
 int ercg_dropout(const float* x, float* out, int64_t n, float p, uint64_t seed, void* stream);
+/* ercg_dropout with the mask drawn from seed + *seed_dev (seed_dev: device uint64, as ercg_gemm_nn's): the inter-layer
+ * dropout of nn.LSTM (dgcn_models.py:17) inside a train step captured in a CUDA graph, which points seed_dev at its
+ * device step counter so that every replay draws a fresh mask.  *seed_dev == 0 gives ercg_dropout(seed) bit for bit;
+ * the backward calls it again with the same seed and word.  seed_dev NULL, n < 0 or p outside [0, 1): ERCG_EINVAL
+ * before any launch. */
+int ercg_dropout_dev(const float* x, float* out, int64_t n, float p, uint64_t seed, const uint64_t* seed_dev, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * K6b packed bidirectional GRU recurrence, one layer: the nn.GRU context encoders of DGCNModule("GRU")
