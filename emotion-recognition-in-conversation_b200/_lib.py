@@ -129,10 +129,12 @@ SIGNATURES = {
     "ercg_mmgcn_spmm": (I, [P, I, P, L, P, L, P, P, P, L, L, I, I, P, L, P, L, P]),
     "ercg_mmgcn_sddmm": (I, [P, L, P, L, P, P, P, L, L, I, I, P, I, P]),
     "ercg_gcnii_layer_fwd": (I, [P, L, P, L, P, L, P, L, L, I, F, F, I, F, U64, P]),
+    "ercg_gcnii_layer_fwd_dev": (I, [P, L, P, L, P, L, P, L, L, I, F, F, I, F, U64, P, P]),
     "ercg_gcnii_layer_bwd_input": (I, [P, L, P, L, P, L, L, I, F, F, P]),
     "ercg_node_rows": (I, [P, P, L, I, I, I, P, P]),
     "ercg_speaker_embed_add": (I, [P, L, P, I, P, P, L, P, L, P, P, L, I, P]),
     "ercg_relu_dropout": (I, [P, P, L, F, U64, P]),
+    "ercg_relu_dropout_dev": (I, [P, P, L, F, U64, P, P]),
     "ercg_masked_edge_att_fwd": (I, [P, L, P, P, P, P, L, I, I, P, P, L, P]),
     "ercg_masked_edge_att_bwd": (I, [P, L, P, P, P, P, L, I, I, P, P, P, P, L, L, P]),
     # K9 / K10 (DAG-ERC)

@@ -77,116 +77,14 @@ __device__ __forceinline__ void load_b_nn(const float* __restrict__ B, long long
   }
 }
 
-template <bool VEC_A, bool VEC_B>
-__global__ void __launch_bounds__(GT, 2)
-gemm_nn_kernel(const float* __restrict__ A, long long lda, const int* __restrict__ a_rows,
-               const float* __restrict__ B, long long ldb, float* __restrict__ C, long long ldc,
-               long long M, int N, int K, Epilogue ep,
-               const float* __restrict__ A2 = nullptr, long long lda2 = 0, int ksplit = 0x7fffffff) {
-  __shared__ __align__(16) float As[2][BK][BM + 4];
-  __shared__ __align__(16) float Bs[2][BK][BN + 4];
-  const int t = threadIdx.x, tx = t & 15, ty = t >> 4;
-  const long long m0 = (long long)blockIdx.x * BM;
-  const int n0 = blockIdx.y * BN;
+#define ERCG_NN_KERNEL gemm_nn_kernel
+#define ERCG_NN_GCNII_SEED ep.seed
+#include "gemm_nn_kernel.cuh"
 
-  const int arow_l = t & 127, ak = (t >> 7) * 8;
-  const long long am = m0 + arow_l;
-  const bool a_ok = am < M;
-  const float* arow = A;
-  if (a_ok) arow = A + (a_rows ? (long long)a_rows[am] : am) * lda;
-  // optional second source for the columns k >= ksplit of the A operand ([A | A2] without materialising the concat;
-  // ksplit % 8 == 0 so every 8-wide thread chunk lies on one side)
-  const float* arow2 = a_ok && A2 ? A2 + am * lda2 - ksplit : arow;
-  const int bk = t >> 5, bn = (t & 31) * 4;
-
-  float acc[8][8];
-#pragma unroll
-  for (int i = 0; i < 8; ++i)
-#pragma unroll
-    for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-
-  float ra[8], rb0[4], rb1[4];
-  load_a_nn<VEC_A>(ak >= ksplit ? arow2 : arow, a_ok, ak, K, ra);
-  load_b_nn<VEC_B>(B, ldb, bk, K, n0 + bn, N, rb0);
-  load_b_nn<VEC_B>(B, ldb, bk + 8, K, n0 + bn, N, rb1);
-  const int nslab = (K + BK - 1) / BK;
-  int buf = 0;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) As[0][ak + i][arow_l] = ra[i];
-  *reinterpret_cast<float4*>(&Bs[0][bk][bn]) = make_float4(rb0[0], rb0[1], rb0[2], rb0[3]);
-  *reinterpret_cast<float4*>(&Bs[0][bk + 8][bn]) = make_float4(rb1[0], rb1[1], rb1[2], rb1[3]);
-  __syncthreads();
-  for (int s = 0; s < nslab; ++s) {
-    const int kn = (s + 1) * BK;
-    if (s + 1 < nslab) {
-      load_a_nn<VEC_A>(kn + ak >= ksplit ? arow2 : arow, a_ok, kn + ak, K, ra);
-      load_b_nn<VEC_B>(B, ldb, kn + bk, K, n0 + bn, N, rb0);
-      load_b_nn<VEC_B>(B, ldb, kn + bk + 8, K, n0 + bn, N, rb1);
-    }
-    mma_slab(As[buf], Bs[buf], acc, ty, tx);
-    if (s + 1 < nslab) {
-      const int nb = buf ^ 1;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) As[nb][ak + i][arow_l] = ra[i];
-      *reinterpret_cast<float4*>(&Bs[nb][bk][bn]) = make_float4(rb0[0], rb0[1], rb0[2], rb0[3]);
-      *reinterpret_cast<float4*>(&Bs[nb][bk + 8][bn]) = make_float4(rb1[0], rb1[1], rb1[2], rb1[3]);
-      __syncthreads();
-      buf = nb;
-    }
-  }
-
-  // epilogue
-  const bool vec_c = ((ldc & 3) == 0) && aligned16(C);
-#pragma unroll
-  for (int ih = 0; ih < 2; ++ih)
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const long long m = m0 + ih * 64 + ty * 4 + i;
-      if (m >= M) continue;
-#pragma unroll
-      for (int jh = 0; jh < 2; ++jh) {
-        const int n = n0 + jh * 64 + tx * 4;
-        if (n >= N) continue;
-        float v[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          float x = acc[ih * 4 + i][jh * 4 + j];
-          const int nn = n + j;
-          if (nn < N) {
-            if (ep.bias) x += __ldg(ep.bias + nn);
-            if (ep.act == ERCG_ACT_RELU) {
-              x = fmaxf(x, 0.f);
-            } else if (ep.act == ERCG_ACT_RELU_DROPOUT) {
-              x = fmaxf(x, 0.f);
-              const bool drop = dropout_drop(dropout_group_hash(ep.seed + (ep.seed_dev ? __ldg(ep.seed_dev) : 0ull), m, nn, N), nn & 3, dropout_thr16(ep.drop_p));
-              x = drop ? 0.f : x * (1.0f / (1.0f - ep.drop_p));
-            } else if (ep.act == ERCG_ACT_MASK_POS) {
-              x = __ldg(ep.aux + m * ep.ldaux + nn) > 0.f ? x * ep.aux_scale : 0.f;
-            } else if (ep.act == ACT_GCNII_FWD) {
-              x = ep.c_acc * x + (ep.c1 * __ldg(ep.aux + m * ep.ldaux + nn) + ep.c2 * __ldg(ep.aux2 + m * ep.ldaux2 + nn));
-              if (ep.half) x = fmaxf(x, 0.f);
-              if (ep.drop_p > 0.f) {
-                const float u = hash_uniform(ep.seed, (unsigned long long)m * (unsigned long long)N + nn);
-                x = u < ep.drop_p ? 0.f : x * (1.0f / (1.0f - ep.drop_p));
-              }
-            } else if (ep.act == ACT_GCNII_BWD) {
-              x = ep.c_acc * x + (nn < ep.half ? ep.c1 * __ldg(ep.aux + m * ep.ldaux + nn)
-                                               : ep.c2 * __ldg(ep.aux + m * ep.ldaux + nn - ep.half));
-            }
-          }
-          v[j] = x;
-        }
-        float* cp = C + m * ldc + n;
-        if (vec_c && n + 4 <= N) {
-          st4(cp, make_float4(v[0], v[1], v[2], v[3]));
-        } else {
-#pragma unroll
-          for (int j = 0; j < 4; ++j)
-            if (n + j < N) cp[j] = v[j];
-        }
-      }
-    }
-}
+// ercg_gcnii_layer_fwd_dev: the GCNII layer with its dropout seed offset read from device memory
+#define ERCG_NN_KERNEL gcnii_fwd_dev_kernel
+#define ERCG_NN_GCNII_SEED (ep.seed + __ldg(ep.seed_dev))
+#include "gemm_nn_kernel.cuh"
 
 // ------------------------------------------------------------------------------------------ TN
 // C[K1,N1] (+)= sum over rows m in this CTA's slab of A[m,k1] * B[m,n1]
@@ -586,21 +484,47 @@ extern "C" int ercg_colsum(const float* A, int64_t lda, int64_t M, int N, float*
 // [hi | h0] is never materialised: the A operand is read from two sources split at k = H.
 // The ReLU and the NEXT layer's input dropout (GCNII_lyc.forward :388-392) are the epilogue.
 // ---------------------------------------------------------------------------------------------
-extern "C" int ercg_gcnii_layer_fwd(const float* hi, int64_t ldhi, const float* h0, int64_t ldh0, const float* W,
-                                    int64_t ldw, float* out, int64_t ldo, int64_t M, int H, float theta, float alpha,
-                                    int relu, float drop_p, uint64_t seed, void* stream) {
+// argument checks of both GCNII forward entries; ERCG_OK with grid set = launch, ERCG_OK with grid.x == 0 = nothing to do
+static int gcnii_fwd_check(const float* hi, int64_t ldhi, const float* h0, int64_t ldh0, const float* W, int64_t ldw,
+                           const float* out, int64_t ldo, int64_t M, int H, float drop_p, dim3& grid) {
+  grid = dim3(0, 0, 0);
   if (M < 0 || H <= 0 || (H & 7)) return ERCG_EINVAL;
   if (M == 0) return ERCG_OK;
   if (!hi || !h0 || !W || !out || ldhi < H || ldh0 < H || ldw < H || ldo < H) return ERCG_EINVAL;
   if (!(drop_p >= 0.f && drop_p < 1.f)) return ERCG_EINVAL;
   if (!aligned16(hi) || !aligned16(h0) || !aligned16(W) || (ldhi & 3) || (ldh0 & 3) || (ldw & 3)) return ERCG_EALIGN;
-  Epilogue ep{nullptr, ACT_GCNII_FWD, hi, (long long)ldhi, 1.f, drop_p, (unsigned long long)seed,
-              h0, (long long)ldh0, theta, (1.f - theta) * (1.f - alpha), (1.f - theta) * alpha, relu ? 1 : 0};
   long long gm = (M + BM - 1) / BM;
   if (gm > 2147483647LL) return ERCG_ERANGE;
-  dim3 grid((unsigned)gm, (unsigned)((H + BN - 1) / BN));
+  grid = dim3((unsigned)gm, (unsigned)((H + BN - 1) / BN));
+  return ERCG_OK;
+}
+
+extern "C" int ercg_gcnii_layer_fwd(const float* hi, int64_t ldhi, const float* h0, int64_t ldh0, const float* W,
+                                    int64_t ldw, float* out, int64_t ldo, int64_t M, int H, float theta, float alpha,
+                                    int relu, float drop_p, uint64_t seed, void* stream) {
+  dim3 grid;
+  const int rc = gcnii_fwd_check(hi, ldhi, h0, ldh0, W, ldw, out, ldo, M, H, drop_p, grid);
+  if (rc != ERCG_OK || grid.x == 0) return rc;
+  Epilogue ep{nullptr, ACT_GCNII_FWD, hi, (long long)ldhi, 1.f, drop_p, (unsigned long long)seed,
+              h0, (long long)ldh0, theta, (1.f - theta) * (1.f - alpha), (1.f - theta) * alpha, relu ? 1 : 0};
   gemm_nn_kernel<true, true><<<grid, GT, 0, (cudaStream_t)stream>>>(hi, ldhi, nullptr, W, ldw, out, ldo, M, H, 2 * H, ep,
                                                                    h0, ldh0, H);
+  return finish_launch();
+}
+
+// ercg_gcnii_layer_fwd with the dropout mask drawn from seed + *seed_dev
+extern "C" int ercg_gcnii_layer_fwd_dev(const float* hi, int64_t ldhi, const float* h0, int64_t ldh0, const float* W,
+                                        int64_t ldw, float* out, int64_t ldo, int64_t M, int H, float theta, float alpha,
+                                        int relu, float drop_p, uint64_t seed, const uint64_t* seed_dev, void* stream) {
+  if (!seed_dev) return ERCG_EINVAL;
+  dim3 grid;
+  const int rc = gcnii_fwd_check(hi, ldhi, h0, ldh0, W, ldw, out, ldo, M, H, drop_p, grid);
+  if (rc != ERCG_OK || grid.x == 0) return rc;
+  Epilogue ep{nullptr, ACT_GCNII_FWD, hi, (long long)ldhi, 1.f, drop_p, (unsigned long long)seed,
+              h0, (long long)ldh0, theta, (1.f - theta) * (1.f - alpha), (1.f - theta) * alpha, relu ? 1 : 0};
+  ep.seed_dev = reinterpret_cast<const unsigned long long*>(seed_dev);
+  gcnii_fwd_dev_kernel<true, true><<<grid, GT, 0, (cudaStream_t)stream>>>(hi, ldhi, nullptr, W, ldw, out, ldo, M, H, 2 * H,
+                                                                         ep, h0, ldh0, H);
   return finish_launch();
 }
 

@@ -382,6 +382,16 @@ __global__ void relu_dropout_kernel(const float* __restrict__ x, float* __restri
   out[i] = v;
 }
 
+// relu_dropout_kernel with the seed offset read from device memory (a step counter that a captured graph advances)
+__global__ void relu_dropout_dev_kernel(const float* __restrict__ x, float* __restrict__ out, long long n, float p, float scale,
+                                        unsigned long long seed, const unsigned long long* __restrict__ seed_dev) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  float v = fmaxf(x[i], 0.f);
+  if (p > 0.f) v = hash_uniform(seed + __ldg(seed_dev), (unsigned long long)i) < p ? 0.f : v * scale;
+  out[i] = v;
+}
+
 static int check_graph(const int32_t* node_off, const int32_t* node_dlg, const int64_t* blk_off, int64_t N, int64_t SB,
                        int M) {
   if (!node_off || !node_dlg || !blk_off || N < 0 || SB < 0 || M < 1 || M > 3) return ERCG_EINVAL;
@@ -501,5 +511,15 @@ extern "C" int ercg_relu_dropout(const float* x, float* out, int64_t n, float p,
   if (n == 0) return ERCG_OK;
   if (!x || !out) return ERCG_EINVAL;
   relu_dropout_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, out, n, p, 1.f / (1.f - p), seed);
+  return finish_launch();
+}
+
+extern "C" int ercg_relu_dropout_dev(const float* x, float* out, int64_t n, float p, uint64_t seed, const uint64_t* seed_dev,
+                                     void* stream) {
+  if (!seed_dev || n < 0 || !(p >= 0.f && p < 1.f)) return ERCG_EINVAL;
+  if (n == 0) return ERCG_OK;
+  if (!x || !out) return ERCG_EINVAL;
+  relu_dropout_dev_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      x, out, n, p, 1.f / (1.f - p), seed, reinterpret_cast<const unsigned long long*>(seed_dev));
   return finish_launch();
 }

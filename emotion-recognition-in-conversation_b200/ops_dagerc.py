@@ -14,7 +14,11 @@ class DagStructure:
 
     __slots__ = ("graph", "lo", "cnt", "eoff", "E", "order", "Tmax", "windowp")
 
-    def __init__(self, graph, lengths_cpu, windowp=1):
+    def __init__(self, graph, lengths_cpu, windowp=1, e_cap=None, order=None):
+        """e_cap (optional): an upper bound on the predecessor count E, such as sum_d L_d (L_d - 1) / 2 (utterance i has at
+        most i predecessors); the attention-weight array is sized to it and E is not read back.  order (optional): the
+        dialogues by descending length (stable), int32 on the device.  With both, nothing waits for the device or copies
+        from the host."""
         self.graph, self.windowp = graph, int(windowp)
         N, dev = graph.N, graph.device
         self.lo = torch.empty(N, dtype=torch.int32, device=dev)
@@ -25,9 +29,21 @@ class DagStructure:
         check(lib().ercg_dag_build(_p(graph.node_off), _p(graph.node_dlg), _p(graph.spk), N, self.windowp, _p(self.lo),
                                    _p(self.cnt), _p(self.eoff), _p(total), _p(ws), ws.numel(), _stream()), "ercg_dag_build")
         lengths_cpu = lengths_cpu.cpu().to(torch.int64)
-        self.order = torch.argsort(lengths_cpu, descending=True, stable=True).to(torch.int32).to(dev)
+        self.order = order if order is not None else dag_order(lengths_cpu, dev)
         self.Tmax = int(lengths_cpu.max()) if lengths_cpu.numel() else 0
-        self.E = int(total.item())            # the one host sync: size of the attention-weight array
+        # size of the attention-weight array (the kernels index it through eoff): without e_cap, the one host sync
+        self.E = int(e_cap) if e_cap is not None else int(total.item())
+
+
+def dag_order(lengths_cpu, device):
+    """The dialogues by descending length (stable), int32 on ``device``: DagStructure.order."""
+    return torch.argsort(lengths_cpu.cpu().to(torch.int64), descending=True, stable=True).to(torch.int32).to(device)
+
+
+def dag_edge_capacity(lengths_cpu):
+    """sum_d L_d (L_d - 1) / 2: no DAG over these dialogues has more predecessor edges."""
+    L = lengths_cpu.cpu().to(torch.int64)
+    return int((L * (L - 1) // 2).sum())
 
 
 def dense_masks(spk_padded, windowp=1):

@@ -116,13 +116,26 @@ def sddmm(dhi, h, layout, G, accumulate):
     return G
 
 
-def _layer_fwd(hi, h0, W, theta, alpha, relu, p, seed):
+def _layer_fwd(hi, h0, W, theta, alpha, relu, p, seed, seed_dev=None):
     M, H = hi.shape
     out = torch.empty((M, H), dtype=torch.float32, device=hi.device)
-    check(lib().ercg_gcnii_layer_fwd(_p(hi), hi.stride(0), _p(h0), h0.stride(0), _p(W), W.stride(0), _p(out), H, M, H,
-                                     float(theta), float(alpha), 1 if relu else 0, float(p), int(seed) & (2 ** 64 - 1),
-                                     _stream()), "ercg_gcnii_layer_fwd")
+    args = (_p(hi), hi.stride(0), _p(h0), h0.stride(0), _p(W), W.stride(0), _p(out), H, M, H, float(theta), float(alpha),
+            1 if relu else 0, float(p), int(seed) & (2 ** 64 - 1))
+    if seed_dev is None:
+        check(lib().ercg_gcnii_layer_fwd(*args, _stream()), "ercg_gcnii_layer_fwd")
+    else:
+        check(lib().ercg_gcnii_layer_fwd_dev(*args, _p(seed_dev), _stream()), "ercg_gcnii_layer_fwd_dev")
     return out
+
+
+# Seeds of the dropout sites of the GCNII stack (the input dropout, h0's dropout, the 64 layers' output dropouts).  With
+# host seeds only, site k draws from seed + k, as before.  With a device word (ops.SEED_DEV: a step counter that grows by
+# 1 per step) site k at step s would then draw the mask site k + 1 drew at step s - 1, so the sites are spaced 2^32 apart.
+SITE_STRIDE = 1 << 32
+
+
+def site_seed(seed, k, seed_dev):
+    return seed + k * (1 if seed_dev is None else SITE_STRIDE)
 
 
 def _layer_bwd_input(dZ, W, theta, alpha):
@@ -182,20 +195,22 @@ class _GcniiStack(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, ahat, fc_w, fc_b, layout, lamda, alpha, p, seed, *Ws):
         x, _ = _rows(x)
+        seed_dev = ops.SEED_DEV                                  # the backward reads the same device word
         h0 = ops.gemm_nn(x, fc_w.t().contiguous(), fc_b, act=ops.ACT_RELU)
         h = h0
         if p > 0:
             h = torch.empty_like(h0)
-            check(lib().ercg_dropout(_p(h0), _p(h), h0.numel(), p, seed & (2 ** 64 - 1), _stream()), "ercg_dropout")
+            ops._dropout_call(h0, h, p, seed, seed_dev)
         saved = [h]
         his = []
         for l, W in enumerate(Ws, start=1):
             theta = math.log(lamda / l + 1)
             hi = spmm(ahat, h, layout)
-            h = _layer_fwd(hi, h0, W.contiguous(), theta, alpha, True, p, seed + l)
+            h = _layer_fwd(hi, h0, W.contiguous(), theta, alpha, True, p, site_seed(seed, l, seed_dev), seed_dev)
             his.append(hi)
             saved.append(h)
         ctx.layout, ctx.lamda, ctx.alpha, ctx.p, ctx.seed, ctx.nl = layout, lamda, alpha, p, seed, len(Ws)
+        ctx.seed_dev = seed_dev
         ctx.save_for_backward(x, ahat, fc_w, h0, *Ws, *his, *saved)
         return h
 
@@ -223,7 +238,7 @@ class _GcniiStack(torch.autograd.Function):
             G.zero_()
         if p > 0:                                                # hs[0] = dropout(h0): same counter-hash mask
             d0 = torch.empty_like(dh)
-            check(lib().ercg_dropout(_p(dh), _p(d0), dh.numel(), p, ctx.seed & (2 ** 64 - 1), _stream()), "ercg_dropout")
+            ops._dropout_call(dh, d0, p, ctx.seed, ctx.seed_dev)
             dh = d0
         dh0.add_(dh)
         dpre = ops.mask_pos(dh0, h0, 1.0)
@@ -279,7 +294,11 @@ class _ReluDropout(torch.autograd.Function):
     def forward(ctx, x, p, seed):
         x = x.contiguous()
         out = torch.empty_like(x)
-        check(lib().ercg_relu_dropout(_p(x), _p(out), x.numel(), p, seed & (2 ** 64 - 1), _stream()), "ercg_relu_dropout")
+        if ops.SEED_DEV is None:
+            check(lib().ercg_relu_dropout(_p(x), _p(out), x.numel(), p, seed & (2 ** 64 - 1), _stream()), "ercg_relu_dropout")
+        else:
+            check(lib().ercg_relu_dropout_dev(_p(x), _p(out), x.numel(), p, seed & (2 ** 64 - 1), _p(ops.SEED_DEV), _stream()),
+                  "ercg_relu_dropout_dev")
         ctx.p = p
         ctx.save_for_backward(out)
         return out

@@ -32,6 +32,11 @@ def _speaker_ids(speakers, device=None):
     return s.argmax(-1) if s.dim() == 3 else s.long()
 
 
+def speaker_count(speakers):
+    """The speaker count the DAG-ERC graph is built with: the one-hot width, or 2 for [B,L] ids."""
+    return max(int(speakers.size(-1)) if speakers.dim() == 3 else 2, 1)
+
+
 class DAGERCModule(nn.Module):
     def __init__(self, emb_dim=100, dropout=0.2, n_classes=7, gnn_layers=4, compute_padding=True):
         super().__init__()
@@ -62,16 +67,26 @@ class DAGERCModule(nn.Module):
         sm = ops_dagerc.dense_masks(ids, self.windowp)[1]
         return sm, torch.nn.functional.one_hot(sm, 2).float()
 
-    def forward(self, input_tensor, text_length, speaker_tensor, **kwargs):
+    def graph_lengths(self, text_length, Lmax):
+        """CPU int64 dialogue lengths the graph is built over: every dialogue padded to Lmax when compute_padding."""
+        if self.compute_padding:
+            return torch.full((text_length.numel(),), int(Lmax), dtype=torch.int64)
+        return text_length.cpu().to(torch.int64)
+
+    def forward(self, input_tensor, text_length, speaker_tensor, graph=None, dag=None, **kwargs):
+        """graph / dag (optional): the K1 graph over graph_lengths() with the speaker ids, and its DagStructure, built by a
+        caller that keeps the batch's sizes on the host (train_step.DagercTrainStep).  With both given, the forward copies
+        nothing from the host and never waits for the device."""
         B, Lmax, emb = input_tensor.shape
         dev = input_tensor.device
-        ids = _speaker_ids(speaker_tensor, dev)
-        lengths = text_length.cpu().to(torch.int64)
-        if self.compute_padding:
-            lengths = torch.full((B,), Lmax, dtype=torch.int64)
-        g = build_graph(lengths, ids, 0, 0, max(int(speaker_tensor.size(-1)) if speaker_tensor.dim() == 3 else 2, 1),
-                        device=dev, reference_layout=False, mean_weight=False)
-        dag = ops_dagerc.DagStructure(g, lengths, self.windowp)
+        if graph is None or dag is None:
+            lengths = self.graph_lengths(text_length, Lmax)
+        if graph is None:
+            graph = build_graph(lengths, _speaker_ids(speaker_tensor, dev), 0, 0, speaker_count(speaker_tensor), device=dev,
+                                reference_layout=False, mean_weight=False)
+        g = graph
+        if dag is None:
+            dag = ops_dagerc.DagStructure(g, lengths, self.windowp)
         flat = input_tensor.reshape(B * Lmax, emb)
         a_rows = None if self.compute_padding else g.pad_row
         H0 = ops.linear(flat, self.fc1.weight, self.fc1.bias, act=ops.ACT_RELU, a_rows=a_rows)

@@ -70,11 +70,14 @@ class MMGCNModule(nn.Module):
         self.smax_fc = nn.Linear(400 * len(self.modals), n_classes)
 
     def forward(self, text_feature=None, audio_feature=None, visual_feature=None, speaker_tensor=None, text_length=None,
-                **kwargs):
+                graph=None, full_graph=None, **kwargs):
+        """graph / full_graph (optional): lengths_graph(text_length) and lengths_graph([Lmax] * B), built once by a caller
+        that runs many batches of the same lengths (train_step.MmgcnTrainStep).  With both given and text_length on the
+        host, the forward copies nothing from the host and never waits for the device."""
         ref = text_feature if text_feature is not None else (audio_feature if audio_feature is not None else visual_feature)
         Lmax, B = ref.shape[0], ref.shape[1]
         dev = ref.device
-        g = lengths_graph(text_length, dev)                                  # the real utterances, dialogue-major
+        g = graph if graph is not None else lengths_graph(text_length, dev)  # the real utterances, dialogue-major
         rows_seq = ops_mmgcn.node_rows(g, Lmax, seq_first=True)              # packed node -> row of a [Lmax*B, *] tensor
         fa = fv = fl = []
         if 'a' in self.modals:
@@ -83,8 +86,7 @@ class MMGCNModule(nn.Module):
             fv = ops.linear(visual_feature.reshape(Lmax * B, -1), self.linear_v.weight, self.linear_v.bias, a_rows=rows_seq)
         if 't' in self.modals:
             # every dialogue as a length-Lmax sequence (padding rows = linear_l(0) = its bias), dialogue-major
-            full_len = torch.full((B,), Lmax, dtype=torch.int64)
-            gf = lengths_graph(full_len, dev)
+            gf = full_graph if full_graph is not None else lengths_graph(torch.full((B,), Lmax, dtype=torch.int64), dev)
             rows_full = ops_mmgcn.node_rows(gf, Lmax, seq_first=True)
             t200 = ops.linear(text_feature.reshape(Lmax * B, -1), self.linear_l.weight, self.linear_l.bias, a_rows=rows_full)
             emo = birnn_forward(self.lstm_l, t200, gf, None, self.training)  # [B*Lmax, 200]

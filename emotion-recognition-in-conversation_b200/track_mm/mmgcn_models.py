@@ -80,7 +80,7 @@ class GCNII_lyc(nn.Module):
             x = ops.dropout(x, p, seed)
         fc = self.fcs[0]
         h = ops_mmgcn.gcnii_stack(x, adj.values, fc.weight, fc.bias, [c.weight for c in self.convs], adj.layout,
-                                  self.lamda, self.alpha, p, seed + 1)
+                                  self.lamda, self.alpha, p, ops_mmgcn.site_seed(seed, 1, ops.SEED_DEV))
         return torch.cat([x, h], dim=-1) if self.use_residue else h
 
 

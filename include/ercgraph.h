@@ -446,6 +446,13 @@ int ercg_mmgcn_sddmm(const float* dhi, int64_t ldd, const float* h, int64_t ldh,
 int ercg_gcnii_layer_fwd(const float* hi, int64_t ldhi, const float* h0, int64_t ldh0, const float* W, int64_t ldw,
                          float* out, int64_t ldo, int64_t M, int H, float theta, float alpha, int relu, float drop_p,
                          uint64_t seed, void* stream);
+/* ercg_gcnii_layer_fwd with the dropout mask drawn from seed + *seed_dev (seed_dev: device uint64, as ercg_gemm_nn's): the
+ * GCNII stack inside a train step captured in a CUDA graph, which points seed_dev at its device step counter so that every
+ * replay draws a fresh mask.  *seed_dev == 0 gives ercg_gcnii_layer_fwd(seed) bit for bit.  seed_dev NULL and every
+ * argument ercg_gcnii_layer_fwd rejects: the same error code before any launch. */
+int ercg_gcnii_layer_fwd_dev(const float* hi, int64_t ldhi, const float* h0, int64_t ldh0, const float* W, int64_t ldw,
+                             float* out, int64_t ldo, int64_t M, int H, float theta, float alpha, int relu, float drop_p,
+                             uint64_t seed, const uint64_t* seed_dev, void* stream);
 int ercg_gcnii_layer_bwd_input(const float* dZ, int64_t lddz, const float* Wt, int64_t ldwt, float* dS, int64_t ldds,
                                int64_t M, int H, float theta, float alpha, void* stream);
 
@@ -461,6 +468,10 @@ int ercg_speaker_embed_add(const float* x, int64_t ldx, const float* qmask, int 
                            int D, void* stream);
 /* out = dropout(relu(x)) with the counter-hash mask (relu(dropout(x)) of mmgcn.py:117-118 is the same function) */
 int ercg_relu_dropout(const float* x, float* out, int64_t n, float p, uint64_t seed, void* stream);
+/* ercg_relu_dropout with the mask drawn from seed + *seed_dev (as ercg_dropout_dev): *seed_dev == 0 gives
+ * ercg_relu_dropout(seed) bit for bit.  seed_dev NULL, n < 0 or p outside [0, 1): ERCG_EINVAL before any launch. */
+int ercg_relu_dropout_dev(const float* x, float* out, int64_t n, float p, uint64_t seed, const uint64_t* seed_dev,
+                          void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Optimizer tail of the train steps (SURVEY.md 8f-3) on ONE flat fp32 buffer of all live parameters and its gradient twin:
