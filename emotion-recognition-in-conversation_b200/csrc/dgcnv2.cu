@@ -95,7 +95,7 @@ using namespace ercg;
 extern "C" int ercg_masked_edge_att_fwd(const float* S, int64_t ldS, const int32_t* node_off, const int32_t* node_dlg,
                                         const int32_t* t_rowptr, const int32_t* t_eid, int64_t Lmax, int wp, int wf,
                                         float* nu, float* stat, int64_t N, void* stream) {
-  if (N < 0 || Lmax < 0) return ERCG_EINVAL;
+  if (N < 0 || Lmax < 1 || ldS < Lmax) return ERCG_EINVAL;     // S holds a column per source position: ldS >= Lmax
   if (N == 0) return ERCG_OK;
   if (!S || !node_off || !node_dlg || !t_rowptr || !t_eid || !nu || !stat) return ERCG_EINVAL;
   masked_edge_att_fwd_kernel<<<(unsigned)((N + EW - 1) / EW), EW * 32, 0, (cudaStream_t)stream>>>(
@@ -107,7 +107,7 @@ extern "C" int ercg_masked_edge_att_bwd(const float* S, int64_t ldS, const int32
                                         const int32_t* t_rowptr, const int32_t* t_eid, int64_t Lmax, int wp, int wf,
                                         const float* nu, const float* dnu, const float* stat, float* dS, int64_t ldd,
                                         int64_t N, void* stream) {
-  if (N < 0 || Lmax < 0) return ERCG_EINVAL;
+  if (N < 0 || Lmax < 1 || ldS < Lmax || ldd < Lmax) return ERCG_EINVAL;
   if (N == 0) return ERCG_OK;
   if (!S || !node_off || !node_dlg || !t_rowptr || !t_eid || !nu || !dnu || !stat || !dS) return ERCG_EINVAL;
   masked_edge_att_bwd_kernel<<<(unsigned)((N + EW - 1) / EW), EW * 32, 0, (cudaStream_t)stream>>>(

@@ -36,7 +36,10 @@ class _MaskedEdgeAtt(torch.autograd.Function):
 
 def masked_edge_att(S, graph, Lmax, wp, wf):
     """S [B*Lmax, >= Lmax'] (dialogue-major full-length rows x max_seq_len columns) -> edge weights in by-destination order."""
-    assert S.size(0) == graph.B * int(Lmax) and S.size(1) >= int(Lmax) or S.size(1) >= 1
+    Lmax = int(Lmax)
+    if S.dim() != 2 or S.size(0) != graph.B * Lmax or S.size(1) < Lmax:
+        raise ValueError("masked_edge_att: S must be [B * Lmax, >= Lmax] = [%d, >= %d], got %s"
+                         % (graph.B * Lmax, Lmax, tuple(S.shape)))
     return _MaskedEdgeAtt.apply(S, graph, Lmax, wp, wf)
 
 

@@ -1,18 +1,19 @@
-"""The COGMEN, DialogueGCN, MMGCN and DAG-ERC train steps as ONE replayable unit each (SURVEY.md 8e / 8f-3; reference:
-CogmenTrainer.train_step, track_mm/cogmen.py:179-195, the DialogueGCN step, dgcn.py:117-134, MMGCN's, mmgcn.py:141-157, and
-DAG-ERC's, dagerc.py:217-237, under accelerate/DDP, lumo/trainer/trainer.py:62-64,315-327).
+"""The COGMEN, DialogueGCN, dgcnv2, MMGCN and DAG-ERC train steps as ONE replayable unit each (SURVEY.md 8e / 8f-3;
+reference: CogmenTrainer.train_step, track_mm/cogmen.py:179-195, the DialogueGCN step, dgcn.py:117-134, dgcnv2's
+(track_mm/dgcnv2.py), MMGCN's, mmgcn.py:141-157, and DAG-ERC's, dagerc.py:217-237, under accelerate/DDP,
+lumo/trainer/trainer.py:62-64,315-327).
 
     graph build (K1) -> forward -> cross entropy -> backward -> gradient all-reduce -> [clip] -> Adam
 
 * Nothing in the step touches the host: sizes and the possible relation ids come from the host-side batch description,
-  the loss normaliser is host-known (COGMEN: the global utterance count) or reduced on the device (the other three), the
+  the loss normaliser is host-known (COGMEN: the global utterance count) or reduced on the device (the other four), the
   optimizer's step counter and the dropout seed live on the device.  ``capture()`` records the step once into a
   CUDA graph (collectives included) and ``replay()`` relaunches it: ~50 kernel launches + autograd bookkeeping per step
   become one graph launch -- what makes 2^20 utterances split over 8 GPUs (1.7 ms of kernels per rank) scale.
 * Collectives per step with world > 1: COGMEN's BatchNorm statistics (2H+1 doubles, forward), their backward sums (2H
   floats) -- both only in ``bn_sync="global"`` mode; ``"local"`` is the reference's DDP behaviour (per-rank statistics) --,
-  the DialogueGCN / MMGCN / DAG-ERC loss (numerator, denominator: 2 floats, forward), and the flat gradient buffer.  COGMEN's loss numerator
-  rides in the tail of the gradient buffer; there is no separate loss collective.
+  the DialogueGCN / dgcnv2 / MMGCN / DAG-ERC loss (numerator, denominator: 2 floats, forward), and the flat gradient buffer.
+  COGMEN's loss numerator rides in the tail of the gradient buffer; there is no separate loss collective.
 * Transport: libercgraph's peer-memory kernels over NVLink (p2p.PeerComm: ercg_p2p_allreduce for the gradient buckets,
   ercg_p2p_bn_stats / ercg_p2p_bn_act_bwd_reduce = the BatchNorm reductions fused with their exchange) when every rank can set
   them up, else torch.distributed on ``group`` -- the results are the same to the last bit (rank-ordered sums).
@@ -319,6 +320,77 @@ class MmgcnTrainStep(_FlatTrainStep):
 
     def global_loss(self):
         """Global mean loss of the last step (eager or replayed)."""
+        return self._last_loss
+
+
+class Dgcnv2TrainStep(_FlatTrainStep):
+    def __init__(self, model, lengths, lmax=None, speakers_present=None, lr=3e-4, weight_decay=0.0, class_weight=None, world=1,
+                 group=None, transport="auto", overlap=True):
+        """dgcnv2 (track_mm.dgcnv2.DGCNModule, base 'LSTM', 'GRU' or 'None') step.  See _FlatTrainStep.  lengths: CPU [B]
+        dialogue lengths of THIS rank's batch.  lmax: the padded length of the GLOBAL batch (default: this batch's longest
+        dialogue; at most max_seq_len = 110).  The unpacked reverse base starts in the padding (dgcnv2.py:151) and the edge
+        attention's softmax runs over all padded positions (dgcnv2_models.py:544), so a rank pads its shard to the global
+        lmax, and the shards then take the step one GPU takes on the whole batch.  speakers_present: the speaker ids the
+        data set uses (default every speaker id of the model).  lr / weight_decay: train_mm's dgcnv2 Adam.  class_weight: the
+        cross entropy's class weights (track_mm.dgcn.LOSS_WEIGHTS in the 6-way setting) or None.  The loss is the weighted
+        mean over the GLOBAL batch (numerator and denominator all-reduced in the forward when world > 1).
+
+        step(x_rows, speaker_ids, labels): x_rows [B * lmax, D] = the batch-first padded input viewed as rows (16-byte
+        aligned), speaker_ids packed [N], labels packed int64 [N]."""
+        self.lengths = _lengths(lengths, "Dgcnv2TrainStep")
+        longest, cap = int(self.lengths.max()), model.att_model.max_seq_len
+        self.lmax = longest if lmax is None else int(lmax)
+        if self.lmax < longest:
+            raise ValueError("Dgcnv2TrainStep: lmax %d is shorter than the longest dialogue (%d)" % (self.lmax, longest))
+        if self.lmax > cap:
+            raise ValueError("Dgcnv2TrainStep: lmax %d exceeds max_seq_len %d" % (self.lmax, cap))
+        if speakers_present is None:
+            speakers_present = range(model.n_speakers)
+        opt = FlatAdam(model.parameters(), lr=lr, weight_decay=weight_decay)
+        # every parameter but the edge attention's dead modules gets a gradient; flat_bytes() bounds it by all parameters
+        super().__init__(model, opt, max(8 << 20, opt.flat_bytes()), world, group, transport, overlap)
+        self.sizes = graph_sizes(self.lengths, model.window_past, model.window_future)
+        self.lengths_dev = self.lengths.to(self.dev)
+        self.rel_ids = relation_ids_for_speakers(speakers_present, model.n_speakers)
+        self.class_weight = None
+        if class_weight is not None:
+            self.class_weight = torch.as_tensor(class_weight, dtype=torch.float32).to(self.dev).contiguous()
+        self.gf = self.gfull = None
+
+    def _forward_backward(self, x, spk, labels):
+        from .track_mm.dgcnv2 import length_graphs
+        m = self.model
+        B, N = self.lengths.numel(), self.sizes[0]
+        if x.dim() != 2 or x.size(0) != B * self.lmax or tuple(spk.shape) != (N,) or tuple(labels.shape) != (N,):
+            raise ValueError("Dgcnv2TrainStep: x_rows %s, speaker_ids %s, labels %s; the step was built for [%d, D], [%d], [%d]"
+                             % (tuple(x.shape), tuple(spk.shape), tuple(labels.shape), B * self.lmax, N, N))
+        if self.gf is None:
+            # these two depend on the lengths alone: built once, by the first step (an eager one: capture() warms up first)
+            self.gf, self.gfull = length_graphs(self.lengths, self.lmax, self.dev)
+        g = build_graph(self.lengths_dev, spk, m.window_past, m.window_future, m.n_speakers, device=self.dev, mean_weight=False,
+                        sizes=self.sizes, relation_ids=self.rel_ids)
+        logits, _ = m.forward_packed(x, spk, self.lengths_dev, self.lmax, graphs=(g, self.gf, self.gfull))
+        loss = ops.cross_entropy(logits, labels, self.class_weight, reduce_sync=self.reduce_main if self.world > 1 else None)
+        self._backward(loss)
+        self._last_graph = g
+        return loss
+
+    def _late_params(self):
+        m = self.model
+        if m.base_model == "None":
+            return m.base_linear.weight, m.base_linear.bias
+        rnn = m.lstm if m.base_model == "LSTM" else m.gru
+        # the LSTM's hoisted input transform folds in b_hh; the GRU applies b_hh inside the recurrence (dgcn_models.py:37-40)
+        names = ("weight_ih", "bias_ih", "bias_hh") if m.base_model == "LSTM" else ("weight_ih", "bias_ih")
+        return tuple(getattr(rnn, n + "_l0" + d) for n in names for d in ("", "_reverse"))
+
+    def _check_inputs(self):
+        self._last_graph.check_inputs()
+        self.gf.check_inputs()
+        self.gfull.check_inputs()
+
+    def global_loss(self):
+        """Global weighted mean loss of the last step (eager or replayed)."""
         return self._last_loss
 
 

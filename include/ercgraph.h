@@ -555,7 +555,8 @@ int ercg_p2p_bn_stats(void* const* regions_dev, int rank, int world, const float
  *   nu[i -> j] = e_j / (Z_win + 1e-10 (Z_all - Z_win)),  e_j' = exp(S[j', i] - max_j' S[., i]) over ALL Lmax positions,
  *   Z_win over the targets j of i's window [max(0, i-wp), min(len-1, i+wf)] (wp / wf = -1: unbounded);
  * nu is written in by-destination edge order (through t_rowptr / t_eid of ercg_graphify_csr); stat [N,2] keeps (max, Den).
- * Backward: dS (zero-initialised by the caller, same layout as S) from dnu. */
+ * Backward: dS (zero-initialised by the caller, same layout as S) from dnu.
+ * ERCG_EINVAL before any launch for Lmax < 1, ldS < Lmax or (backward) ldd < Lmax. */
 int ercg_masked_edge_att_fwd(const float* S, int64_t ldS, const int32_t* node_off, const int32_t* node_dlg,
                              const int32_t* t_rowptr, const int32_t* t_eid, int64_t Lmax, int wp, int wf,
                              float* nu, float* stat, int64_t N, void* stream);
